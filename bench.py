@@ -15,15 +15,19 @@ C3 (paired OT, 2 x 100k, 10k genes, batch 1024, dense fp32 plan resident: 40 GB)
 n_hidden 256, batch 2048, plan resident as bf16: 80 GB), each with value / e2e / roofline, as far as the time budget allows
 (--budget seconds).  `--workload` picks another headline.
 
-Timed region: R blocks of exactly K steps each (CUDA events on the launching stream, barrier + synchronize on both sides of
-every block, max over ranks); the reported ms_per_step is the MEDIAN block (R >= 5 and >= ~1 s of steps in total), so a
-20-step driver run is not at the mercy of one slow block.  Prints ONE JSON line on rank 0.
+Timed region: exactly K steps (CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks),
+after W untimed warm-up steps (at least MIN_WARMUP).  That one window is all that is timed, and a short one is noisy (see
+DESIGN.md section 6): take K in the hundreds for a steadier number.  Prints ONE JSON line on rank 0.
+
+    python bench.py --steps K --warmup W --dump-outputs DIR
+
+also writes what the last timed step handed its caller to DIR/*.npy (see dump_outputs), so that two builds can be compared
+output for output: with the same arguments every input is the same from run to run.
 """
 from __future__ import annotations
 
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -47,6 +51,11 @@ WORKLOADS = {
 S_DIM, P_DIM, HD = 25, 10, 256
 METRIC = "training cells/sec (fwd+bwd ELBO + Adam)"
 T_START = time.time()
+# least number of warm-up steps of the CUDA path: on a B200, C5 steps reached their steady time only after ~150 steps (the
+# first 100 ran 2-3 % slower).  A count, not a time, so that what precedes the last timed step (and with it the
+# --dump-outputs files) depends on the arguments alone.
+MIN_WARMUP = 256
+DUMP_SAMPLE = 1 << 22  # elements kept of a dumped vector longer than this (16 MB as float32)
 
 
 def peaks():
@@ -207,8 +216,7 @@ def run_reference(args):
     if rank != 0:
         return
     workload = args.workload
-    B = WORKLOADS[workload][4]
-    steps = max(2, min(args.steps, 20 if B <= 1024 else 8))  # bounded sample: a C5-shaped minibatch costs ~1-2 s on the host
+    steps = args.steps  # a C5-shaped minibatch costs ~1-2 s on the host
     warm = min(args.warmup, 1)
     v, ms, cores, sample = cpu_reference_cells_per_sec(workload, steps, warm)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "cells/s", "n_gpus": args.gpus, "steps": steps,
@@ -290,10 +298,11 @@ class Bench:
             self.dist.barrier()
         torch.cuda.synchronize()
 
-    def timed_blocks(self, K, W, step_fn, profile=False):
-        """W warm-up steps, then R blocks of exactly K steps; returns the per-block ms (max over ranks each).
-        profile: cudaProfilerStart after the warm-up (`ncu --profile-from-start off` then sees only training steps, not the
-        data generation, the index draws or the graph capture)"""
+    def timed_steps(self, K, W, step_fn, profile=False):
+        """W untimed warm-up steps, then exactly K timed steps; returns their ms (max over ranks) and the number of steps
+        run in all.
+        profile: cudaProfilerStart before the timed steps (`ncu --profile-from-start off` then sees only training steps, not
+        the data generation, the index draws or the graph capture)"""
         n_steps_hint = 64
         rows = self.draw_rows(n_steps_hint)
         for s in range(W):
@@ -301,31 +310,18 @@ class Bench:
         self.barrier()
         if profile:
             torch.cuda.profiler.start()
-        # pilot block to size R: >= 5 blocks and ~1 s of timed steps in total, at most 60 blocks
-        blocks, s = [], W
-        R = 5
-        while len(blocks) < R:
-            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            self.barrier()
-            ev0.record()
-            for _ in range(K):
-                step_fn(rows, s % n_steps_hint)
-                s += 1
-            ev1.record()
-            self.barrier()
-            ms = ev0.elapsed_time(ev1)
-            if self.dist is not None:
-                t = torch.tensor([ms], device=self.dev)
-                self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
-                ms = float(t.item())
-            blocks.append(ms)
-            if len(blocks) == 1:
-                R = int(min(60, max(5, math.ceil(1000.0 / max(ms, 1e-3)))))
-                if self.dist is not None:  # same R on every rank
-                    t = torch.tensor([R], device=self.dev)
-                    self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
-                    R = int(t.item())
-        return blocks
+        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        ev0.record()
+        for s in range(W, W + K):
+            step_fn(rows, s % n_steps_hint)
+        ev1.record()
+        self.barrier()
+        ms = ev0.elapsed_time(ev1)
+        if self.dist is not None:
+            t = torch.tensor([ms], device=self.dev)
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
+            ms = float(t.item())
+        return ms, W + K
 
     # ---- device-resident throughput (graph replay)
     def measure_value(self, K, W):
@@ -342,15 +338,10 @@ class Bench:
                 self.loop.step(self.static)
 
         n0 = self.lib.spv_launch_count()
-        blocks = self.timed_blocks(K, W, step, profile=bool(os.environ.get("SPV_PROFILE_RANGE")))
-        ms = float(np.median(blocks))
-        if use_graph:
-            launches, per_step = self.per_step_launches * K * len(blocks), self.per_step_launches
-        else:
-            launches = self.lib.spv_launch_count() - n0
-            per_step = launches // (K * len(blocks) + W)
-        return {"value": self.world * 2 * self.B * K / (ms * 1e-3), "ms_per_step": ms / K, "blocks_ms": [round(b, 4) for b in blocks],
-                "launches_per_step": int(per_step), "gpu_launches": int(launches)}
+        ms, n_run = self.timed_steps(K, W, step, profile=bool(os.environ.get("SPV_PROFILE_RANGE")))
+        per_step = self.per_step_launches if use_graph else (self.lib.spv_launch_count() - n0) // n_run
+        return {"value": self.world * 2 * self.B * K / (ms * 1e-3), "ms_per_step": ms / K, "ms": round(ms, 4),
+                "launches_per_step": int(per_step), "gpu_launches": int(per_step * K)}
 
     # ---- the likelihood kernels alone, timed with CUDA events on the launching stream (eager passes, second group off)
     def measure_roofline(self, K):
@@ -490,8 +481,7 @@ class Bench:
             opt.step()
             out_host.copy_(lo.loss.detach(), non_blocking=True)
 
-        blocks = self.timed_blocks(K, max(W, 4), step)  # the first three calls run eagerly / capture the two buffer sets' graphs
-        ms = float(np.median(blocks))
+        ms, _ = self.timed_steps(K, max(W, 4), step)  # the first three calls run eagerly / capture the two buffer sets' graphs
         esz = 2 if x_dtype == torch.uint16 else 4
         h2d = 2 * (B * G * esz) + 2 * 2 * B * 4
         del m, opt, host
@@ -544,11 +534,27 @@ class Bench:
             out_host.copy_(loop.engine.loss_out, non_blocking=True)
             state["n"] = i + 1
 
-        blocks = self.timed_blocks(K, W, step)
-        ms = float(np.median(blocks))
+        ms, _ = self.timed_steps(K, W, step)
         h2d = sum(host_x[g][0].numel() * 2 + host_l[g][0].numel() * 4 for g in (0, 1))
         return {"value": self.world * 2 * B * K / (ms * 1e-3), "unit": "cells/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": 32,
                 "ms_per_step": ms / K, "api": "spvipes_b200.trainer.TrainLoop (host uint16 minibatches in pinned memory, loss terms read back)"}
+
+
+def dump_outputs(eng, out_dir):
+    """what the last step handed its caller, as float32 DIR/<name>.npy: the loss terms (engine.loss_terms()), the parameters
+    after the optimiser step, their gradients and the BatchNorm running statistics (the engine's flat stores, in their fixed
+    layout).  A vector longer than DUMP_SAMPLE is cut to the same seeded sample of positions on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    torch.cuda.synchronize()
+    n = eng.params.numel
+    keep = None
+    if n > DUMP_SAMPLE:
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values.to(eng.device)
+    sample = lambda t: t if keep is None else t[keep]
+    arrays = {"loss_terms": eng.loss_terms(), "params": sample(eng.params.flat), "grads": sample(eng.grads),
+              "running_stats": eng.buffers.flat}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_ours(args):
@@ -577,6 +583,8 @@ def run_ours(args):
         clk.start()
     res = bench.measure_value(K, W)
     clocks = clk.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(bench.eng, args.dump_outputs)
     if hasattr(bench.loop.grad_sync, "check"):
         bench.loop.grad_sync.check()  # a handshake that timed out would have produced a number without the exchange
     sync_kind = bench.sync_kind
@@ -595,8 +603,7 @@ def run_ours(args):
                       if args.precision == "bf16" else "f32"),
             "data": "synthetic", "config": dict(workload_config(workload, world), grad_sync=sync_kind), "clocks": clocks, "e2e": e2e,
             "e2e_uint16_input": e2e_u16, "e2e_trainloop": e2e_tl, "e2e_torch_adam": e2e_torch, "gpu_launches": res["gpu_launches"],
-            "launches_per_step": res["launches_per_step"], "timing": {"blocks": len(res["blocks_ms"]), "steps_per_block": K,
-                                                                        "block_ms": res["blocks_ms"], "reported": "median block"},
+            "launches_per_step": res["launches_per_step"], "timing": {"timed_steps": K, "ms": res["ms"]},
             "roofline": roofline, "cpu_baseline": None, "final_loss": loss}
     # ---- the other BASELINE configs in the same run (N = 1 only), within the time budget
     configs = []
@@ -611,7 +618,7 @@ def run_ours(args):
                 b2 = Bench(wl, args, dev, None, 0, 1)
                 r2 = b2.measure_value(K, W)
                 entry = {"config": workload_config(wl, 1), "value": r2["value"], "unit": "cells/s", "ms_per_step": r2["ms_per_step"],
-                         "launches_per_step": r2["launches_per_step"], "blocks": len(r2["blocks_ms"]),
+                         "launches_per_step": r2["launches_per_step"],
                          "final_loss": float(b2.eng.loss_out[0].item()), "roofline": b2.measure_roofline(K)}
                 if not args.no_e2e:
                     entry["e2e"] = b2.measure_e2e_plugin(K, W, torch.float32)
@@ -637,7 +644,8 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--warmup", type=int, default=MIN_WARMUP,
+                    help=f"untimed steps before the timed ones (CUDA path: at least {MIN_WARMUP})")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C5", choices=list(WORKLOADS))
     ap.add_argument("--cpu-steps", type=int, default=12)
@@ -648,8 +656,13 @@ def main():
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"],
                     help="bf16: tcgen05 tensor-core path for the large GEMMs; fp32: SIMT path")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the host-fed measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/*.npy (float32)")
     args = ap.parse_args()
-    args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl ours)")
+    args.warmup = max(args.warmup, MIN_WARMUP) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
     else:
