@@ -15,6 +15,10 @@ POE_LABEL, POE_PAIRED, POE_CLUSTER = 0, 1, 2
 PARTNER_PAD, PARTNER_ABSENT = -1, -2
 POE_MODES = {"label": POE_LABEL, "paired": POE_PAIRED, "cluster": POE_CLUSTER}
 GENEC_ROWS = 21  # decoder_common.cuh GC_N
+# widest latent input (P + S, plus one copy of the batch covariates per branch) of the decoder kernels: the fused tensor-core
+# decoder (decoder_common.cuh ZK_MAX_LATENT) and every decoder path (DEC_MAX_LATENT: spv_dec_fold, spv_dec_gene_bwd)
+ZK_MAX_LATENT = 58
+DEC_MAX_LATENT = 96
 
 p, i, ll, f, u64, u32 = C.c_void_p, C.c_int, C.c_longlong, C.c_float, C.c_ulonglong, C.c_uint
 

@@ -41,6 +41,7 @@ enum {
 #define ZK_RP 60
 #define ZK_RS 62
 #define ZK_MAX_LATENT 58   // P + S (+ covariate columns) must fit below ZK_ONE
+#define DEC_MAX_LATENT 96  // P + S (+ covariate columns) of every decoder path: the per-gene kernels' shared-memory sizing
 
 // Per-gene count tables (spv_dec_theta_tables): for raw counts c < NB_TAB, t = log1p(c) and
 //   forward  tgf[g][c] = (t, lgamma(t + theta) - lgamma(theta) - lgamma(t + 1))

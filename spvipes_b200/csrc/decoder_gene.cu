@@ -435,7 +435,7 @@ extern "C" int spv_dec_theta_tables(const float* px_r, int G, void* tgf, void* t
 // ptrs: Wp, Ws, gamma_p, beta_p, gamma_s, beta_s, px_r, rm_p, rv_p, rm_s, rv_s, zz, zsum, (unused), wfold, genec, zmean, zcov
 extern "C" int spv_dec_fold(const void* const* ptrs, long long ld_zz, int B, int G, int P, int S, int training, float eps,
                             float momentum, void* wz_bf16, long long ld_wz, int Gp, int HD, void* wz_f16, void* zc_f16, void* stream) {
-    if (!ptrs || B <= 0 || G <= 0 || P <= 0 || S <= 0 || P + S > 96) return SPV_ERR_ARG;
+    if (!ptrs || B <= 0 || G <= 0 || P <= 0 || S <= 0 || P + S > DEC_MAX_LATENT) return SPV_ERR_ARG;
     for (int i = 0; i < 18; ++i)
         if (!ptrs[i]) return SPV_ERR_ARG;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -656,7 +656,7 @@ extern "C" int spv_dec_gene_bwd_parts(int G) { return G > 0 ? (G + GENES_PER_CTA
 // colsum_in_q != 0 (needs ldq > 0): the column sums of dyp / dys are not rows 0 / 1 of colsum but the column right behind each Q
 // block, Qp[g * ldq + P] and Qs[g * ldq + S] (the ones column of the single-sweep Q GEMM, spv_dec_zq4)
 extern "C" int spv_dec_gene_bwd(const void* const* ptrs, long long ldq, int B, int G, int P, int S, int colsum_in_q, void* stream) {
-    if (!ptrs || B <= 0 || G <= 0 || P <= 0 || S <= 0 || P + S > 96) return SPV_ERR_ARG;
+    if (!ptrs || B <= 0 || G <= 0 || P <= 0 || S <= 0 || P + S > DEC_MAX_LATENT) return SPV_ERR_ARG;
     for (int i = 0; i < 18; ++i)
         if (!ptrs[i]) return SPV_ERR_ARG;
     GeneBwdP p;

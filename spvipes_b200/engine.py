@@ -339,9 +339,14 @@ class StepEngine:
             raise ValueError("precision must be 'fp32' or 'bf16'")
         self.precision = precision
         self.bf16 = precision == "bf16"
-        # fused tcgen05 decoder-GEMMs + NB-likelihood kernel (bf16 mode); the latent columns must fit one 64-wide k-block
+        # fused tcgen05 decoder-GEMMs + NB-likelihood kernel (bf16 mode); the latent columns must fit the 64-wide branch k-block
+        # below its six additive columns (decoder_common.cuh ZK_MAX_LATENT); wider latents take the unfused bf16 decoder
         nb_cols = int(n_batch) if int(n_batch) > 1 else 0
-        self.fused_nb = self.bf16 and int(n_shared) + int(n_private) + 2 * nb_cols <= 64
+        kz_dec = int(n_shared) + int(n_private) + 2 * nb_cols
+        if kz_dec > L.DEC_MAX_LATENT:
+            raise NotImplementedError(f"n_dimensions_shared + n_dimensions_private (+ 2 n_batch) = {kz_dec} is not implemented (the "
+                                      f"decoder kernels take at most {L.DEC_MAX_LATENT} latent columns)")
+        self.fused_nb = self.bf16 and kz_dec <= L.ZK_MAX_LATENT
         # operands of the decoder GEMMs: fp16 on the fused path (2^-12 rounding, three bits more than bf16; every operand's range
         # is bounded: activations after BatchNorm, weights, gradients stored in natural units), bf16 on the unfused fallback
         # one sweep over [B, G] per training step: the forward sweep also emits what the backward needs (csrc/nb_tc_train.cu);
