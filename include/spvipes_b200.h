@@ -125,6 +125,17 @@ int spv_to_bf16_block(const float* src, long long ld_src, void* dst, long long l
  * appended to the encoders' input, nn/networks.py:110-118); they do not enter the library size */
 int spv_counts_to_bf16(int src, const void* X, long long ldx, const int* rows, void* dst, void* dst_lo, long long ld_dst, int B,
                        int G, float* lib, const int* cov, int n_cov, void* stream);
+/* minibatch gather from a device-resident CSR count matrix [N, G]: indptr int64 [N + 1], indices uint16 [nnz] (canonical: no
+ * column twice in a row), values [nnz] uint16 (src = SPV_SRC_U16_LOG1P) or float (SPV_SRC_F32_LOG1P).  xs[b, :] = dense row
+ * rows[b] (rows NULL: b) in the dtype of `values`, zero padded to the next 16-byte boundary; ld_xs >= G, a multiple of 8 (uint16)
+ * resp. 4 (float), xs 16-byte aligned.  dst != NULL: also T / T_lo / lib / covariate columns exactly as spv_counts_to_bf16 on
+ * the gathered rows (bit-identical to it on a 16-byte aligned dense row; ld_dst a multiple of 8); dst == NULL: xs only (lib and
+ * cov unused).  G <= spv_csr_max_genes(src): the row is assembled in shared memory (65536 for uint16, the range of the column
+ * index; 58104 for float, 227 KB).  Host-side query. */
+int spv_csr_max_genes(int src);
+int spv_csr_gather(int src, const long long* indptr, const unsigned short* indices, const void* values, const int* rows, int B,
+                   int G, void* xs, long long ld_xs, void* dst, void* dst_lo, long long ld_dst, float* lib, const int* cov,
+                   int n_cov, void* stream);
 
 /* batch covariates (n_batch > 1; nn/utils.py:9-13, scvi FCLayers inject_covariates).  spv_one_hot: out[b, 0:nb] = one_hot(code[b]).
  * spv_cov_expand: zzb[b] = [zz[b, 0:P] | oh | zz[b, P:P+S] | oh] (the inputs of the two factor regressors, whose weights are

@@ -42,6 +42,8 @@ _SIGS = {
     "spv_to_f16": [p, ll, p, ll, i, i, p],
     "spv_to_bf16_split": [p, ll, p, p, ll, i, i, p],
     "spv_counts_to_bf16": [i, p, ll, p, p, p, ll, i, i, p, p, i, p],
+    "spv_csr_max_genes": [i],
+    "spv_csr_gather": [i, p, p, p, p, i, i, p, ll, p, p, ll, p, p, i, p],
     "spv_one_hot": [p, p, ll, i, i, p],
     "spv_cov_expand": [p, ll, p, p, ll, p, ll, i, i, i, i, p],
     "spv_cov_compact": [p, ll, p, ll, i, i, i, i, p, ll, p],

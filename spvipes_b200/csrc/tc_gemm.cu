@@ -570,6 +570,174 @@ extern "C" int spv_counts_to_bf16(int src, const void* X, long long ldx, const i
     return SPV_OK;
 }
 
+// Minibatch gather from a device-resident CSR count matrix (int64 row offsets, uint16 column indices) into a dense staging
+// tile xs [B, ld_xs] that every count consumer then reads with rows = NULL.  One CTA per minibatch row: zero a row in dynamic
+// shared memory, scatter the row's nonzeros into it (coalesced loads of indices / values), then write it out with 16-byte
+// stores.  With dst != NULL the same CTA also does what counts_to_bf16_kernel does for a 16-byte aligned dense row (split-bf16
+// pair, covariate columns, library size), with the same per-thread gene assignment, tables and reduction order: its outputs
+// are bit-identical to spv_counts_to_bf16 on the gathered rows.  The CSR must be canonical (no duplicate column in a row).
+#define CSR_SMEM_OPTIN (227 * 1024)  // largest dynamic + static shared memory of one CTA on sm_100
+#define CSR_MAX_G_U16 65536          // range of the uint16 column index; the row takes 128 KB
+#define CSR_MAX_G_F32 ((CSR_SMEM_OPTIN - (int)(ENC_IN_THREADS / 32 * sizeof(float))) / 4 / 4 * 4)  // static: the reduction slots
+template <int SRC>
+__global__ void __launch_bounds__(ENC_IN_THREADS) csr_gather_kernel(const long long* __restrict__ indptr,
+                                                                    const unsigned short* __restrict__ indices,
+                                                                    const void* __restrict__ values, const int* __restrict__ rows,
+                                                                    int G, void* __restrict__ xs, long ld_xs,
+                                                                    __nv_bfloat16* __restrict__ dst, __nv_bfloat16* __restrict__ dst_lo,
+                                                                    long ld_dst, float* __restrict__ lib, const int* __restrict__ cov,
+                                                                    int n_cov) {
+    constexpr bool U16 = SRC == SPV_SRC_U16_LOG1P;
+    constexpr int PER_VEC = U16 ? 8 : 4;  // elements per 16-byte word
+    extern __shared__ uint4 csr_row4[];
+    __shared__ float red[ENC_IN_THREADS / 32];
+    __shared__ float lut[256];          // uint16 instantiation only
+    __shared__ unsigned int lutp[256];
+    const int b = blockIdx.x;
+    const long long r = rows ? (long long)rows[b] : (long long)b;
+    const int nrow4 = (G + PER_VEC - 1) / PER_VEC;  // the row rounded up to whole 16-byte words; ld_xs covers it
+    for (int v = threadIdx.x; v < nrow4; v += ENC_IN_THREADS) csr_row4[v] = make_uint4(0u, 0u, 0u, 0u);
+    if constexpr (U16) {
+        if (dst) {
+            lut[threadIdx.x] = threadIdx.x == 0 ? 0.0f : log1pf((float)threadIdx.x);
+            lutp[threadIdx.x] = pack_split(lut[threadIdx.x]);
+        }
+    }
+    __syncthreads();
+    const long long p0 = __ldg(indptr + r), p1 = __ldg(indptr + r + 1);
+    if constexpr (U16) {
+        unsigned short* srow = reinterpret_cast<unsigned short*>(csr_row4);
+        const unsigned short* val = reinterpret_cast<const unsigned short*>(values);
+        for (long long k = p0 + threadIdx.x; k < p1; k += ENC_IN_THREADS) srow[__ldg(indices + k)] = __ldg(val + k);
+    } else {
+        float* srow = reinterpret_cast<float*>(csr_row4);
+        const float* val = reinterpret_cast<const float*>(values);
+        for (long long k = p0 + threadIdx.x; k < p1; k += ENC_IN_THREADS) srow[__ldg(indices + k)] = __ldg(val + k);
+    }
+    __syncthreads();
+    uint4* xrow4 = reinterpret_cast<uint4*>(reinterpret_cast<char*>(xs) + (long)b * ld_xs * (U16 ? 2 : 4));
+    if (!dst) {
+        for (int v = threadIdx.x; v < nrow4; v += ENC_IN_THREADS) xrow4[v] = csr_row4[v];
+        return;
+    }
+    __nv_bfloat16* out = dst + (long)b * ld_dst;
+    __nv_bfloat16* out_lo = dst_lo ? dst_lo + (long)b * ld_dst : nullptr;
+    const int my_cov = cov ? __ldg(cov + b) : -1;
+    float sum = 0.0f;
+    if constexpr (U16) {
+        // counts_to_bf16_kernel's vectorised path, the row read from shared memory
+        const unsigned short* srow = reinterpret_cast<const unsigned short*>(csr_row4);
+        const int nvec = G / 8;
+        for (int v = threadIdx.x; v < nvec; v += ENC_IN_THREADS) {
+            uint4 raw = csr_row4[v];
+            xrow4[v] = raw;
+            unsigned int w[4] = {raw.x, raw.y, raw.z, raw.w};
+            uint4 o, ol;
+            unsigned int* ow = &o.x;
+            unsigned int* olw = &ol.x;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                unsigned int c0 = w[j] & 0xffffu, c1 = w[j] >> 16;
+                float f0, f1;
+                unsigned int e0, e1;
+                if (c0 < 256u) { f0 = lut[c0]; e0 = lutp[c0]; } else { f0 = log1pf((float)c0); e0 = pack_split(f0); }
+                if (c1 < 256u) { f1 = lut[c1]; e1 = lutp[c1]; } else { f1 = log1pf((float)c1); e1 = pack_split(f1); }
+                sum += f0;
+                sum += f1;
+                ow[j] = __byte_perm(e0, e1, 0x5410);
+                olw[j] = __byte_perm(e0, e1, 0x7632);
+            }
+            *(reinterpret_cast<uint4*>(out) + v) = o;
+            if (out_lo) *(reinterpret_cast<uint4*>(out_lo) + v) = ol;
+        }
+        if (nvec < nrow4 && threadIdx.x == ENC_IN_THREADS - 1) xrow4[nvec] = csr_row4[nvec];  // last partial word (zero padded)
+        for (int g = nvec * 8 + threadIdx.x; g < ld_dst; g += ENC_IN_THREADS) {
+            float f = 0.0f;
+            if (g < G) {
+                unsigned int c = srow[g];
+                f = c < 256u ? lut[c] : log1pf((float)c);
+                sum += f;
+            } else if (g - G < n_cov) {
+                f = (g - G == my_cov) ? 1.0f : 0.0f;
+            }
+            __nv_bfloat16 hi, lo;
+            split_bf16(f, hi, lo);
+            out[g] = hi;
+            if (out_lo) out_lo[g] = lo;
+        }
+    } else {
+        // counts_to_bf16_kernel's scalar float path (load_src<SPV_SRC_F32_LOG1P>)
+        for (int v = threadIdx.x; v < nrow4; v += ENC_IN_THREADS) xrow4[v] = csr_row4[v];
+        const float* srow = reinterpret_cast<const float*>(csr_row4);
+        for (int g = threadIdx.x; g < ld_dst; g += ENC_IN_THREADS) {
+            float f = 0.0f;
+            if (g < G) {
+                const float c = srow[g];
+                f = c == 0.0f ? 0.0f : logf(1.0f + c);
+                sum += f;
+            } else if (g - G < n_cov) {
+                f = (g - G == my_cov) ? 1.0f : 0.0f;
+            }
+            __nv_bfloat16 hi, lo;
+            split_bf16(f, hi, lo);
+            out[g] = hi;
+            if (out_lo) out_lo[g] = lo;
+        }
+    }
+    if (!lib) return;
+    sum = warp_sum(sum);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = sum;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float s = 0.0f;
+#pragma unroll
+        for (int i = 0; i < ENC_IN_THREADS / 32; ++i) s += red[i];
+        lib[b] = logf(s);
+    }
+}
+
+extern "C" int spv_csr_max_genes(int src) {
+    if (src == SPV_SRC_U16_LOG1P) return CSR_MAX_G_U16;
+    if (src == SPV_SRC_F32_LOG1P) return CSR_MAX_G_F32;
+    return SPV_ERR_ARG;
+}
+
+extern "C" int spv_csr_gather(int src, const long long* indptr, const unsigned short* indices, const void* values, const int* rows,
+                              int B, int G, void* xs, long long ld_xs, void* dst, void* dst_lo, long long ld_dst, float* lib,
+                              const int* cov, int n_cov, void* stream) {
+    const int max_g = spv_csr_max_genes(src);
+    if (max_g < 0 || !indptr || !indices || !values || !xs || B <= 0 || G <= 0 || G > max_g || n_cov < 0) return SPV_ERR_ARG;
+    const int per_vec = src == SPV_SRC_U16_LOG1P ? 8 : 4;
+    if (ld_xs < G || (ld_xs % per_vec) || (reinterpret_cast<uintptr_t>(xs) & 15)) return SPV_ERR_ARG;
+    if (dst && (ld_dst < G + n_cov || (ld_dst & 7) || (reinterpret_cast<uintptr_t>(dst) & 15) ||
+                (dst_lo && (reinterpret_cast<uintptr_t>(dst_lo) & 15))))
+        return SPV_ERR_ARG;
+    if (n_cov > 0 && !cov) return SPV_ERR_ARG;
+    if (n_cov == 0) cov = nullptr;
+    static bool done_u16[64] = {}, done_f32[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    bool& done = (src == SPV_SRC_U16_LOG1P ? done_u16 : done_f32)[dev & 63];
+    if (!done) {
+        cudaError_t e = src == SPV_SRC_U16_LOG1P
+            ? cudaFuncSetAttribute(csr_gather_kernel<SPV_SRC_U16_LOG1P>, cudaFuncAttributeMaxDynamicSharedMemorySize, CSR_MAX_G_U16 * 2)
+            : cudaFuncSetAttribute(csr_gather_kernel<SPV_SRC_F32_LOG1P>, cudaFuncAttributeMaxDynamicSharedMemorySize, CSR_MAX_G_F32 * 4);
+        if (e != cudaSuccess) return SPV_ERR_LAUNCH;
+        done = true;
+    }
+    const size_t smem = (size_t)((G + per_vec - 1) / per_vec) * 16;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    __nv_bfloat16* d = reinterpret_cast<__nv_bfloat16*>(dst);
+    __nv_bfloat16* dl = dst ? reinterpret_cast<__nv_bfloat16*>(dst_lo) : nullptr;
+    float* lb = dst ? lib : nullptr;
+    if (src == SPV_SRC_U16_LOG1P)
+        csr_gather_kernel<SPV_SRC_U16_LOG1P><<<B, ENC_IN_THREADS, smem, st>>>(indptr, indices, values, rows, G, xs, ld_xs, d, dl, ld_dst, lb, cov, n_cov);
+    else
+        csr_gather_kernel<SPV_SRC_F32_LOG1P><<<B, ENC_IN_THREADS, smem, st>>>(indptr, indices, values, rows, G, xs, ld_xs, d, dl, ld_dst, lb, cov, n_cov);
+    SPV_CHECK_LAUNCH();
+    return SPV_OK;
+}
+
 // =======================================================================================================================
 // Encoder first layer with the count transform fused into the GEMM's operand path (BASELINE.json north_star: "a tcgen05/TMEM GEMM
 // fed by TMA that consumes raw counts and fuses log1p into its prologue"; reference module/spVIPESmodule.py:428-433 +

@@ -169,10 +169,66 @@ class FlatStore:
 
 
 # ------------------------------------------------------------------------------------------------
+def _count_dtype(values) -> "np.dtype":
+    """uint16 when every value is an integer in [0, 65535], float32 otherwise (the rule of the dense model path)"""
+    import numpy as np
+    v = np.asarray(values)
+    if v.size == 0:
+        return np.dtype(np.uint16)
+    if v.dtype.kind in "ui":
+        return np.dtype(np.uint16) if v.min() >= 0 and v.max() <= 65535 else np.dtype(np.float32)
+    return np.dtype(np.uint16) if np.all(v == np.round(v)) and v.min() >= 0 and v.max() <= 65535 else np.dtype(np.float32)
+
+
+@dataclass
+class CsrCounts:
+    """one group's count matrix [N, G] as device-resident CSR: a minibatch is gathered into a dense staging tile by
+    spv_csr_gather, so the matrix itself takes 4 bytes per nonzero (uint16 values) instead of 2 G bytes per row.
+    Canonical: every row's columns sorted and distinct, no stored zeros."""
+    indptr: torch.Tensor    # int64 [N + 1]
+    indices: torch.Tensor   # uint16 [nnz] column indices
+    values: torch.Tensor    # uint16 or float32 [nnz]
+    shape: Tuple[int, int]
+
+    @property
+    def dtype(self):
+        return self.values.dtype
+
+    @staticmethod
+    def canonical_arrays(mat):
+        """host side of from_scipy: (indptr int64, indices uint16, values uint16 | float32, shape) of a scipy sparse matrix, with
+        duplicate entries summed (scipy's meaning of them), explicit zeros dropped and the columns of every row sorted"""
+        import numpy as np
+        import scipy.sparse as sp
+        m = sp.csr_matrix(mat, copy=True)
+        m.sum_duplicates()  # also sorts the indices
+        m.eliminate_zeros()
+        N, G = (int(x) for x in m.shape)
+        data = m.data
+        if data.dtype.kind == "f" and data.dtype != np.float32:
+            data = data.astype(np.float32)  # the dtype rule looks at the values the kernels will see
+        dt = _count_dtype(data)
+        limit = int(L.load().spv_csr_max_genes(L.SRC_U16_LOG1P if dt == np.uint16 else L.SRC_F32_LOG1P))
+        if G > limit:
+            raise ValueError(f"a CSR count matrix with {dt.name} values holds at most {limit} genes (a row is assembled in "
+                             f"shared memory), got {G}")
+        return (m.indptr.astype(np.int64), m.indices.astype(np.uint16), data.astype(dt), (N, G))
+
+    @classmethod
+    def from_scipy(cls, mat, device="cuda") -> "CsrCounts":
+        indptr, indices, values, shape = cls.canonical_arrays(mat)
+        up = lambda a: torch.from_numpy(a).to(device)
+        return cls(up(indptr), up(indices), up(values), shape)
+
+    def resident_bytes(self) -> int:
+        return sum(t.numel() * t.element_size() for t in (self.indptr, self.indices, self.values))
+
+
 @dataclass
 class GroupBatch:
     """one group's minibatch: a device-resident count matrix plus optional row-gather indices"""
-    X: torch.Tensor                       # [N, ld] uint16 or float32 counts (device); columns col0 .. col0+G are this group's genes
+    X: object                             # [N, ld] uint16 or float32 counts (device tensor); columns col0 .. col0+G are this group's
+                                          # genes; or a CsrCounts of the group's own genes (col0 = 0)
     rows: Optional[torch.Tensor] = None   # int32 [B] row indices into X, or None for X[:B]
     col0: int = 0
     labels: Optional[torch.Tensor] = None  # int32 [B] cell-type labels (label mode) or cluster labels (cluster mode)
@@ -184,7 +240,7 @@ class GroupBatch:
     def batch_size(self):
         if self.B is not None:
             return self.B
-        return int(self.rows.shape[0]) if self.rows is not None else int(self.X.shape[0])
+        return int(self.rows.shape[0]) if self.rows is not None else int(self.X.shape[0])  # (a CsrCounts has .shape too)
 
 
 @dataclass
@@ -325,6 +381,16 @@ def _need_tb(self, dev):
 
 
 _GroupWS.need_tb = _need_tb
+
+
+def _need_xs(self, dtype, dev):
+    """dense staging tile [B, Gp] of a CSR minibatch (spv_csr_gather): what every count consumer reads with rows = NULL"""
+    if getattr(self, "xs", None) is None or self.xs.dtype != dtype:
+        self.xs = torch.zeros(self.B, self.Gp, dtype=dtype, device=dev)
+    return self.xs
+
+
+_GroupWS.need_xs = _need_xs
 
 
 class StepEngine:
@@ -596,14 +662,32 @@ class StepEngine:
             bt, w, st = batches[g], ws[g], self._stream()
             G, B = d.genes[g], Bs[g]
             src, esz = self._src_of(bt.X)
-            if bt.X.dim() != 2 or bt.X.stride(1) != 1:
-                raise ValueError("the count matrix must be row-major (unit stride along the genes)")
-            ldx = bt.X.stride(0)
-            xptr = bt.X.data_ptr() + bt.col0 * esz
-            srcs.append((src, xptr, ldx))
             nb, Gc = d.nb, G + d.nb
             if nb and bt.batch is None:
                 raise ValueError("batch codes are required when the model was built with n_batch > 1")
+            fused1 = self.bf16 and self.fused_fc1 and src == L.SRC_U16_LOG1P
+            # (src, xptr, ldx, count_rows): where every consumer of the counts reads this minibatch
+            if isinstance(bt.X, CsrCounts):
+                if bt.col0 != 0 or bt.X.shape[1] != G:
+                    raise ValueError(f"a CSR count matrix holds exactly the group's own {G} genes (col0 = 0), got shape "
+                                     f"{bt.X.shape} and col0 = {bt.col0}")
+                # gather the minibatch into the dense staging tile; in the default bf16 mode the same launch writes the encoder's
+                # split-bf16 input and the library size (what spv_counts_to_bf16 does on dense rows)
+                xs = w.need_xs(bt.X.dtype, self.device)
+                conv = self.bf16 and not fused1
+                if conv:
+                    w.need_tb(self.device)
+                L.check(lib.spv_csr_gather(src, L.ptr(bt.X.indptr), L.ptr(bt.X.indices), L.ptr(bt.X.values), L.ptr(bt.rows), B, G,
+                                           L.ptr(xs), w.Gp, L.ptr(w.Tb) if conv else None, L.ptr(w.Tb_lo) if conv else None, w.Gpe,
+                                           L.ptr(w.lib) if conv else None, L.ptr(bt.batch) if (conv and nb) else None,
+                                           nb if conv else 0, st), "spv_csr_gather")
+                xptr, ldx, count_rows = L.ptr(xs), w.Gp, None
+            else:
+                if bt.X.dim() != 2 or bt.X.stride(1) != 1:
+                    raise ValueError("the count matrix must be row-major (unit stride along the genes)")
+                conv = False
+                xptr, ldx, count_rows = bt.X.data_ptr() + bt.col0 * esz, bt.X.stride(0), bt.rows
+            srcs.append((src, xptr, ldx, count_rows))
             if convert:  # bf16 copies of the two big weights do not depend on the minibatch: off the critical path
                 with self._branch(g, "w1"):
                     L.check(lib.spv_to_bf16_split(L.ptr(self.P(g, "W1")), Gc, L.ptr(w.W1b), L.ptr(w.W1b_lo), w.Gpe, 2 * H, Gc,
@@ -611,39 +695,39 @@ class StepEngine:
                 if decode or self.stage_in_adam:
                     with self._branch(g, "wm"):
                         self._to_dec(L.ptr(self.P(g, "Wm")), KMIX, L.ptr(w.Wmb), w.KMp, G, KMIX)
-            fused1 = self.bf16 and self.fused_fc1 and src == L.SRC_U16_LOG1P
             if fused1:
                 # first layer straight from the raw counts: the producer warps of the GEMM gather the rows, look log1p up as a
                 # split-bf16 pair and write the tensor-core operand tiles (spv_enc_fc1_fwd); the library size on the side
                 with self._branch(g, "lib"):
-                    L.check(lib.spv_library_size(src, xptr, ldx, L.ptr(bt.rows), B, G, L.ptr(w.lib), self._stream()),
+                    L.check(lib.spv_library_size(src, xptr, ldx, L.ptr(count_rows), B, G, L.ptr(w.lib), self._stream()),
                             "spv_library_size")
                 if nb:  # covariate term + bias as a pre-activation addend
                     L.check(lib.spv_one_hot(L.ptr(bt.batch), L.ptr(w.oh), nb, B, nb, st), "spv_one_hot")
                     self._gemm(L.ptr(w.oh), self.P(g, "W1").data_ptr() + 4 * G, L.ptr(w.h1), B, 2 * H, nb, lda=nb, ldb=Gc, ldc=2 * H,
                                tb=1, bias=L.ptr(self.P(g, "b1")))
                 self._join(g, "w1")
-                L.check(lib.spv_enc_fc1_fwd(xptr, ldx, L.ptr(bt.rows), L.ptr(w.W1b), L.ptr(w.W1b_lo), w.Gpe, L.ptr(w.h1), 2 * H, B,
+                L.check(lib.spv_enc_fc1_fwd(xptr, ldx, L.ptr(count_rows), L.ptr(w.W1b), L.ptr(w.W1b_lo), w.Gpe, L.ptr(w.h1), 2 * H, B,
                                             2 * H, G, None if nb else L.ptr(self.P(g, "b1")), 1, 1 if nb else 0, w.tc_splits_fc1,
                                             L.ptr(w.ws), st), "spv_enc_fc1_fwd")
             elif self.bf16:  # encoder input and library size from one pass over the gathered rows
                 # (with batch covariates: their one-hot columns behind the genes, so that fc1 stays one GEMM over K = G + nb)
-                w.need_tb(self.device)
-                L.check(lib.spv_counts_to_bf16(src, xptr, ldx, L.ptr(bt.rows), L.ptr(w.Tb), L.ptr(w.Tb_lo), w.Gpe, B, G,
-                                               L.ptr(w.lib), L.ptr(bt.batch) if nb else None, nb, st), "spv_counts_to_bf16")
+                if not conv:  # (a CSR minibatch was converted by its gather)
+                    w.need_tb(self.device)
+                    L.check(lib.spv_counts_to_bf16(src, xptr, ldx, L.ptr(count_rows), L.ptr(w.Tb), L.ptr(w.Tb_lo), w.Gpe, B, G,
+                                                   L.ptr(w.lib), L.ptr(bt.batch) if nb else None, nb, st), "spv_counts_to_bf16")
                 self._join(g, "w1")
                 self._tc_gemm_split(L.ptr(w.Tb), L.ptr(w.Tb_lo), L.ptr(w.W1b), L.ptr(w.W1b_lo), L.ptr(w.h1), B, 2 * H, Gc, lda=w.Gpe,
                                     ldb=w.Gpe, ldc=2 * H, bias=L.ptr(self.P(g, "b1")), relu=1, splits=w.tc_splits_fc1, ws=w.ws)
             else:
                 with self._branch(g, "lib"):
-                    L.check(lib.spv_library_size(src, xptr, ldx, L.ptr(bt.rows), B, G, L.ptr(w.lib), self._stream()),
+                    L.check(lib.spv_library_size(src, xptr, ldx, L.ptr(count_rows), B, G, L.ptr(w.lib), self._stream()),
                             "spv_library_size")
                 if nb:  # covariate term + bias first (pre-activation), then the count GEMM adds to it and applies the ReLU
                     L.check(lib.spv_one_hot(L.ptr(bt.batch), L.ptr(w.oh), nb, B, nb, st), "spv_one_hot")
                     self._gemm(L.ptr(w.oh), self.P(g, "W1").data_ptr() + 4 * G, L.ptr(w.h1), B, 2 * H, nb, lda=nb, ldb=Gc, ldc=2 * H,
                                tb=1, bias=L.ptr(self.P(g, "b1")))
                 self._gemm(xptr, L.ptr(self.P(g, "W1")), L.ptr(w.h1), B, 2 * H, G, lda=ldx, ldb=Gc, ldc=2 * H, tb=1, srcA=src,
-                           rowsA=bt.rows, bias=None if nb else L.ptr(self.P(g, "b1")), relu=1, acc=2 if nb else 0,
+                           rowsA=count_rows, bias=None if nb else L.ptr(self.P(g, "b1")), relu=1, acc=2 if nb else 0,
                            splits=w.splits_fc1, ws=w.ws)
             mask = noise.drop[g] if (training and noise.drop is not None) else None
             dropping = training and (mask is not None or self.dropout_rate > 0)
@@ -692,7 +776,7 @@ class StepEngine:
         for g in self._fork_groups():
             bt, w, st = batches[g], ws[g], self._stream()
             G, B = d.genes[g], Bs[g]
-            src, xptr, ldx = srcs[g]
+            src, xptr, ldx, count_rows = srcs[g]
             if self.bf16 and not ctx["wm_staged"]:  # decode() after an encoder-only pass: the mixture weight's bf16 copy
                 self._to_dec(L.ptr(self.P(g, "Wm")), KMIX, L.ptr(w.Wmb), w.KMp, G, KMIX)
             zzp = w.amix.data_ptr() + 4 * HD
@@ -730,7 +814,7 @@ class StepEngine:
                 self._join(g, "hm")
             else:
                 self._hidden_mix(g, w, B, tr, zzp)
-            dptrs = self._dec_ptrs(g, w, xptr, bt.rows, with_grad)
+            dptrs = self._dec_ptrs(g, w, xptr, count_rows, with_grad)
             self._join(g, "lib")
             if not self.fused_nb:
                 L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
@@ -891,7 +975,7 @@ class StepEngine:
         for g in self._fork_groups():
             bt, w, st = batches[g], ws[g], self._stream()
             G, B = d.genes[g], Bs[g]
-            src, xptr, ldx = srcs[g]
+            src, xptr, ldx, count_rows = srcs[g]
             zzp = w.amix.data_ptr() + 4 * HD
             nb, Pb, Sb, KZb = d.nb, d.Pb, d.Sb, d.KZb
             zb, ld_zb = (L.ptr(w.zzb), KZb) if nb else (zzp, KMIX)
@@ -925,7 +1009,7 @@ class StepEngine:
                 evs = next(self.nb_bwd_events) if self.nb_bwd_events is not None else None
                 if evs is not None:
                     evs[0].record()
-                L.check(lib.spv_dec_nb_bwd_tc(src, self._dec_ptrs(g, w, xptr, bt.rows, True), ldx, L.ptr(w.amixb), w.KMp,
+                L.check(lib.spv_dec_nb_bwd_tc(src, self._dec_ptrs(g, w, xptr, count_rows, True), ldx, L.ptr(w.amixb), w.KMp,
                                               L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb), L.ptr(w.wzf), L.ptr(w.D3), w.Bp, B, G, HD, Pb, Sb,
                                               -float(grad_scale) / B, L.ptr(w.colsum), KMIX, st), "spv_dec_nb_bwd_tc")
                 if evs is not None:
@@ -955,7 +1039,7 @@ class StepEngine:
                 self._tc_gemm(L.ptr(w.D3), L.ptr(w.Wstack), L.ptr(w.damix), B, KMIX, G, lda=Bp, ldb=w.KMp, ldc=KMIX, a_mn=1, b_mn=1,
                               splits=w.tc_splits_damix, ws=w.ws, fmt=f3, alpha=al)
             else:
-                L.check(lib.spv_dec_nb_bwd(src, self._dec_ptrs(g, w, xptr, bt.rows, True), ldx, KMIX, B, G, HD, Pb, Sb,
+                L.check(lib.spv_dec_nb_bwd(src, self._dec_ptrs(g, w, xptr, count_rows, True), ldx, KMIX, B, G, HD, Pb, Sb,
                                            -float(grad_scale) / B, L.ptr(w.colsum), L.ptr(w.dpib) if self.bf16 else None,
                                            3 * w.Gp if self.bf16 else 0, L.ptr(w.zzb) if nb else None, KZb, KMIX, st),
                         "spv_dec_nb_bwd")
@@ -1047,7 +1131,7 @@ class StepEngine:
         for g in self._fork_groups():
             bt, w, st = batches[g], ws[g], self._stream()
             G, B = d.genes[g], Bs[g]
-            src, xptr, ldx = srcs[g]
+            src, xptr, ldx, count_rows = srcs[g]
             L.check(lib.spv_bn_bwd(L.ptr(w.dstats), NST, L.ptr(w.r), NST, None, 0, L.ptr(w.dr), NST, B, NST,
                                    L.ptr(self.P(g, "ghd")), L.ptr(w.bn_hd_mean), L.ptr(w.bn_hd_istd), L.ptr(self.Gd(g, "ghd")),
                                    L.ptr(self.Gd(g, "bthd")), st), "spv_bn_bwd")
@@ -1104,7 +1188,7 @@ class StepEngine:
                     L.check(lib.spv_to_bf16_split(L.ptr(w.dh1), 2 * H, L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H, B, 2 * H, st),
                             "spv_to_bf16_split")
                 if self.fused_fc1 and src == L.SRC_U16_LOG1P:  # counts transformed in the GEMM's producer warps (as the forward)
-                    L.check(lib.spv_enc_fc1_dw(xptr, ldx, L.ptr(bt.rows), L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H,
+                    L.check(lib.spv_enc_fc1_dw(xptr, ldx, L.ptr(count_rows), L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H,
                                                L.ptr(self.Gd(g, "W1")), G + d.nb, B, 2 * H, G, st), "spv_enc_fc1_dw")
                     if d.nb:  # covariate columns of the first layer's weight: dh1^T one_hot
                         self._gemm(L.ptr(w.dh1), L.ptr(w.oh), self.Gd(g, "W1").data_ptr() + 4 * G, 2 * H, d.nb, B, lda=2 * H,
@@ -1114,7 +1198,7 @@ class StepEngine:
                                         G + d.nb, B, lda=2 * H, ldb=w.Gpe, ldc=G + d.nb, a_mn=1, b_mn=1)
             else:
                 self._gemm(L.ptr(w.dh1), xptr, L.ptr(self.Gd(g, "W1")), 2 * H, G, B, lda=2 * H, ldb=ldx, ldc=G + d.nb, ta=1, srcB=src,
-                           rowsB=bt.rows)
+                           rowsB=count_rows)
                 if d.nb:  # covariate columns of the first layer's weight: dh1^T one_hot
                     self._gemm(L.ptr(w.dh1), L.ptr(w.oh), self.Gd(g, "W1").data_ptr() + 4 * G, 2 * H, d.nb, B, lda=2 * H, ldb=d.nb,
                                ldc=G + d.nb, ta=1)

@@ -5,8 +5,9 @@ model/base/training_mixin.py:19-123, data/prepare_adatas.py:7-134).
 
 anndata / scvi-tools / lightning are not dependencies of this package: any object with `.X` (scipy sparse or ndarray),
 `.obs` (pandas DataFrame), `.var_names`, `.obs_names` and `.uns` (dict) works, a real AnnData included; `GroupedData` is the
-minimal stand-in.  What differs from the reference is WHERE things run: the count matrices live on the GPU as uint16, a
-minibatch is a list of row indices gathered inside the kernels (no per-step CSR densification / host->device copy), the step
+minimal stand-in.  What differs from the reference is WHERE things run: the count matrices live on the GPU as uint16 (or as
+CSR when `.X` is scipy-sparse), a minibatch is a list of row indices gathered on the device (no per-step host-side
+densification / host->device copy), the step
 is one CUDA-graph replay, and the optimiser is the fused Adam kernel with the scvi TrainingPlan defaults
 (lr 1e-3, eps 0.01, weight_decay 1e-6, KL warm-up over n_epochs_kl_warmup epochs).
 """
@@ -21,7 +22,7 @@ import numpy as np
 import pandas as pd
 import torch
 
-from .engine import GroupBatch
+from .engine import CsrCounts, GroupBatch
 from .module import spVIPESmodule
 from .trainer import TrainLoop, epoch_batches, split_indices
 
@@ -52,12 +53,22 @@ def _dense(X):
     return np.asarray(X.todense()) if hasattr(X, "todense") else np.asarray(X)
 
 
+def _is_sparse(X):
+    return hasattr(X, "tocsr")
+
+
 def prepare_adatas(adatas: Dict[str, object], layers: Optional[Sequence[Optional[str]]] = None) -> GroupedData:
     """concatenate two groups on the obs axis with an OUTER join on genes prefixed by their group key, and record the
-    per-group obs / var index lists in `.uns` (reference data/prepare_adatas.py:94-132)."""
+    per-group obs / var index lists in `.uns` (reference data/prepare_adatas.py:94-132).
+
+    The joined `.X` is a dense float32 array when every input `.X` is dense.  When any input `.X` is scipy-sparse it is a
+    float32 scipy CSR matrix (the group blocks stacked with empty blocks for the other group's genes, as the reference's
+    anndata concat keeps it): the dense join of two 1 M-cell x 20 k-gene groups would take 320 GB of host memory.
+    `spVIPES` then keeps each group's counts as CSR on the GPU as well."""
     if len(adatas) != 2:
         raise ValueError("spVIPES currently supports exactly 2 groups")
     keys = list(adatas.keys())
+    sparse = any(_is_sparse(a.X) for a in adatas.values())
     blocks, obs_frames, var_names, lengths = [], [], [], {}
     groups_obs_names, groups_var_names, groups_obs_indices, groups_var_indices = [], {}, [], []
     col0 = row0 = 0
@@ -67,9 +78,15 @@ def prepare_adatas(adatas: Dict[str, object], layers: Optional[Sequence[Optional
         n, G = a.X.shape
         vn = [f"{k}_{v}" for v in a.var_names]
         var_names += vn
-        full = np.zeros((n, total_genes), dtype=np.float32)  # the other group's genes are absent: zero fill of the outer join
-        full[:, col0:col0 + G] = _dense(a.X)
-        blocks.append(full)
+        if sparse:
+            import scipy.sparse as sp
+            own = sp.csr_matrix(a.X, dtype=np.float32)
+            parts = [sp.csr_matrix((n, col0), dtype=np.float32), own, sp.csr_matrix((n, total_genes - col0 - G), dtype=np.float32)]
+            blocks.append(sp.hstack(parts, format="csr"))
+        else:
+            full = np.zeros((n, total_genes), dtype=np.float32)  # the other group's genes are absent: zero fill of the outer join
+            full[:, col0:col0 + G] = _dense(a.X)
+            blocks.append(full)
         obs = a.obs.copy()
         obs["groups"] = k
         obs["indices"] = np.arange(n)  # within-group position (reference :94-97)
@@ -84,7 +101,12 @@ def prepare_adatas(adatas: Dict[str, object], layers: Optional[Sequence[Optional
     obs = pd.concat(obs_frames, ignore_index=True)
     uns = {"groups_lengths": lengths, "groups_obs_names": groups_obs_names, "groups_var_names": groups_var_names,
            "groups_obs_indices": groups_obs_indices, "groups_var_indices": groups_var_indices, "groups_mapping": dict(enumerate(keys))}
-    return GroupedData(X=np.concatenate(blocks, 0), obs=obs, var_names=var_names, uns=uns)
+    if sparse:
+        import scipy.sparse as sp
+        X = sp.vstack(blocks, format="csr")
+    else:
+        X = np.concatenate(blocks, 0)
+    return GroupedData(X=X, obs=obs, var_names=var_names, uns=uns)
 
 
 class spVIPES:
@@ -154,19 +176,27 @@ class spVIPES:
 
     # ------------------------------------------------------------------ device-resident data
     def _to_device(self):
-        """per group: uint16 [N_g, G_g] counts of the group's own genes (float32 if the data are not small integers)"""
+        """per group: uint16 [N_g, G_g] counts of the group's own genes (float32 if the data are not small integers); a
+        scipy-sparse `adata.X` stays sparse: each group becomes a CSR matrix on the GPU (engine.CsrCounts)"""
         if self._device_data is not None:
             return self._device_data
         dev = self.module.device
         uns = self.adata.uns
         X = self.adata.X
+        Xcsr = X.tocsr() if _is_sparse(X) else None
         data = []
         for g in (0, 1):
             rows, cols = np.asarray(uns["groups_obs_indices"][g]), np.asarray(uns["groups_var_indices"][g])
-            blk = _dense(X[rows][:, cols]) if not hasattr(X, "tocsr") else _dense(X.tocsr()[rows][:, cols])
-            integral = np.all(blk == np.round(blk)) and blk.min() >= 0 and blk.max() <= 65535
-            # (numpy's column selection hands back a Fortran-ordered block: make it row-major, the kernels read rows)
-            t = torch.from_numpy(np.ascontiguousarray(blk.astype(np.uint16 if integral else np.float32)))
+            if Xcsr is not None:
+                # the group's rows and its column range (contiguous as prepare_adatas lays it out: a sparse slice)
+                contiguous = len(cols) > 0 and np.array_equal(cols, np.arange(cols[0], cols[0] + len(cols)))
+                sel = slice(int(cols[0]), int(cols[0]) + len(cols)) if contiguous else cols
+                t = CsrCounts.from_scipy(Xcsr[rows][:, sel], dev)
+            else:
+                blk = _dense(X[rows][:, cols])
+                integral = np.all(blk == np.round(blk)) and blk.min() >= 0 and blk.max() <= 65535
+                # (numpy's column selection hands back a Fortran-ordered block: make it row-major, the kernels read rows)
+                t = torch.from_numpy(np.ascontiguousarray(blk.astype(np.uint16 if integral else np.float32))).to(dev)
             labels = None
             if self._label_codes is not None:
                 labels = torch.from_numpy(self._label_codes[rows].astype(np.int32)).to(dev)
@@ -174,7 +204,7 @@ class spVIPES:
             batch = None
             if self.module.engine.d.nb:
                 batch = torch.from_numpy(self._batch_codes[rows].astype(np.int32)).to(dev)
-            data.append({"X": t.to(dev), "labels": labels, "idx": idx, "row0": int(rows[0]), "rows": rows, "batch": batch})
+            data.append({"X": t, "labels": labels, "idx": idx, "row0": int(rows[0]), "rows": rows, "batch": batch})
         self._device_data = data
         return data
 
