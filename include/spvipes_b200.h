@@ -68,21 +68,6 @@ int spv_gemm_fused(int srcA, int transA, int srcB, int transB, const void* A, lo
                    unsigned int drop_stream, const int* drop_step, long long drop_ld, void* c_bf16, void* c_bf16_lo,
                    long long ld_cbf16, void* stream);
 
-/* Middle of the two encoders of a group in one launch per direction (nn/networks.py:119-125):
- *   forward : h2 = dropout(relu(h1 W2^T + b2)) [B, 2H], r = h2 Whead^T + bhead [B, 2P + 2S]   (blocks: private | shared)
- *   backward: dh2 = (dr Whead) * gate(h2, dropout), dh1 = (dh2 W2) * gate(h1); dh1_bf16 optional (operand of the dW1 GEMM)
- * W2 [2H, H], Whp [2P, H], Whs [2S, H], bhd [2P + 2S].  Dropout: explicit multiplier matrix drop_mask or Philox
- * (seed, stream id, *step, index m * 2H + column) as spv_dropout; backward multiplier drop_mask or drop_scale.
- * Needs H <= 128, H % 4 == 0, 2P, 2S <= 128 (spv_enc_mid_supported), 16-byte aligned rows. */
-int spv_enc_mid_supported(int H, int P, int S);
-int spv_enc_mid_fwd(const float* h1, long long ld_h1, const float* W2, const float* b2, const float* Whp, const float* Whs,
-                    const float* bhd, float* h2, long long ld_h2, float* r, long long ld_r, const float* drop_mask,
-                    long long ld_mask, float drop_p, unsigned long long seed, unsigned int stream_id, const int* step, int B,
-                    int H, int P, int S, void* stream);
-int spv_enc_mid_bwd(const float* dr, long long ld_dr, const float* Whp, const float* Whs, const float* W2, const float* h2,
-                    long long ld_h2, const float* h1, long long ld_h1, const float* drop_mask, long long ld_mask,
-                    float drop_scale, float* dh2, long long ld_dh2, float* dh1, long long ld_dh1, void* dh1_bf16,
-                    long long ld_dh1b, int B, int H, int P, int S, void* stream);
 /* bf16 tensor-core GEMM (tcgen05.mma, TMEM accumulator, TMA-fed): C[M,N] (+)= act(A B^T + bias), fp32 output.
  * a_mn = 0: A stored [M][K], 1: A stored [K][M];  b_mn = 0: B stored [N][K], 1: B stored [K][N]; lda / ldb in bf16
  * elements, multiples of 8, bases 16-byte aligned.  Same call sites as spv_gemm, for the "bf16 tensor-core path". */
@@ -215,7 +200,8 @@ int spv_loss(const float* rec0, const float* rec1, const float* klp0, const floa
 int spv_dec_fold(const void* const* ptrs, long long ld_zz, int B, int G, int P, int S, int training, float eps, float momentum,
                  void* wz_bf16, long long ld_wz, int Gp, int HD, void* wz_f16, void* zc_f16, void* stream);
 /* fused decoder + NB-mixture likelihood sweeps.  ptrs (SPV_DEC_NPTR): X, rows, amix, wfold, wm, bm, genec, lib, part_stats,
- * rowc, pi, part_nb, dyp, dys, dpi, colpart, rec, tgf, tgb (the last two: spv_dec_theta_tables, tensor-core sweeps only).
+ * rowc, pi, part_nb, dyp, dys, dpi, colpart, rec, tgf, tb1 (the last two: spv_dec_theta_tables, tensor-core sweeps only;
+ * tb1 only for the training sweep).
  * nn/networks.py:314-325; module/spVIPESmodule.py:759, 817-824 */
 #define SPV_DEC_NPTR 19
 /* phases: bit 0 = gene-axis softmax normaliser sweep, bit 1 = mixture GEMM + NB log-likelihood sweep (3 = both),
@@ -242,26 +228,16 @@ int spv_dec_nb_fwd_tc(int src, const void* const* ptrs, long long ldx, const voi
  * nn/networks.py:318-320, module/spVIPESmodule.py:751-757 */
 int spv_dec_stats_tc(void* zc_f16, const void* wz_f16, int Gp, const float* genec, const float* lib, float* part_stats,
                      float* rowc, int B, int G, int P, int S, void* stream);
-/* count tables of the tensor-core likelihood sweeps (csrc/decoder_common.cuh NB_TAB = 16 entries per gene, float2 each):
- * tgf[g][c] = (log1p(c), lgamma(log1p(c) + theta_g) - lgamma(theta_g) - lgamma(log1p(c) + 1)), tgb[g][c] = (log1p(c),
- * digamma(log1p(c) + theta_g) - digamma(theta_g)), theta = exp(px_r) (module/spVIPESmodule.py:758).  They depend on the
- * parameter only; any of the pointers may be NULL.  tb1 [G, 16] floats: the digamma terms alone (training sweep).  16-byte
- * aligned. */
-int spv_dec_theta_tables(const float* px_r, int G, void* tgf, void* tgb, float* tb1, void* stream);
+/* count tables of the tensor-core likelihood sweeps (csrc/decoder_common.cuh NB_TAB = 16 entries per gene):
+ * tgf [G, 16] float2: tgf[g][c] = (log1p(c), lgamma(log1p(c) + theta_g) - lgamma(theta_g) - lgamma(log1p(c) + 1)),
+ * tb1 [G, 16] float: tb1[g][c] = digamma(log1p(c) + theta_g) - digamma(theta_g) (training sweep), theta = exp(px_r)
+ * (module/spVIPESmodule.py:758).  They depend on the parameter only; either pointer may be NULL.  16-byte aligned. */
+int spv_dec_theta_tables(const float* px_r, int G, void* tgf, float* tb1, void* stream);
 /* floats spv_dec_nb_fwd_tc needs in part_nb (ptrs[11]) for a [B, G] problem */
 long long spv_dec_nb_part_floats(int B, int G);
 /* rec[b] (ptrs[16] of the forward) and the softmax-backward row sums rowc[:, 2:4] from the row partials part_nb that
  * spv_dec_nb_fwd_tc wrote for the same B, G, HD */
 int spv_dec_nb_rowreduce(const float* part_nb, int G, int B, int HD, float* rowc, float* rec, void* stream);
-/* tensor-core backward sweep: recomputes the three logit tiles on tcgen05 and writes D3T = [dpi ; dyp ; dys] / scale (FP16,
- * GENE-major [3 Gp, ld_d3], ld_d3 >= B a multiple of 8: a warp's 32 cells are contiguous, so the stores coalesce; operand of
- * the gradient GEMMs, which apply the signed scale as spv_tc_gemm_ex's alpha) and colsum [4, G] (column sums of dyp, dys, dpi,
- * d loss / d theta, true scale);
- * ptrs[15] = colpart workspace [ceil(B/128), 4, G].  scale = - grad_scale / B.  rowc (ptrs[9], [B, 4] floats) must be
- * 16-byte aligned (SPV_ERR_ARG otherwise): a row is read as one float4. */
-int spv_dec_nb_bwd_tc(int src, const void* const* ptrs, long long ldx, const void* amix_bf16, long long ld_amixb,
-                      const void* wstack_bf16, long long ld_w, int Gp, const void* zc_f16, const void* wz_f16, void* d3_f16,
-                      long long ld_d3, int B, int G, int HD, int P, int S, float scale, float* colsum, int kmix, void* stream);
 /* ptrs (18): Wp, Ws, Qp, Qs, genec, colsum, zmean, zcov, dWp, dWs, dgamma_p, dbeta_p, dgamma_s, dbeta_s, dpx_r, dbm,
  * vpart [parts, P+S], mpart [parts, (P+S)^2] with parts = spv_dec_gene_bwd_parts(G)
  * (backward of nn/networks.py:314-320 through the folded BatchNorm) */

@@ -29,9 +29,6 @@ _SIGS = {
     "spv_arch_check": [i],
     "spv_copy2d_h2d": [p, ll, p, ll, ll, ll, p],
     "spv_gemm": [i, i, i, i, p, ll, p, p, ll, p, p, ll, i, i, i, i, ll, ll, ll, p, ll, i, i, i, p, p],
-    "spv_enc_mid_supported": [i, i, i],
-    "spv_enc_mid_fwd": [p, ll, p, p, p, p, p, p, ll, p, ll, p, ll, f, u64, u32, p, i, i, i, i, p],
-    "spv_enc_mid_bwd": [p, ll, p, p, p, p, ll, p, ll, p, ll, f, p, ll, p, ll, p, ll, i, i, i, i, p],
     "spv_gemm_fused": [i, i, i, i, p, ll, p, p, ll, p, p, ll, i, i, i, i, ll, ll, ll, p, ll, i, i, i, p, p, ll, p, ll, f, f, p, u64, u32, p, ll, p, p, ll, p],
     "spv_tc_gemm": [i, i, p, ll, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
     "spv_tc_gemm_ex": [i, f, i, i, p, ll, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
@@ -66,12 +63,11 @@ _SIGS = {
     "spv_dec_nb_bwd": [i, p, ll, ll, i, i, i, i, i, f, p, p, ll, p, ll, i, p],
     "spv_dec_nb_fwd_tc": [i, p, ll, p, ll, p, ll, i, p, p, i, i, i, i, i, i, i, p],
     "spv_dec_nb_rowreduce": [p, i, i, i, p, p, p],
-    "spv_dec_nb_bwd_tc": [i, p, ll, p, ll, p, ll, i, p, p, p, ll, i, i, i, i, i, f, p, i, p],
     "spv_dec_gene_bwd": [p, ll, i, i, i, i, i, p],
     "spv_dec_gene_bwd_parts": [i],
     "spv_dec_nb_part_floats": [i, i],
     "spv_dec_stats_tc": [p, p, i, p, p, p, p, i, i, i, i, p],
-    "spv_dec_theta_tables": [p, i, p, p, p, p],
+    "spv_dec_theta_tables": [p, i, p, p, p],
     "spv_dec_nb_train_tc": [i, p, ll, p, ll, p, ll, i, p, p, p, ll, p, ll, i, i, i, i, i, i, p],
     "spv_dec_nb_train_colsum": [p, i, i, f, p, p],
     "spv_dec_zq4": [p, ll, p, p, ll, i, i, i, p],

@@ -45,6 +45,6 @@ enum {
 
 // Per-gene count tables (spv_dec_theta_tables): for raw counts c < NB_TAB, t = log1p(c) and
 //   forward  tgf[g][c] = (t, lgamma(t + theta) - lgamma(theta) - lgamma(t + 1))
-//   backward tgb[g][c] = (t, digamma(t + theta) - digamma(theta))
+//   backward tb1[g][c] = digamma(t + theta) - digamma(theta)
 // (both 0 at c = 0).  Larger or non-integer counts take an out-of-line path that evaluates the same terms directly.
 #define NB_TAB 16

@@ -226,7 +226,7 @@ struct FoldP {
     long ld_wz;
     int Gp, HD;
     int stack_f16;  // the stacked operand holds fp16 (the fused tensor-core decoder) instead of bf16 values
-    // optional fp16 operands of the branch-logit MMAs (forward / statistics / backward sweeps): wz_f16 [2 Gp, 64] = folded
+    // optional fp16 operands of the branch-logit MMAs (forward / statistics / training sweeps): wz_f16 [2 Gp, 64] = folded
     // private weights in columns [0, P) of rows [0, G), folded shared weights in columns [P, P + S) of rows [Gp, Gp + G);
     // zc_f16 [B, 64] = zz - m (m = batch mean when training, else 0) in columns [0, P + S).  Centring makes the shift exactly
     // beta and keeps the operand rounding (2^-12) from acting on the common part of the latents.
@@ -406,28 +406,28 @@ __device__ double digamma_d(double x) {
 }
 
 __global__ void __launch_bounds__(256) theta_tables_kernel(const float* __restrict__ px_r, int G, float2* __restrict__ tgf,
-                                                           float2* __restrict__ tgb, float* __restrict__ tb1) {
+                                                           float* __restrict__ tb1) {
     const int i = blockIdx.x * 256 + threadIdx.x;  // entry (gene, count): 16 consecutive threads share a gene
     const int g = i / NB_TAB, c = i - g * NB_TAB;
     if (g >= G) return;
     const float thf = expf(__ldg(px_r + g));  // reference module/spVIPESmodule.py:758 (the same fp32 value as GC_THETA)
-    float2 f = make_float2(0.0f, 0.0f), b = make_float2(0.0f, 0.0f);
+    float2 f = make_float2(0.0f, 0.0f);
+    float b = 0.0f;
     if (c > 0) {
         const double th = (double)thf;
         const float tf = log1pf((float)c);  // the fp32 value the reference's log1p produces
         const double t = (double)tf;
         f = make_float2(tf, (float)(lgamma(t + th) - lgamma(th) - lgamma(t + 1.0)));
-        b = make_float2(tf, (float)(digamma_d(t + th) - digamma_d(th)));
+        b = (float)(digamma_d(t + th) - digamma_d(th));
     }
     if (tgf) tgf[i] = f;
-    if (tgb) tgb[i] = b;
-    if (tb1) tb1[i] = b.y;
+    if (tb1) tb1[i] = b;
 }
 
-extern "C" int spv_dec_theta_tables(const float* px_r, int G, void* tgf, void* tgb, float* tb1, void* stream) {
-    if (!px_r || G <= 0 || (!tgf && !tgb && !tb1)) return SPV_ERR_ARG;
+extern "C" int spv_dec_theta_tables(const float* px_r, int G, void* tgf, float* tb1, void* stream) {
+    if (!px_r || G <= 0 || (!tgf && !tb1)) return SPV_ERR_ARG;
     theta_tables_kernel<<<(G * NB_TAB + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        px_r, G, reinterpret_cast<float2*>(tgf), reinterpret_cast<float2*>(tgb), tb1);
+        px_r, G, reinterpret_cast<float2*>(tgf), tb1);
     SPV_CHECK_LAUNCH();
     return SPV_OK;
 }

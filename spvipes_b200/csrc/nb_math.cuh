@@ -22,7 +22,6 @@ __device__ __forceinline__ float fast_log(float x) { return fast_lg2(x) * 0.6931
 __device__ __forceinline__ float fast_exp(float x) { return fast_ex2(x * 1.44269504089f); }
 
 // outputs of the element functions below
-struct NbGrad { float dyp, dys, dpi, dth; };
 struct NbOut { float ll, ep, es; };
 
 // ================================================================================================================
@@ -77,46 +76,10 @@ __device__ __forceinline__ NbOut nb_forward_v5(float t, float Ct, float xp, floa
     return o;
 }
 
-// gradients of the log-likelihood (NOT of the loss: the consumers apply the signed scale) w.r.t. the two branch logits, the
-// mixture logit and theta.  DpI = exp(-lib) Dp, DsI = exp(-lib) Ds: the softmax-backward row sums of the forward sweep.
-template <bool EXACT>
-__device__ __forceinline__ NbGrad nb_backward_v5(float t, float Ct, float xp, float xs, float pi, float th, float thE, float K1c,
-                                                 float DpI, float DsI) {
-    const float rp = fast_ex2(xp), rs = fast_ex2(xs);
-    const float d1 = rp + thE, d2 = rs + thE;
-    const float L1 = fast_lg2(d1), L2 = fast_lg2(d2);
-    const float x = t + th;
-    float Lap = xp, Las = xs, fp = 1.0f, fs = 1.0f;
-    if (EXACT) {
-        const float ap = rp + NB_EPS, as = rs + NB_EPS;
-        Lap = fast_lg2(ap); Las = fast_lg2(as);
-        fp = rp * fast_rcp(ap); fs = rs * fast_rcp(as);
-    }
-    const float m1 = fmaf(-t, Lap, x * L1), m2 = fmaf(-t, Las, x * L2);
-    const float df = fmaf(m2 - m1, NB_LN2, pi);
-    const float e = fast_ex2(-NB_LOG2E * fabsf(df)), epi = fast_ex2(-NB_LOG2E * fabsf(pi));
-    const float o1 = 1.0f + e, o2 = 1.0f + epi;
-    const float d12 = d1 * d2, oo = o1 * o2;
-    const float r = fast_rcp(d12 * oo);
-    const float rd = r * oo, ro = r * d12;
-    const float id1 = rd * d2, id2 = rd * d1, i1 = ro * o2, i2 = ro * o1;
-    const float wmin = e * i1;
-    const float wa = df >= 0.0f ? 1.0f - wmin : wmin, wb = 1.0f - wa;
-    const float q1 = x * id1, q2 = x * id2;
-    const float ep = wa * fmaf(t, fp, -q1 * rp), es = wb * fmaf(t, fs, -q2 * rs);
-    const float sneg = (pi >= 0.0f ? epi : 1.0f) * i2;  // sigmoid(-pi)
-    NbGrad o;
-    o.dyp = fmaf(-rp, DpI, ep);
-    o.dys = fmaf(-rs, DsI, es);
-    o.dpi = sneg - wb;
-    o.dth = (K1c + Ct) - wa * fmaf(L1, NB_LN2, q1) - wb * fmaf(L2, NB_LN2, q2);
-    return o;
-}
-
 // Forward and backward of one element in one evaluation (the training sweep, nb_tc_train.cu): the log-likelihood, the two branch
 // terms WITHOUT the softmax coupling (ep, es: d ll / d log rho at fixed normaliser; d ll / d y = e - rho exp(-lib) D with the row
 // sum D known only after the sweep), rho of both branches, and the gradients w.r.t. the mixture logit and theta.
-// Ctf / Ctb: the count-dependent lgamma / digamma terms (tables), Kc / K1c the per-gene constants of nb_forward_v5 / nb_backward_v5.
+// Ctf / Ctb: the count-dependent lgamma / digamma terms (tables), Kc / K1c the per-gene forward / backward constants above.
 struct NbTrain { float ll, ep, es, rp, rs, dpi, dth; };
 template <bool EXACT>
 __device__ __forceinline__ NbTrain nb_train_v5(float t, float Ctf, float Ctb, float xp, float xs, float pi, float th, float thE, float Kc,

@@ -10,9 +10,9 @@
 // and the consumers apply the coupling through their other operand:
 //   [Qp | sum dyp | Qs | sum dys] = E4T . ZQ4,  ZQ4 [4 Bp, KZ + 2] rows (4b .. 4b+3) = [zp 1 0 0], -Dp'/1 [zp 1 0 0], [0 0 zs 1], -Ds' [0 0 zs 1]
 //   T [4 Bp, KZ] = E4T^T . [W'p | W's],   d zz[b] = T[4b] - Dp' T[4b+1] (private columns), T[4b+2] - Ds' T[4b+3] (shared), D' = D / 4096
-// (spv_dec_zq4, spv_dec_dz4_combine).  Column sums of d pi and d theta are reduced here as in the backward sweep; those of
+// (spv_dec_zq4, spv_dec_dz4_combine).  Column sums of d pi and d theta are reduced here; those of
 // dyp / dys come out of the first GEMM's ones column.  Row partials (ll, sum ep, sum es) as the forward sweep.
-// Same tiling, pipeline and tensor-memory protocol as nb_tc.cu / nb_tc_bwd.cu.  8 SFU operations per element.
+// Same tiling, pipeline and tensor-memory protocol as nb_tc.cu.  8 SFU operations per element.
 // Reference: nn/networks.py:314-325 + scvi log_mixture_nb (module/spVIPESmodule.py:759, 823-824) and their autograd.
 #include <cuda_fp16.h>
 #include "tc_common.cuh"

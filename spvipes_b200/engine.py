@@ -23,6 +23,8 @@ from . import _lib as L
 HD = 256  # decoder hidden width is fixed (reference nn/networks.py:194, quirk Q8)
 ENC_BN_EPS, ENC_BN_MOM = 1e-5, 0.1
 DEC_BN_EPS, DEC_BN_MOM = 1e-3, 0.01
+# grid cap of the decoder-range Adam update that overlaps the encoder backward (measured optimum on B200 at C5, DESIGN.md section 5)
+ADAM_OVERLAP_BLOCKS = 296
 
 
 # ------------------------------------------------------------------------------------------------
@@ -251,27 +253,12 @@ class Noise:
     drop: Optional[Sequence[torch.Tensor]] = None          # per group [B, 2H] multipliers (private | shared)
 
 
-def _pick_splits(tiles: int, num_kb: int, sms: int = 148, min_kb: int = 4, max_splits: int = 16) -> int:
-    """split-K factor of a GEMM whose output tiles do not fill the SMs evenly: the smallest factor (each split keeps >= min_kb
-    k-blocks) whose CTA count wastes the least of its last wave; 157 tiles on 148 SMs run two rounds unsplit, 942 CTAs run 6.4"""
-    best, best_eff = 1, 0.0
-    for sp in range(1, max_splits + 1):
-        if sp > 1 and num_kb // sp < min_kb:
-            break
-        ctas = tiles * sp
-        eff = ctas / (math.ceil(ctas / sms) * sms)
-        if eff >= 0.9:  # good enough: more splits only add partial-sum traffic
-            return sp
-        if eff > best_eff + 0.02:
-            best, best_eff = sp, eff
-    return best
-
-
 class _GroupWS:
-    def __init__(self, B, G, d: Dims, dev, with_grad: bool, bf16: bool = False, wb=None, dec_dtype=torch.bfloat16, single_sweep=False):
+    def __init__(self, B, G, d: Dims, dev, with_grad: bool, bf16: bool = False, wb=None, fused=False):
         H, S, P, KZ, KMIX, NST = d.n_hidden, d.n_shared, d.n_private, d.KZ, d.KMIX, d.NST
         f = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
         self.B, self.G = B, G
+        self.xs = None
         self.nTG, self.nTB = (G + 63) // 64, (B + 63) // 64
         self.lib = f(B)
         self.h1, self.h2 = f(B, 2 * H), f(B, 2 * H)
@@ -311,30 +298,26 @@ class _GroupWS:
         self.Gp, self.Gpe, self.KMp = r8(G), r8(G + nb), r8(max(KMIX, HD + KZb))
         if bf16:
             h = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)
-            hd = lambda *s: torch.zeros(*s, dtype=dec_dtype, device=dev)  # decoder operands: fp16 on the fused path
+            hd = lambda *s: torch.zeros(*s, dtype=torch.float16 if fused else torch.bfloat16, device=dev)  # decoder operands
             self.amixb = hd(B, self.KMp)
             self.Tb = self.Tb_lo = None  # log1p(counts) as a bf16 pair: only the unfused first layer needs it (need_tb)
-            self.zzb16 = hd(B, r8(KZb)) if nb else None  # 16-bit copy of zzb (operand of the Q = dy^T zz GEMM)
             # fp16 operands of the branch-logit MMAs (spv_dec_fold writes them): centred latents and folded weights
             self.zcb = torch.zeros(B, 64, dtype=torch.float16, device=dev)
             self.wzf = torch.zeros(2 * self.Gp, 64, dtype=torch.float16, device=dev)
-            # count tables of the likelihood sweeps (spv_dec_theta_tables): [G, 16] float2 each, forward / backward
-            self.tgf, self.tgb = f(G, 16, 2), (f(G, 16, 2) if (with_grad and not single_sweep) else None)
-            self.tb1 = f(G, 16) if (with_grad and single_sweep) else None  # digamma terms alone (training sweep)
+            # count tables of the likelihood sweeps (spv_dec_theta_tables): [G, 16] float2 lgamma terms, [G, 16] digamma terms
+            self.tgf = f(G, 16, 2)
+            self.tb1 = f(G, 16) if (with_grad and fused) else None
             # bf16 weight operands are per engine (shared by every workspace): W1b [2H, Gp] and the stacked operand
             # Wstack [3 Gp, KMp]: rows [0, G) mixture weight, [Gp, Gp+G) / [2Gp, 2Gp+G) the folded private / shared
             # factor-regressor weights of the current minibatch in the latent columns (zero elsewhere)
             self.W1b, self.Wstack, self.W1b_lo = wb
             self.Wmb = self.Wstack[:G]
             if with_grad:
-                # D3: the backward sweep's output = fp16 operand of the gradient GEMMs.  Fused path: GENE-major
-                # D3T [3 Gp, Bp] = [dpi ; dyp ; dys] (coalesced stores from the TMEM epilogue, thread = cell); unfused path: cell-major
-                # [B, 3 Gp], only the first Gp columns used
-                self.Bp = r8(B)
                 self.dh1b, self.dh1b_lo = h(B, 2 * H), h(B, 2 * H)
-                if single_sweep:
+                if fused:
                     # outputs of the training sweep (csrc/nb_tc_train.cu), gene-major fp16: E4T [Gp, 4 Bp] = (ep, rp', es, rs') per
-                    # cell, DPIT [Gp, Bp] = d ll / d pi; and the small operands / results of the single-sweep backward
+                    # cell, DPIT [Gp, Bp] = d ll / d pi; and the small operands / results of the backward GEMMs
+                    self.Bp = r8(B)
                     self.E4T, self.DPIT = hd(self.Gp * 4 * self.Bp), hd(self.Gp * self.Bp)
                     self.ldq4 = r8(KZb + 2)
                     self.ZQ4 = hd(4 * self.Bp, self.ldq4)
@@ -342,23 +325,13 @@ class _GroupWS:
                     self.T4 = f(4 * self.Bp, KZb)
                     self.Wcomb = hd(self.Gp, r8(KZb))    # [W'p | W's] (fp16 copy of wfold)
                     self.tc_splits_dz4 = max(1, min(148 // ((4 * B + 127) // 128), (self.Gp + 63) // 64 // 2))
-                    # unsplit by default: measured on B200 at C5, 157 CTAs that leave SMs to the kernels running beside this GEMM give
-                    # a faster STEP (1.85 ms) than 942 evenly filling ones (1.89 ms); _pick_splits stays for A/B (SPV_Q4_SPLITS=auto)
-                    q4 = os.environ.get("SPV_Q4_SPLITS", "1")
-                    self.tc_splits_q4 = _pick_splits((G + 127) // 128, (4 * B + 63) // 64) if q4 == "auto" else max(1, int(q4))
-                    self.ws_q4 = f(max(1, self.tc_splits_q4 * G * (KZb + 2))) if self.tc_splits_q4 > 1 else None
-                    self.D3 = None
                 else:
-                    self.D3 = hd(3 * self.Gp * self.Bp).view(-1)
-                    self.dpib = self.D3.view(-1)[:B * 3 * self.Gp].view(B, 3 * self.Gp)
-                    self.CQ = f(2 * self.Gp, KZb)
+                    self.dpib = hd(B, self.Gp)  # d ll / d pi of spv_dec_nb_bwd (bf16): operand of the two mixture-weight GEMMs
             # split-K factors of the tensor-core GEMMs (128-wide tiles): fill the 148 SMs
             tiles = ((B + 127) // 128) * ((2 * H + 127) // 128)
             self.tc_splits_fc1 = max(1, min(148 // tiles, (G + 63) // 64 // 2))
             tiles = ((B + 127) // 128) * ((KMIX + 127) // 128)
             self.tc_splits_damix = max(1, min(148 // tiles, (G + 63) // 64 // 2))
-            self.tc_splits_damix3 = max(1, min(148 // tiles, (3 * self.Gp + 63) // 64 // 2))
-            self.tc_splits_dz = max(1, min(148 // ((B + 127) // 128), (2 * self.Gp + 63) // 64 // 2))
         if with_grad:
             self.dyp, self.dys, self.dpi = f(B, G), f(B, G), f(B, G)
             self.colpart, self.colsum = f(self.nTB, 4, G), f(4, G)
@@ -373,24 +346,16 @@ class _GroupWS:
             self.g_own, self.g_contrib, self.dexpert = f(B, 2 * S), f(B, 2 * S), f(B, 2 * S)
             self.dh2, self.dh1 = f(B, 2 * H), f(B, 2 * H)
 
+    def need_tb(self, dev):
+        if self.Tb is None:
+            self.Tb = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
+            self.Tb_lo = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
 
-def _need_tb(self, dev):
-    if self.Tb is None:
-        self.Tb = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
-        self.Tb_lo = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
-
-
-_GroupWS.need_tb = _need_tb
-
-
-def _need_xs(self, dtype, dev):
-    """dense staging tile [B, Gp] of a CSR minibatch (spv_csr_gather): what every count consumer reads with rows = NULL"""
-    if getattr(self, "xs", None) is None or self.xs.dtype != dtype:
-        self.xs = torch.zeros(self.B, self.Gp, dtype=dtype, device=dev)
-    return self.xs
-
-
-_GroupWS.need_xs = _need_xs
+    def need_xs(self, dtype, dev):
+        """dense staging tile [B, Gp] of a CSR minibatch (spv_csr_gather): what every count consumer reads with rows = NULL"""
+        if self.xs is None or self.xs.dtype != dtype:
+            self.xs = torch.zeros(self.B, self.Gp, dtype=dtype, device=dev)
+        return self.xs
 
 
 class StepEngine:
@@ -413,11 +378,11 @@ class StepEngine:
             raise NotImplementedError(f"n_dimensions_shared + n_dimensions_private (+ 2 n_batch) = {kz_dec} is not implemented (the "
                                       f"decoder kernels take at most {L.DEC_MAX_LATENT} latent columns)")
         self.fused_nb = self.bf16 and kz_dec <= L.ZK_MAX_LATENT
+        # one sweep over [B, G] per training step on the fused path: the forward sweep also emits what the backward needs
+        # (csrc/nb_tc_train.cu)
+        self.single_sweep = self.fused_nb
         # operands of the decoder GEMMs: fp16 on the fused path (2^-12 rounding, three bits more than bf16; every operand's range
         # is bounded: activations after BatchNorm, weights, gradients stored in natural units), bf16 on the unfused fallback
-        # one sweep over [B, G] per training step: the forward sweep also emits what the backward needs (csrc/nb_tc_train.cu);
-        # SPV_NB_SWEEPS=2 keeps the separate backward sweep (csrc/nb_tc_bwd.cu) for A/B measurements
-        self.single_sweep = self.fused_nb and os.environ.get("SPV_NB_SWEEPS", "1") != "2"
         self.dec_dtype = torch.float16 if self.fused_nb else torch.bfloat16
         self.dec_fmt = 3 if self.fused_nb else 0
         self.lib = L.load()
@@ -454,14 +419,8 @@ class StepEngine:
         self._ctx = None
         self._side = None
         self._aux = None
-        self._aux_lanes = int(__import__("os").environ.get("SPV_AUX_LANES", "2"))  # A/B switch
         self._pending = {}
         self.parallel_groups = True
-        # fc2 + heads (and their backward) as one launch each (spv_enc_mid_*): opt-in.  Measured at C2 it is slower than the
-        # separate whole-K GEMMs (0.404 against 0.385 ms per step): 143 KB of shared memory per CTA means one 4-warp CTA per SM
-        # and no overlap of the two groups' launches (15 us alone, 21-30 us for the second group).
-        self.enc_mid = (self.device.type == "cuda" and bool(self.lib.spv_enc_mid_supported(self.d.n_hidden, self.d.n_private, self.d.n_shared))
-                        and __import__("os").environ.get("SPV_ENC_MID", "0") == "1")
         r8 = lambda x: (x + 7) // 8 * 8
         self.wb = None
         if self.bf16:
@@ -483,9 +442,8 @@ class StepEngine:
         # weight gradient 183 us per group against 60 (staging pass, HBM bound) + 71 resp. 88 us for the TMA-fed split GEMMs:
         # one scattered 16-byte access per lane makes every warp load 32 L1 wavefronts, and table look-ups, operand stores and
         # the tensor core's operand reads share the shared-memory pipe.
-        self.fused_fc1 = __import__("os").environ.get("SPV_FUSED_FC1", "0") == "1"
+        self.fused_fc1 = os.environ.get("SPV_FUSED_FC1", "0") == "1"
         self.nb_events = None  # bench hook: iterator of (start, end) CUDA events bracketing the NB-loglik sweep
-        self.nb_bwd_events = None  # ... and its backward sweep
 
     # -------------------------------------------------------------------------------- helpers
     def P(self, g, name):
@@ -573,7 +531,7 @@ class StepEngine:
         cur = torch.cuda.current_stream(self.device)
         fork = torch.cuda.Event()
         fork.record(cur)
-        aux = self._aux[g][lane if self._aux_lanes > 1 else 0]
+        aux = self._aux[g][lane]
         aux.wait_event(fork)
         with torch.cuda.stream(aux):
             yield
@@ -608,7 +566,7 @@ class StepEngine:
         key = (B0, B1, with_grad)
         if key not in self._ws:
             self._ws[key] = [_GroupWS(B, G, self.d, self.device, with_grad, self.bf16, self.wb[g] if self.bf16 else None,
-                                      self.dec_dtype, self.single_sweep) for g, (B, G) in enumerate(zip((B0, B1), self.d.genes))]
+                                      self.fused_nb) for g, (B, G) in enumerate(zip((B0, B1), self.d.genes))]
         return self._ws[key]
 
     @staticmethod
@@ -733,26 +691,19 @@ class StepEngine:
             dropping = training and (mask is not None or self.dropout_rate > 0)
             for ev in self._noise_events:
                 torch.cuda.current_stream(self.device).wait_event(ev)
+            fuse_drop = dropping and self._can_fuse(H)  # dropout in the fc2 epilogue (same keep mask as spv_dropout)
+            self._gemm(L.ptr(w.h1), L.ptr(self.P(g, "W2")), L.ptr(w.h2), B, H, H, lda=2 * H, ldb=H, ldc=2 * H, tb=1, batch=2,
+                       sA=H, sB=H * H, sC=H, bias=L.ptr(self.P(g, "b2")), sBias=H, relu=1,
+                       drop=(0.0 if mask is not None else self.dropout_rate, L.ptr(mask), 8 + g, 2 * H) if fuse_drop else None)
+            if dropping and not fuse_drop:
+                L.check(lib.spv_dropout(L.ptr(w.h2), 2 * H, B, 2 * H, L.ptr(mask), 2 * H, self.dropout_rate, self.seed,
+                                        8 + g, L.ptr(self.noise_dev), st), "spv_dropout")
             bhd = self.P(g, "bhd")
-            if self.enc_mid:  # fc2 -> ReLU -> dropout -> mu / logvar heads of both encoders in one launch
-                L.check(lib.spv_enc_mid_fwd(L.ptr(w.h1), 2 * H, L.ptr(self.P(g, "W2")), L.ptr(self.P(g, "b2")),
-                                            L.ptr(self.P(g, "Whp")), L.ptr(self.P(g, "Whs")), L.ptr(bhd), L.ptr(w.h2), 2 * H,
-                                            L.ptr(w.r), NST, L.ptr(mask), 2 * H, self.dropout_rate if dropping else 0.0,
-                                            self.seed, 8 + g, L.ptr(self.noise_dev), B, H, P, S, st), "spv_enc_mid_fwd")
-            else:
-                fuse_drop = dropping and self._can_fuse(H)  # dropout in the fc2 epilogue (same keep mask as spv_dropout)
-                self._gemm(L.ptr(w.h1), L.ptr(self.P(g, "W2")), L.ptr(w.h2), B, H, H, lda=2 * H, ldb=H, ldc=2 * H, tb=1, batch=2,
-                           sA=H, sB=H * H, sC=H, bias=L.ptr(self.P(g, "b2")), sBias=H, relu=1,
-                           drop=(0.0 if mask is not None else self.dropout_rate, L.ptr(mask), 8 + g, 2 * H) if fuse_drop else None)
-                if dropping and not fuse_drop:
-                    L.check(lib.spv_dropout(L.ptr(w.h2), 2 * H, B, 2 * H, L.ptr(mask), 2 * H, self.dropout_rate, self.seed,
-                                            8 + g, L.ptr(self.noise_dev), st), "spv_dropout")
-                bhd = self.P(g, "bhd")
-                with self._branch(g, "headp"):  # the private and the shared heads are independent
-                    self._gemm(L.ptr(w.h2), L.ptr(self.P(g, "Whp")), L.ptr(w.r), B, 2 * P, H, lda=2 * H, ldb=H, ldc=NST, tb=1,
-                               bias=L.ptr(bhd))
-                self._gemm(w.h2.data_ptr() + 4 * H, L.ptr(self.P(g, "Whs")), w.r.data_ptr() + 4 * 2 * P, B, 2 * S, H, lda=2 * H,
-                           ldb=H, ldc=NST, tb=1, bias=bhd.data_ptr() + 4 * 2 * P)
+            with self._branch(g, "headp"):  # the private and the shared heads are independent
+                self._gemm(L.ptr(w.h2), L.ptr(self.P(g, "Whp")), L.ptr(w.r), B, 2 * P, H, lda=2 * H, ldb=H, ldc=NST, tb=1,
+                           bias=L.ptr(bhd))
+            self._gemm(w.h2.data_ptr() + 4 * H, L.ptr(self.P(g, "Whs")), w.r.data_ptr() + 4 * 2 * P, B, 2 * S, H, lda=2 * H,
+                       ldb=H, ldc=NST, tb=1, bias=bhd.data_ptr() + 4 * 2 * P)
             self._join(g, "headp")
             L.check(lib.spv_bn_fwd(L.ptr(w.r), NST, L.ptr(w.stats), NST, B, NST, L.ptr(self.P(g, "ghd")),
                                    L.ptr(self.P(g, "bthd")), ENC_BN_EPS, ENC_BN_MOM, L.ptr(self.Bf(g, "rm_hd")),
@@ -797,8 +748,8 @@ class StepEngine:
             if self.fused_nb:
                 # count tables of the likelihood sweeps: a function of px_r only, on the second auxiliary stream
                 with self._branch(g, "tg", lane=1):
-                    L.check(lib.spv_dec_theta_tables(L.ptr(self.P(g, "px_r")), G, L.ptr(w.tgf), L.ptr(w.tgb), L.ptr(w.tb1),
-                                                     self._stream()), "spv_dec_theta_tables")
+                    L.check(lib.spv_dec_theta_tables(L.ptr(self.P(g, "px_r")), G, L.ptr(w.tgf), L.ptr(w.tb1), self._stream()),
+                            "spv_dec_theta_tables")
                 # hidden layer of the mixing net (needs only zz) on the auxiliary stream, beside latent stats / fold / normalisers;
                 # the bf16 operand [hm | zz] of the mixture GEMM in one conversion pass after it
                 with self._branch(g, "hm"):
@@ -829,7 +780,7 @@ class StepEngine:
                 evs[0].record()
             if self.bf16:
                 if self.fused_nb:
-                    if self.single_sweep and training and with_grad:  # one sweep: likelihood + everything the backward needs
+                    if training and with_grad:  # one sweep: likelihood + everything the backward needs
                         L.check(lib.spv_dec_nb_train_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp,
                                                         L.ptr(w.zcb), L.ptr(w.wzf), L.ptr(w.E4T), 4 * w.Bp, L.ptr(w.DPIT), w.Bp, B, G, HD,
                                                         Pb, Sb, KMIX, st), "spv_dec_nb_train_tc")
@@ -858,8 +809,7 @@ class StepEngine:
         wg = with_grad
         return L.ptr_array([xptr, rows, w.amix, w.wfold, self.P(g, "Wm"), self.P(g, "bm"), w.genec, w.lib, w.part_stats,
                             w.rowc, w.pi, w.part_nb, w.dyp if wg else None, w.dys if wg else None, w.dpi if wg else None,
-                            w.colpart if wg else None, w.rec, getattr(w, "tgf", None),
-                            getattr(w, "tb1", None) if self.single_sweep else getattr(w, "tgb", None)])
+                            w.colpart if wg else None, w.rec, getattr(w, "tgf", None), getattr(w, "tb1", None)])
 
     def _pairing(self, batches, ws, Bs):
         lib, st, d = self.lib, self._stream(), self.d
@@ -979,7 +929,7 @@ class StepEngine:
             zzp = w.amix.data_ptr() + 4 * HD
             nb, Pb, Sb, KZb = d.nb, d.Pb, d.Sb, d.KZb
             zb, ld_zb = (L.ptr(w.zzb), KZb) if nb else (zzp, KMIX)
-            if self.fused_nb and self.single_sweep:
+            if self.fused_nb:
                 # the training sweep of the forward left E4T = (ep, rp', es, rs') and DPIT = d ll / d pi (fp16, gene-major): the
                 # backward of the likelihood is four GEMMs; the softmax coupling rides in their small operands (csrc/nb_tc_train.cu)
                 f3, al = self.dec_fmt, -float(grad_scale) / B
@@ -995,59 +945,26 @@ class StepEngine:
                     self._tc_gemm(L.ptr(w.DPIT), L.ptr(w.amixb), L.ptr(self.Gd(g, "Wm")), G, KMIX, B, lda=Bp, ldb=w.KMp, ldc=KMIX,
                                   a_mn=0, b_mn=1, fmt=f3, alpha=al)
                 with self._branch(g, "gene", lane=1):
-                    # [Qp | sum dyp | Qs | sum dys] = E4T . ZQ4 (K = 4 B: the coupling -D' [z 1] rides in ZQ4's odd rows)
+                    # [Qp | sum dyp | Qs | sum dys] = E4T . ZQ4 (K = 4 B: the coupling -D' [z 1] rides in ZQ4's odd rows); unsplit:
+                    # measured faster in the step than a split that fills the SMs evenly (DESIGN.md section 8)
                     L.check(lib.spv_dec_zq4(zb, ld_zb, L.ptr(w.rowc), L.ptr(w.ZQ4), w.ldq4, B, Pb, Sb, self._stream()), "spv_dec_zq4")
                     self._tc_gemm(L.ptr(w.E4T), L.ptr(w.ZQ4), L.ptr(w.CQ), G, ldq, 4 * B, lda=4 * Bp, ldb=w.ldq4, ldc=ldq,
-                                  a_mn=0, b_mn=1, splits=w.tc_splits_q4, ws=w.ws_q4, fmt=f3, alpha=al)
+                                  a_mn=0, b_mn=1, fmt=f3, alpha=al)
                     self._gene_bwd(g, w, w.CQ.data_ptr(), w.CQ.data_ptr() + 4 * (Pb + 1), ldq, B, G, colsum_in_q=1)
-                Qp, Qs, dzraw = None, None, None
+                dzraw = None
                 # d [hm | zz] (mixture part) = dpi Wm
                 self._tc_gemm(L.ptr(w.DPIT), L.ptr(w.Wstack), L.ptr(w.damix), B, KMIX, G, lda=Bp, ldb=w.KMp, ldc=KMIX, a_mn=1, b_mn=1,
-                              splits=w.tc_splits_damix, ws=w.ws, fmt=f3, alpha=al)
-            elif self.fused_nb:
-                # logits recomputed on the tensor cores, gradients in the TMEM epilogue -> D3 = [dpi | dyp | dys] (bf16)
-                evs = next(self.nb_bwd_events) if self.nb_bwd_events is not None else None
-                if evs is not None:
-                    evs[0].record()
-                L.check(lib.spv_dec_nb_bwd_tc(src, self._dec_ptrs(g, w, xptr, count_rows, True), ldx, L.ptr(w.amixb), w.KMp,
-                                              L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb), L.ptr(w.wzf), L.ptr(w.D3), w.Bp, B, G, HD, Pb, Sb,
-                                              -float(grad_scale) / B, L.ptr(w.colsum), KMIX, st), "spv_dec_nb_bwd_tc")
-                if evs is not None:
-                    evs[1].record()
-                Bp, d3_branches = w.Bp, w.D3.data_ptr() + 2 * w.Gp * w.Bp  # D3T rows Gp .. 3 Gp: [dyp ; dys]
-                # d zz through the two softmax branches: [dyp | dys] against the folded weights' latent columns (K = 2 Gp,
-                # N = P + S).  Kept out of the mixture GEMM below: stacked into its K it would triple that GEMM's operand traffic.
-                f3, al = self.dec_fmt, -float(grad_scale) / B  # D3T holds d log-likelihood: the GEMMs apply the signed scale
-                with self._branch(g, "dzg"):
-                    self._tc_gemm(d3_branches, w.Wstack.data_ptr() + 2 * (w.Gp * w.KMp + HD), L.ptr(w.dzraw), B, KZb,
-                                  2 * w.Gp, lda=Bp, ldb=w.KMp, ldc=KZb, a_mn=1, b_mn=1, splits=w.tc_splits_dz, ws=w.ws2, fmt=f3, alpha=al)
-                with self._branch(g, "wgrad"):  # d Wm = dpi^T [hm | zz]
-                    self._tc_gemm(L.ptr(w.D3), L.ptr(w.amixb), L.ptr(self.Gd(g, "Wm")), G, KMIX, B, lda=Bp, ldb=w.KMp, ldc=KMIX,
-                                  a_mn=0, b_mn=1, fmt=f3, alpha=al)
-                Qp, Qs, ldq, dzraw = w.CQ.data_ptr(), w.CQ.data_ptr() + 4 * (w.Gp * KZb + Pb), KZb, None
-                if nb:  # 16-bit copy of the regressors' inputs (without covariates they are the latent columns of amixb)
-                    self._to_dec(L.ptr(w.zzb), KZb, L.ptr(w.zzb16), w.zzb16.stride(0), B, KZb)
-                zb16, ld_zb16 = (L.ptr(w.zzb16), w.zzb16.stride(0)) if nb else (w.amixb.data_ptr() + 2 * HD, w.KMp)
-                # per-gene BatchNorm backward chain on the second auxiliary stream: it needs Q and the column sums, not
-                # d [hm | zz], so it runs beside the input-gradient GEMM and the hidden layer's backward
-                with self._branch(g, "gene", lane=1):
-                    # [Qp | .] = dyp^T zz, [. | Qs] = dys^T zz in one GEMM over the stacked rows (rows g and Gp + g)
-                    self._tc_gemm(d3_branches, zb16, L.ptr(w.CQ), 2 * w.Gp, KZb, B, lda=Bp,
-                                  ldb=ld_zb16, ldc=KZb, a_mn=0, b_mn=1, fmt=f3, alpha=al)
-                    self._gene_bwd(g, w, Qp, Qs, ldq, B, G)
-                # d [hm | zz] (mixture part) = dpi Wm
-                self._tc_gemm(L.ptr(w.D3), L.ptr(w.Wstack), L.ptr(w.damix), B, KMIX, G, lda=Bp, ldb=w.KMp, ldc=KMIX, a_mn=1, b_mn=1,
                               splits=w.tc_splits_damix, ws=w.ws, fmt=f3, alpha=al)
             else:
                 L.check(lib.spv_dec_nb_bwd(src, self._dec_ptrs(g, w, xptr, count_rows, True), ldx, KMIX, B, G, HD, Pb, Sb,
                                            -float(grad_scale) / B, L.ptr(w.colsum), L.ptr(w.dpib) if self.bf16 else None,
-                                           3 * w.Gp if self.bf16 else 0, L.ptr(w.zzb) if nb else None, KZb, KMIX, st),
+                                           w.Gp if self.bf16 else 0, L.ptr(w.zzb) if nb else None, KZb, KMIX, st),
                         "spv_dec_nb_bwd")
                 # d Wm = dpi^T [hm | zz];   d [hm | zz] = dpi Wm
                 if self.bf16:
-                    self._tc_gemm(L.ptr(w.dpib), L.ptr(w.amixb), L.ptr(self.Gd(g, "Wm")), G, KMIX, B, lda=3 * w.Gp, ldb=w.KMp,
+                    self._tc_gemm(L.ptr(w.dpib), L.ptr(w.amixb), L.ptr(self.Gd(g, "Wm")), G, KMIX, B, lda=w.Gp, ldb=w.KMp,
                                   ldc=KMIX, a_mn=1, b_mn=1)
-                    self._tc_gemm(L.ptr(w.dpib), L.ptr(w.Wmb), L.ptr(w.damix), B, KMIX, G, lda=3 * w.Gp, ldb=w.KMp, ldc=KMIX,
+                    self._tc_gemm(L.ptr(w.dpib), L.ptr(w.Wmb), L.ptr(w.damix), B, KMIX, G, lda=w.Gp, ldb=w.KMp, ldc=KMIX,
                                   b_mn=1, splits=w.tc_splits_damix, ws=w.ws)
                 else:
                     self._gemm(L.ptr(w.dpi), L.ptr(w.amix), L.ptr(self.Gd(g, "Wm")), G, KMIX, B, lda=G, ldb=KMIX, ldc=KMIX, ta=1)
@@ -1141,15 +1058,8 @@ class StepEngine:
             fuse2 = self._can_fuse(2 * S)  # ReLU + dropout backward in the epilogue of the two head input-gradient GEMMs
             gate_p = (L.ptr(w.h2), 2 * H, L.ptr(mask), 2 * H, scale) if fuse2 else None
             gate_s = (w.h2.data_ptr() + 4 * H, 2 * H, mask.data_ptr() + 4 * H if mask is not None else None, 2 * H, scale) if fuse2 else None
-            if self.enc_mid:  # heads -> (ReLU, dropout) -> fc2 -> ReLU backward of both encoders in one launch: dh2, dh1 (+ bf16)
-                L.check(lib.spv_enc_mid_bwd(L.ptr(w.dr), NST, L.ptr(self.P(g, "Whp")), L.ptr(self.P(g, "Whs")),
-                                            L.ptr(self.P(g, "W2")), L.ptr(w.h2), 2 * H, L.ptr(w.h1), 2 * H, L.ptr(mask), 2 * H,
-                                            scale, L.ptr(w.dh2), 2 * H, L.ptr(w.dh1), 2 * H,
-                                            L.ptr(w.dh1b) if self.bf16 else None, 2 * H, B, H, P, S, st), "spv_enc_mid_bwd")
-            else:
-                with self._branch(g, "dh2p"):  # first on its auxiliary stream: this one is on the critical path
-                    self._gemm(L.ptr(w.dr), L.ptr(self.P(g, "Whp")), L.ptr(w.dh2), B, H, 2 * P, lda=NST, ldb=H, ldc=2 * H,
-                               gate=gate_p)
+            with self._branch(g, "dh2p"):  # first on its auxiliary stream: this one is on the critical path
+                self._gemm(L.ptr(w.dr), L.ptr(self.P(g, "Whp")), L.ptr(w.dh2), B, H, 2 * P, lda=NST, ldb=H, ldc=2 * H, gate=gate_p)
             if adam is not None and not adam.get("enc_only"):  # every decoder gradient of this group is final: update that range now
                 self._join(g, "wgrad")
                 self._join(g, "wgrad1")
@@ -1157,7 +1067,7 @@ class StepEngine:
                     for ev in tick_events:
                         torch.cuda.current_stream(self.device).wait_event(ev)
                     lo, hi = self.params.group_ranges[PHASE_DEC][g]
-                    self._adam_range(lo, hi, adam, max_blocks=int(__import__("os").environ.get("SPV_ADAM_BLOCKS", "296")))
+                    self._adam_range(lo, hi, adam, max_blocks=ADAM_OVERLAP_BLOCKS)
             with self._branch(g, "wgrad1", lane=1):
                 L.check(lib.spv_colsum(L.ptr(w.dr), NST, B, NST, L.ptr(self.Gd(g, "bhd")), self._stream()), "spv_colsum")
             with self._branch(g, "wgrad"):
@@ -1165,26 +1075,23 @@ class StepEngine:
                            splits=w.splits_b, ws=w.ws2)
                 self._gemm(drs, w.h2.data_ptr() + 4 * H, L.ptr(self.Gd(g, "Whs")), 2 * S, H, B, lda=NST, ldb=2 * H, ldc=H, ta=1,
                            splits=w.splits_b, ws=w.ws2)
-            if not self.enc_mid:
-                self._gemm(drs, L.ptr(self.P(g, "Whs")), w.dh2.data_ptr() + 4 * H, B, H, 2 * S, lda=NST, ldb=H, ldc=2 * H,
-                           gate=gate_s)
-                self._join(g, "dh2p")
-                if not fuse2:
-                    L.check(lib.spv_relu_bwd(L.ptr(w.dh2), 2 * H, L.ptr(w.h2), 2 * H, B, 2 * H, L.ptr(mask), 2 * H, scale, st),
-                            "spv_relu_bwd")
+            self._gemm(drs, L.ptr(self.P(g, "Whs")), w.dh2.data_ptr() + 4 * H, B, H, 2 * S, lda=NST, ldb=H, ldc=2 * H, gate=gate_s)
+            self._join(g, "dh2p")
+            if not fuse2:
+                L.check(lib.spv_relu_bwd(L.ptr(w.dh2), 2 * H, L.ptr(w.h2), 2 * H, B, 2 * H, L.ptr(mask), 2 * H, scale, st),
+                        "spv_relu_bwd")
             with self._branch(g, "wgrad1", lane=1):
                 self._gemm(L.ptr(w.dh2), L.ptr(w.h1), L.ptr(self.Gd(g, "W2")), H, H, B, lda=2 * H, ldb=2 * H, ldc=H, ta=1,
                            batch=2, sA=H, sB=H, sC=H * H, splits=w.splits_b, ws=w.ws3)
                 L.check(lib.spv_colsum(L.ptr(w.dh2), 2 * H, B, 2 * H, L.ptr(self.Gd(g, "b2")), self._stream()), "spv_colsum")
-            fuse1 = self.enc_mid or self._can_fuse(H)  # ReLU backward + bf16 copy in the fc2 input-gradient GEMM's epilogue
-            if not self.enc_mid:
-                self._gemm(L.ptr(w.dh2), L.ptr(self.P(g, "W2")), L.ptr(w.dh1), B, H, H, lda=2 * H, ldb=H, ldc=2 * H, batch=2,
-                           sA=H, sB=H * H, sC=H, gate=(L.ptr(w.h1), 2 * H, None, 0, 1.0) if fuse1 else None,
-                           c_bf16=(L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H) if (fuse1 and self.bf16) else None)
+            fuse1 = self._can_fuse(H)  # ReLU backward + bf16 copy in the fc2 input-gradient GEMM's epilogue
+            self._gemm(L.ptr(w.dh2), L.ptr(self.P(g, "W2")), L.ptr(w.dh1), B, H, H, lda=2 * H, ldb=H, ldc=2 * H, batch=2,
+                       sA=H, sB=H * H, sC=H, gate=(L.ptr(w.h1), 2 * H, None, 0, 1.0) if fuse1 else None,
+                       c_bf16=(L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H) if (fuse1 and self.bf16) else None)
             if not fuse1:
                 L.check(lib.spv_relu_bwd(L.ptr(w.dh1), 2 * H, L.ptr(w.h1), 2 * H, B, 2 * H, None, 0, 1.0, st), "spv_relu_bwd")
             if self.bf16:
-                if not fuse1 or self.enc_mid:
+                if not fuse1:
                     L.check(lib.spv_to_bf16_split(L.ptr(w.dh1), 2 * H, L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H, B, 2 * H, st),
                             "spv_to_bf16_split")
                 if self.fused_fc1 and src == L.SRC_U16_LOG1P:  # counts transformed in the GEMM's producer warps (as the forward)

@@ -143,7 +143,6 @@ ENGINE_CASES = [  # (id, mode, precision, env, n_batch, counts, training)
     ("paired-fp32", "paired", "fp32", {}, 0, "u16", True),
     ("label-bf16-covariates", "label", "bf16", {}, 3, "u16", True),
     ("label-fp32-covariates", "label", "fp32", {}, 3, "u16", True),
-    ("label-bf16-two-sweeps", "label", "bf16", {"SPV_NB_SWEEPS": "2"}, 0, "u16", True),
     ("label-bf16-fused-fc1", "label", "bf16", {"SPV_FUSED_FC1": "1"}, 0, "u16", True),
     ("label-bf16-float-counts", "label", "bf16", {}, 0, "f32", True),
     ("label-fp32-float-counts", "label", "fp32", {}, 0, "f32", True),

@@ -454,18 +454,16 @@ def _compare(eng, ws, case, training, fused, single):
     return err, where, refs
 
 
-def _check(name, precision, training, sweeps, monkeypatch, expect_fused=None):
-    if sweeps == 2:
-        monkeypatch.setenv("SPV_NB_SWEEPS", "2")
+def _check(name, precision, training, expect_fused=None):
     case = build_case(name)
     eng, ws = _run_engine(case, precision, training)
     if expect_fused is not None:
         assert eng.fused_nb == expect_fused
-    single = eng.fused_nb and eng.single_sweep and training
+    single = eng.fused_nb and training
     err, where, refs = _compare(eng, ws, case, training, eng.fused_nb, single)
     if training:
         assert_classes(case, refs)
-    print(f"\n[f64] {name} {precision} {'train' if training else 'eval'} sweeps={sweeps} fused={eng.fused_nb}: "
+    print(f"\n[f64] {name} {precision} {'train' if training else 'eval'} fused={eng.fused_nb}: "
           + " ".join(f"{k}={v:.2e}" for k, v in sorted(err.items())) + f" worst at {where}")
     gates = FP32_GATES if precision == "fp32" else TC_GATES
     bad = {k: v for k, v in err.items() if not v <= gates[k]}
@@ -475,28 +473,21 @@ def _check(name, precision, training, sweeps, monkeypatch, expect_fused=None):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["b300", "b300-f32", "b1000", "b1000-offset", "b2100", "b8300"])
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
-def test_training_step_against_f64(name, precision, monkeypatch):
+def test_training_step_against_f64(name, precision):
     """fp32 SIMT decoder and the default bf16 single-sweep decoder, one training step"""
-    _check(name, precision, True, 1, monkeypatch, expect_fused=precision == "bf16" or None)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("name", ["b300", "b300-f32", "b1000"])
-def test_two_sweep_training_step_against_f64(name, monkeypatch):
-    """SPV_NB_SWEEPS=2: forward sweep + separate backward sweep (spv_dec_nb_fwd_tc, spv_dec_nb_bwd_tc)"""
-    _check(name, "bf16", True, 2, monkeypatch, expect_fused=True)
+    _check(name, precision, True, expect_fused=precision == "bf16" or None)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["b300", "b300-f32", "b1000"])
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
-def test_eval_forward_against_f64(name, precision, monkeypatch):
+def test_eval_forward_against_f64(name, precision):
     """eval forward: BatchNorm on the running statistics, per-cell reconstruction term"""
-    _check(name, precision, False, 1, monkeypatch)
+    _check(name, precision, False)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,fused", [("w58", True), ("w59", False), ("w64", False), ("w65", False), ("w96", False)])
-def test_latent_width_against_f64(name, fused, monkeypatch):
+def test_latent_width_against_f64(name, fused):
     """bf16 engines around the fused decoder's latent limit: fused up to 58 columns, the unfused bf16 decoder above"""
-    _check(name, "bf16", True, 1, monkeypatch, expect_fused=fused)
+    _check(name, "bf16", True, expect_fused=fused)

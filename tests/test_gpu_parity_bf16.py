@@ -192,24 +192,6 @@ def test_philox_noise_is_the_same_in_forward_and_backward():
         assert int(engA.step_dev) == 3 and int(engA.noise_dev) == 3
 
 
-def test_enc_mid_kernels_match_separate_launches():
-    """opt-in fused fc2 + heads kernels (spv_enc_mid_fwd / _bwd) against the default separate GEMM launches: same step.
-    fp32 engine, so that rounding-order differences (~1e-7) are not amplified by bf16 operand rounding downstream."""
-    gd = Golden("label_tiny")
-    res = []
-    for fused in (False, True):
-        eng, batches, noise = engine_from_golden(gd, precision="fp32")
-        eng.enc_mid = fused and bool(eng.lib.spv_enc_mid_supported(eng.d.n_hidden, eng.d.n_private, eng.d.n_shared))
-        if fused and not eng.enc_mid:
-            pytest.skip("sizes not supported by the fused kernels")
-        ws = eng.forward(batches, training=True, noise=noise)
-        eng.backward()
-        torch.cuda.synchronize()
-        res.append((eng.loss_out.clone(), eng.grads.clone(), ws[0].r.clone(), ws[0].h2.clone(), ws[0].dh1.clone()))
-    for a, b in zip(*res):
-        assert float((a - b).abs().max()) <= 2e-5 * float(b.abs().max()) + 1e-7
-
-
 @pytest.mark.parametrize("mode,precision", [("paired", "fp32"), ("cluster", "fp32"), ("paired", "bf16"), ("cluster", "bf16")])
 def test_ot_modes_hidden256_against_oracle(mode, precision):
     """BASELINE.json configs[2] / [3] flavour at a size the oracle finishes in seconds: OT-paired and OT-cluster PoE with

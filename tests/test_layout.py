@@ -22,18 +22,6 @@ def test_state_dict_roundtrip_matches_reference_names():
     assert set(eng.grad_dict().keys()) == set(gd.grads.keys())
 
 
-def test_pick_splits_prefers_even_waves():
-    """engine._pick_splits: the smallest split-K factor whose CTA count fills its last wave on 148 SMs (>= 90 %), never leaving a
-    split fewer than four k-blocks"""
-    from spvipes_b200.engine import _pick_splits
-    assert _pick_splits(148, 64) == 1            # one full wave as it is
-    assert _pick_splits(157, 128) == 6           # 157 tiles: 2 rounds unsplit, 942 CTAs = 6.4 waves
-    assert _pick_splits(157, 8) in (1, 2)        # cannot split below four k-blocks per CTA
-    for tiles, kb in ((1, 8), (40, 32), (79, 64), (313, 16)):
-        sp = _pick_splits(tiles, kb)
-        assert 1 <= sp <= 16 and (sp == 1 or kb // sp >= 4)
-
-
 def test_flat_ranges_are_float4_aligned():
     """every phase / group range of the flat parameter layout starts and ends on a multiple of 4 floats: the gradient exchange
     kernel (csrc/xgpu.cu) and Adam work on float4"""

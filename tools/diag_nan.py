@@ -30,7 +30,6 @@ for s in range(30):
     print(s, "loss", [round(float(x), 3) for x in eng.loss_out[:7]], "grads/params finite", fin, "bad", bad[:12], flush=True)
     if bad or not fin:
         for g, w in enumerate(ws):
-            d3 = w.D3 if getattr(w, "D3", None) is not None else w.E4T  # two-sweep / single-sweep gradient operand
-            print(" g", g, "max |D3 / E4T|", float(d3.float().abs().max()), "max |amixb|", float(w.amixb.float().abs().max()), "max |wzf|", float(w.wzf.float().abs().max()),
+            print(" g", g, "max |E4T|", float(w.E4T.float().abs().max()), "max |amixb|", float(w.amixb.float().abs().max()), "max |wzf|", float(w.wzf.float().abs().max()),
                   "max |Wstack|", float(w.Wstack.float().abs().max()), "max |zcb|", float(w.zcb.float().abs().max()), "max lib", float(w.lib.max()), "max rowc", w.rowc.abs().max(0).values.tolist())
         break
