@@ -223,6 +223,23 @@ int spv_dec_nb_bwd(int src, const void* const* ptrs, long long ldx, long long ld
 int spv_dec_nb_fwd_tc(int src, const void* const* ptrs, long long ldx, const void* amix_bf16, long long ld_amixb,
                       const void* wstack_bf16, long long ld_w, int Gp, const void* zc_f16, const void* wz_f16, int B, int G,
                       int HD, int P, int S, int store_pi, int kmix, void* stream);
+/* per-element outputs of the likelihood sweeps (scvi NegativeBinomialMixture: px.log_prob, mu1, mu2, mixture_logits, mean),
+ * stored instead of reduced.  outs: HOST array of 5 device pointers, each [B, ld_out] fp32 row-major or NULL (not written):
+ *   outs[0] ll      log_mixture_nb(t; rate_p, rate_s, theta, pi) per element (eps 1e-8), t = log1p(count) or, for src
+ *                   SPV_SRC_F32, the value in ptrs[0] as given (px.log_prob(value))
+ *   outs[1] rate_p  exp(lib) softmax_g(BN_p(z_private_arg Wp^T))          (px_rate_private)
+ *   outs[2] rate_s  exp(lib) softmax_g(BN_s(z_shared_arg Ws^T))           (px_rate_shared)
+ *   outs[3] pi      mixing logit, bias included                           (px_mixing)
+ *   outs[4] mean    sigmoid(pi) rate_p + (1 - sigmoid(pi)) rate_s
+ * Counts / targets (ptrs[0], ptrs[1]) and the count table are read only when outs[0] is requested.  module/spVIPESmodule.py:751-759
+ * spv_dec_nb_elems_tc: the element sweep of spv_dec_nb_fwd_tc (same operands, state of the same pass; part_nb unused).
+ * spv_dec_nb_elems: the element pass of spv_dec_nb_fwd's phase 2, after phase 1 (rowc); pi_ready: the mixture logits are in
+ * ptrs[10] (spv_tc_gemm) - else the pass computes them from amix / wm as phase 2 does. */
+int spv_dec_nb_elems_tc(int src, const void* const* ptrs, long long ldx, const void* amix_bf16, long long ld_amixb,
+                        const void* wstack_bf16, long long ld_w, int Gp, const void* zc_f16, const void* wz_f16, int B, int G,
+                        int HD, int P, int S, int kmix, void* const* outs, long long ld_out, void* stream);
+int spv_dec_nb_elems(int src, const void* const* ptrs, long long ldx, long long ld_amix, int B, int G, int HD, int P, int S,
+                     int pi_ready, const float* zzb, long long ld_zzb, int kmix, void* const* outs, long long ld_out, void* stream);
 /* tensor-core version of phase 1 of spv_dec_nb_fwd: softmax normalisers rowc[b, 0:2] = lib[b] - logsumexp_g(y_p), (y_s)
  * from the fp16 branch operands (spv_dec_fold); part_stats: scratch of 2 * ceil(G/64) * B * 4 floats.
  * nn/networks.py:318-320, module/spVIPESmodule.py:751-757 */

@@ -62,6 +62,8 @@ _SIGS = {
     "spv_dec_nb_fwd": [i, p, ll, ll, i, i, i, i, i, i, p, ll, i, p],
     "spv_dec_nb_bwd": [i, p, ll, ll, i, i, i, i, i, f, p, p, ll, p, ll, i, p],
     "spv_dec_nb_fwd_tc": [i, p, ll, p, ll, p, ll, i, p, p, i, i, i, i, i, i, i, p],
+    "spv_dec_nb_elems_tc": [i, p, ll, p, ll, p, ll, i, p, p, i, i, i, i, i, i, p, ll, p],
+    "spv_dec_nb_elems": [i, p, ll, ll, i, i, i, i, i, i, p, ll, i, p, ll, p],
     "spv_dec_nb_rowreduce": [p, i, i, i, p, p, p],
     "spv_dec_gene_bwd": [p, ll, i, i, i, i, i, p],
     "spv_dec_gene_bwd_parts": [i],

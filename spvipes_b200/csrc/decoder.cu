@@ -46,6 +46,22 @@ __device__ __forceinline__ NbFwd nb_forward(float t, float lp, float ls, float p
     return o;
 }
 
+// The same element in float64 from the fp32 rates: the per-element value of the element pass (PASS_ELEM).  Summed into a per-cell
+// term, the fp32 form's absolute errors (lgamma(t + theta) - lgamma(theta) of a gene with theta ~ e^9 carries ~1e-2 of fp32
+// rounding; theta (log(theta + eps) - log(theta + rho + eps)) cancels likewise) are small against the sum, but one element's
+// value can be smaller than them.  Off the training step, so the float64 cost does not matter.
+static __device__ __noinline__ float nb_ll_f64(double t, double rp, double rs, double pi, double th) {
+    const double eps = 1e-8;
+    const double lte = log(th + eps), l1 = log(th + rp + eps), l2 = log(th + rs + eps);
+    const double lg = t != 0.0 ? lgamma(t + th) - lgamma(th) - lgamma(t + 1.0) : 0.0;
+    const double a = th * (lte - l1) + t * (log(rp + eps) - l1) + lg;
+    const double b = th * (lte - l2) + t * (log(rs + eps) - l2) + lg - pi;
+    const double mx = fmax(a, b);
+    const double lse = mx + log1p(exp(-fabs(a - b)));
+    const double softplus_neg_pi = fmax(-pi, 0.0) + log1p(exp(-fabs(pi)));
+    return (float)(lse - softplus_neg_pi);
+}
+
 struct NbBwd { float dyp, dys, dpi, dth; };
 
 // scale = upstream d loss / d ll  (= -grad_scale / B)
@@ -97,9 +113,10 @@ struct DecP {
     float scale;
     int pi_ready;                                        // PASS_NB: pi already holds the mixture logits (tensor-core GEMM)
     __nv_bfloat16* dpi_bf16; long ld_dpi_bf16;           // PASS_BWD: write d pi as bf16 (operand of the tensor-core GEMMs)
+    float* eo[5]; long ld_out;                           // PASS_ELEM: ll, rate_p, rate_s, pi, mean [B, ld_out] (NULL = not written)
 };
 
-enum { PASS_STATS = 0, PASS_NB = 1, PASS_BWD = 2 };
+enum { PASS_STATS = 0, PASS_NB = 1, PASS_BWD = 2, PASS_ELEM = 3 };
 
 template <int PASS, int SRC>
 __global__ void __launch_bounds__(GT_THREADS) dec_tile_kernel(DecP p) {
@@ -117,7 +134,7 @@ __global__ void __launch_bounds__(GT_THREADS) dec_tile_kernel(DecP p) {
     const float* azz = p.zz;
     tile_mainloop<SPV_SRC_F32, false, SPV_SRC_F32, true>(lp, azz, p.ld_zz, nullptr, p.wfold, KZ, nullptr, B, G, 0, p.P, m0, n0, sm);
     tile_mainloop<SPV_SRC_F32, false, SPV_SRC_F32, true>(ls, azz + p.P, p.ld_zz, nullptr, p.wfold + p.P, KZ, nullptr, B, G, 0, p.S, m0, n0, sm);
-    if (PASS == PASS_NB && !p.pi_ready)
+    if ((PASS == PASS_NB || PASS == PASS_ELEM) && !p.pi_ready)
         tile_mainloop<SPV_SRC_F32, false, SPV_SRC_F32, true>(pi, p.amix, p.ld_amix, nullptr, p.wm, KMIX, nullptr, B, G, 0, KMIX, m0, n0, sm);
 
     // per-gene constants of this thread's 4 genes
@@ -133,8 +150,8 @@ __global__ void __launch_bounds__(GT_THREADS) dec_tile_kernel(DecP p) {
         if (PASS != PASS_STATS) {
             th[j] = p.genec[GC_THETA * (long)G + nn];
             lte[j] = p.genec[GC_LTE * (long)G + nn];
-            lgx[j] = p.genec[(PASS == PASS_NB ? GC_LGT : GC_DGT) * (long)G + nn];
-            bm[j] = PASS == PASS_NB ? p.bm[nn] : 0.0f;
+            lgx[j] = p.genec[(PASS != PASS_BWD ? GC_LGT : GC_DGT) * (long)G + nn];
+            bm[j] = PASS != PASS_BWD ? p.bm[nn] : 0.0f;
         }
     }
 
@@ -165,6 +182,43 @@ __global__ void __launch_bounds__(GT_THREADS) dec_tile_kernel(DecP p) {
             if (tx == 0 && m < B) {
                 float* o = p.part_stats + ((long)blockIdx.x * B + m) * 4;
                 o[0] = mp; o[1] = sp; o[2] = ms; o[3] = ss;
+            }
+        }
+        return;
+    }
+
+    if (PASS == PASS_ELEM) {  // the elements of the likelihood sweep, stored instead of reduced
+        const int n = n0 + tx * 4;
+        const bool vec = n + 3 < G && (p.ld_out & 3) == 0;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const int m = m0 + ty * 4 + i;
+            if (m >= B) break;
+            const float Rp = p.rowc[(long)m * 4 + 0], Rs = p.rowc[(long)m * 4 + 1];
+            const long xr = (p.rows ? (long)p.rows[m] : (long)m) * p.ldx;
+            float v[5][4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const float piv = p.pi_ready ? (nok[j] ? p.pi[(long)m * G + n + j] : 0.0f) : pi[i][j] + bm[j];
+                const float lpj = lp[i][j] + cp[j], lsj = ls[i][j] + cs[j];
+                v[1][j] = expf(lpj + Rp);  // the rates as nb_forward forms them
+                v[2][j] = expf(lsj + Rs);
+                v[0][j] = (p.eo[0] && nok[j]) ? nb_ll_f64(load_src<SRC>(p.X, xr + n + j), v[1][j], v[2][j], piv, th[j]) : 0.0f;
+                v[3][j] = piv;
+                v[4][j] = v[1][j] / (1.0f + expf(-piv)) + v[2][j] / (1.0f + expf(piv));
+            }
+#pragma unroll
+            for (int o = 0; o < 5; ++o) {
+                float* dst = p.eo[o];
+                if (!dst) continue;
+                dst += (long)m * p.ld_out + n;
+                if (vec && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+                    *reinterpret_cast<float4*>(dst) = make_float4(v[o][0], v[o][1], v[o][2], v[o][3]);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        if (nok[j]) dst[j] = v[o][j];
+                }
             }
         }
         return;
@@ -379,6 +433,8 @@ static void fill_decp(DecP& p, const void* const* ptrs, long long ldx, long long
     p.dyp = (float*)ptrs[12]; p.dys = (float*)ptrs[13]; p.dpi = (float*)ptrs[14]; p.colpart = (float*)ptrs[15];
     p.ldx = ldx; p.ld_amix = ld_amix; p.B = B; p.G = G; p.HD = HD; p.P = P; p.S = S; p.scale = scale;
     p.pi_ready = 0; p.dpi_bf16 = nullptr; p.ld_dpi_bf16 = 0;
+    for (float*& o : p.eo) o = nullptr;
+    p.ld_out = 0;
     p.zz = zzb ? zzb : p.amix + HD;
     p.ld_zz = zzb ? ld_zzb : ld_amix;
     p.kmix = kmix > 0 ? kmix : HD + P + S;
@@ -413,6 +469,35 @@ extern "C" int spv_dec_nb_fwd(int src, const void* const* ptrs, long long ldx, l
         rownb_kernel<<<(B + 7) / 8, 256, 0, st>>>(p.part_nb, nTG, B, p.rowc, (float*)ptrs[16]);
         SPV_CHECK_LAUNCH();
     }
+    return SPV_OK;
+}
+
+// Element pass: the per-element outputs of phase 2, stored into `outs` (a HOST array of 5 device pointers [B, ld_out], NULL = not
+// written: ll, rate_p, rate_s, pi, mean) after phase 1 has left the normalisers in rowc.  pi_ready: the mixture logits are in
+// ptrs[10] (tensor-core GEMM), else they are computed here.  src SPV_SRC_F32 reads ptrs[0] as target values (no log1p).
+extern "C" int spv_dec_nb_elems(int src, const void* const* ptrs, long long ldx, long long ld_amix, int B, int G, int HD, int P,
+                                int S, int pi_ready, const float* zzb, long long ld_zzb, int kmix, void* const* outs,
+                                long long ld_out, void* stream) {
+    if (!ptrs || !outs || B <= 0 || G <= 0 || HD < 0 || P <= 0 || S <= 0 || ld_out < G) return SPV_ERR_ARG;
+    if (src != SPV_SRC_F32 && src != SPV_SRC_U16_LOG1P && src != SPV_SRC_F32_LOG1P) return SPV_ERR_ARG;
+    const int need[] = {2, 3, 5, 6, 9};
+    for (int i : need)
+        if (!ptrs[i]) return SPV_ERR_ARG;
+    if (pi_ready ? !ptrs[10] : !ptrs[4]) return SPV_ERR_ARG;
+    bool any = false;
+    for (int o = 0; o < 5; ++o) any = any || outs[o] != nullptr;
+    if (!any || (outs[0] && !ptrs[0])) return SPV_ERR_ARG;
+    DecP p;
+    fill_decp(p, ptrs, ldx, ld_amix, B, G, HD, P, S, 0.0f, zzb, ld_zzb, kmix);
+    p.pi_ready = pi_ready ? 1 : 0;
+    for (int o = 0; o < 5; ++o) p.eo[o] = reinterpret_cast<float*>(outs[o]);
+    p.ld_out = ld_out;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    dim3 grid((G + GT_BN - 1) / GT_BN, (B + GT_BM - 1) / GT_BM);
+    if (src == SPV_SRC_F32) dec_tile_kernel<PASS_ELEM, SPV_SRC_F32><<<grid, GT_THREADS, 0, st>>>(p);
+    else if (src == SPV_SRC_U16_LOG1P) dec_tile_kernel<PASS_ELEM, SPV_SRC_U16_LOG1P><<<grid, GT_THREADS, 0, st>>>(p);
+    else dec_tile_kernel<PASS_ELEM, SPV_SRC_F32_LOG1P><<<grid, GT_THREADS, 0, st>>>(p);
+    SPV_CHECK_LAUNCH();
     return SPV_OK;
 }
 

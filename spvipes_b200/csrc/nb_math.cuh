@@ -123,6 +123,10 @@ static __device__ __noinline__ float2 nb_count_terms_fwd_slow(float xraw, float 
     const float t = log1pf(xraw);
     return make_float2(t, xraw > 0.0f ? lgammaf(t + th) - lgt - lgammaf(t + 1.0f) : 0.0f);
 }
+// ... of a target value t given as it is (SPV_SRC_F32: px.log_prob(value) at an arbitrary value)
+static __device__ __noinline__ float2 nb_target_terms_fwd(float t, float th, float lgt) {
+    return make_float2(t, t != 0.0f ? lgammaf(t + th) - lgt - lgammaf(t + 1.0f) : 0.0f);
+}
 static __device__ __noinline__ float2 nb_count_terms_bwd_slow(float xraw, float th, float dgt) {
     const float t = log1pf(xraw);
     return make_float2(t, xraw > 0.0f ? digammaf_pos(t + th) - dgt : 0.0f);
@@ -171,6 +175,9 @@ __device__ __forceinline__ uint32_t nb_pair_codes(uint2 raw) {
         const uint32_t lo = (w & 0xfff0u) ? NB_CODE_SLOW : (w & 0xffffu) << 3;
         const uint32_t hi = (w & 0xfff00000u) ? NB_CODE_SLOW : (w >> 16) << 3;
         return lo | (hi << 16);
+    } else if (SRC == 0 /* SPV_SRC_F32: target values t, not counts */) {
+        // the tables are indexed by count (t = log1p(c)); a target hits them only at t = 0 = log1p(0), entry 0
+        return (__uint_as_float(raw.x) == 0.0f ? 0u : NB_CODE_SLOW) | ((__uint_as_float(raw.y) == 0.0f ? 0u : NB_CODE_SLOW) << 16);
     } else {
         return nb_code_f32(__uint_as_float(raw.x)) | (nb_code_f32(__uint_as_float(raw.y)) << 16);
     }

@@ -46,6 +46,17 @@ constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 2 * B_BYTES + 1024 + BN * 16 +
 static_assert(BM * CNT_PITCH_W * 4 <= STAGES * STAGE_BYTES, "count tile must fit in the operand stages");
 static_assert(3 * (SMEM_BYTES + 1024) <= 228 * 1024, "three CTAs per SM");
 
+// Element sweep (ELEM variant): five optional fp32 outputs per element, in this order (spv_dec_nb_elems_tc)
+enum { EO_LL = 0, EO_RATE_P, EO_RATE_S, EO_PI, EO_MEAN, EO_N };
+// Each epilogue warp stages a 32-cell x EO_CH-gene slab per output in the operand stages and the folded-weight tiles (both free
+// once the accumulators are complete), behind the count tile; lane -> (cell lane / EO_CH + 32 / EO_CH * k, gene lane % EO_CH)
+// then makes every warp store four whole 32-byte sectors instead of 32 rows x 16 bytes.  Pitch EO_CH + 1: the thread = cell
+// writes are conflict-free.
+constexpr int EO_CH = 8, EO_PITCH = EO_CH + 1;
+constexpr int EO_SLAB_OFF = BM * CNT_PITCH_W * 4;
+constexpr int EO_WARP_FLOATS = EO_N * 32 * EO_PITCH;
+static_assert(EO_SLAB_OFF + EPI_WARPS * EO_WARP_FLOATS * 4 <= STAGES * STAGE_BYTES + 2 * B_BYTES, "element slabs must fit");
+
 struct NbTcParams {
     const void* X; long ldx; const int* rows;
     const float* bm;                   // [G]
@@ -55,6 +66,8 @@ struct NbTcParams {
     int B, G, K;
     int Gp;                            // row offset of the shared block inside the folded-weight operand
     long long* trace;                  // diagnostic (NB_TRACE builds): 6 globaltimer stamps per CTA
+    float* eo[EO_N];                   // ELEM variant: the outputs [B, ld_out] (NULL = not written)
+    long ld_out;
 };
 
 // row of the count tile that lane `lane` of epilogue warp e loads in its i-th gather: a warp covers GATHER_ROWS rows per load
@@ -70,15 +83,21 @@ template <int SRC>
 __device__ __noinline__ NbOut nb_fwd_general(uint32_t code, float xp, float xs, float acc_pi, float4 gc, const uint8_t* tg_row,
                                              const void* X, long xidx, const float* lgt) {
     float2 tcn;
-    if (code == NB_CODE_SLOW) tcn = nb_count_terms_fwd_slow(nb_load_raw<SRC>(X, xidx), gc.x, __ldg(lgt));
+    if (code == NB_CODE_SLOW) {
+        if (SRC == SPV_SRC_F32) tcn = nb_target_terms_fwd(nb_load_raw<SRC>(X, xidx), gc.x, __ldg(lgt));
+        else tcn = nb_count_terms_fwd_slow(nb_load_raw<SRC>(X, xidx), gc.x, __ldg(lgt));
+    }
     else tcn = *reinterpret_cast<const float2*>(tg_row + code);
     const float pi = acc_pi + gc.w;
     if (tcn.x != 0.0f && fminf(xp, xs) < NB_X_RARE) return nb_forward_v5<true>(tcn.x, tcn.y, xp, xs, pi, gc.x, gc.y, gc.z);
     return nb_forward_v5<false>(tcn.x, tcn.y, xp, xs, pi, gc.x, gc.y, gc.z);
 }
 
-template <int SRC>
-__global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_constant__ CUtensorMap mapA,
+// ELEM = false: the reducing sweep (row partials of the log-likelihood).  ELEM = true: the element sweep - the same MMAs and the
+// same element math, but the epilogue stores the per-element outputs selected in p.eo (no partials) and gathers the counts only
+// when the log-likelihood is requested.  It is not on the training step and gives up the third resident CTA.
+template <int SRC, bool ELEM = false>
+__global__ void __launch_bounds__(THREADS, ELEM ? 2 : 3) nb_tc_fwd_kernel(const __grid_constant__ CUtensorMap mapA,
                                                                const __grid_constant__ CUtensorMap mapB,
                                                                const __grid_constant__ CUtensorMap mapZ,
                                                                const __grid_constant__ CUtensorMap mapZc, NbTcParams p) {
@@ -236,6 +255,7 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
             ridx[i] = gm < p.B ? (p.rows ? __ldg(p.rows + gm) : gm) : -1;
         }
         const int my_row = p.rows ? __ldg(p.rows + mm) : mm;
+        const bool counts = !ELEM || p.eo[EO_LL] != nullptr;  // CTA-uniform
         float4 gcv = make_float4(1.0f, 1.0f, 0.0f, 0.0f);
         static_assert(BN <= EPI_THREADS, "one thread per gene of the tile stages its constants");
         if (et < BN && n0 + et < p.G) {
@@ -247,9 +267,10 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
         }
         // the tile's slice of the count table: BN * NB_TAB * 8 bytes = 2 x 16 bytes per epilogue thread
         static_assert(BN * NB_TAB * 8 == EPI_THREADS * 32, "two 16-byte table words per epilogue thread");
-        float4 tgv[2];
+        float4 tgv[2] = {};
 #pragma unroll
         for (int u = 0; u < 2; ++u) {
+            if (!counts) break;
             const int w16 = et + u * EPI_THREADS;          // 16-byte word of the slice: gene w16 / 8
             const int g = n0 + (w16 >> 3);
             tgv[u] = g < p.G ? __ldg(reinterpret_cast<const float4*>(p.tgf + (long)n0 * NB_TAB) + w16) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
@@ -262,7 +283,8 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
 #pragma unroll
             for (int i = 0; i < NGATHER; ++i) cw[i] = 0u;
             constexpr int BATCH = SRC == SPV_SRC_U16_LOG1P ? NGATHER : NGATHER / 2;  // every load of a batch in flight before any is used
-            if (nb_pair_vec_ok<SRC>(p.X, p.ldx, g, p.G)) {
+            if (!counts) {
+            } else if (nb_pair_vec_ok<SRC>(p.X, p.ldx, g, p.G)) {
 #pragma unroll
                 for (int i0 = 0; i0 < NGATHER; i0 += BATCH) {
                     uint2 raw[BATCH];
@@ -282,7 +304,8 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
         }
         if (et < BN) s_gc[et] = gcv;
 #pragma unroll
-        for (int u = 0; u < 2; ++u) reinterpret_cast<float4*>(s_tg)[et + u * EPI_THREADS] = tgv[u];
+        for (int u = 0; u < 2; ++u)
+            if (counts) reinterpret_cast<float4*>(s_tg)[et + u * EPI_THREADS] = tgv[u];
         const long xrow = (long)my_row * p.ldx;
         stamp(2);  // count gather issued
         tc::mbar_wait(tmem_ready, 0);
@@ -292,13 +315,73 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
         tc::fence_after_sync();
         stamp(3);  // accumulators complete
 #pragma unroll
-        for (int i = 0; i < NGATHER; ++i) s_cnt[cnt_row(e, lane, i) * CNT_PITCH_W + lane % (BN / 2)] = cw[i];
+        for (int i = 0; i < NGATHER; ++i)
+            if (counts) s_cnt[cnt_row(e, lane, i) * CNT_PITCH_W + lane % (BN / 2)] = cw[i];
         asm volatile("bar.sync 1, %0;" ::"r"(EPI_THREADS) : "memory");  // constants + counts staged (epilogue warps only)
         stamp(4);  // counts staged
+        const uint32_t* cnt_row_p = s_cnt + rloc * CNT_PITCH_W + half * (WCOLS / 2);
+        if constexpr (ELEM) {
+            const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16), lane_z = tmem_z + ((uint32_t)(q * 32) << 16);
+            float* slab = reinterpret_cast<float*>(tiles + EO_SLAB_OFF) + e * EO_WARP_FLOATS;
+#pragma unroll 1
+            for (int j8 = 0; j8 < WCOLS; j8 += EO_CH) {
+#pragma unroll
+                for (int j4 = j8; j4 < j8 + EO_CH; j4 += 4) {
+                    const int c0 = half * WCOLS + j4;
+                    uint32_t rpi[4], rlp[4], rls[4];
+                    tc::tmem_ld4(lane_addr + (uint32_t)c0, rpi);
+                    tc::tmem_ld4(lane_z + (uint32_t)c0, rlp);
+                    tc::tmem_ld4(lane_z + (uint32_t)(BN + c0), rls);
+                    const uint2 cc = counts ? *reinterpret_cast<const uint2*>(cnt_row_p + (j4 >> 1)) : make_uint2(0u, 0u);
+                    tc::tmem_ld_wait();
+#pragma unroll
+                    for (int jj = 0; jj < 4; ++jj) {
+                        const int gl = c0 + jj, g = n0 + gl;
+                        const float4 gc = s_gc[gl];
+                        const float xp = __uint_as_float(rlp[jj]), xs = __uint_as_float(rls[jj]), pi = __uint_as_float(rpi[jj]) + gc.w;
+                        float ll = 0.0f;
+                        if (counts && mok && g < p.G) {  // the element form the reducing sweep takes for this element
+                            const uint32_t w = jj < 2 ? cc.x : cc.y;
+                            const uint32_t code = (jj & 1) ? (w >> 16) : (w & 0xffffu);
+                            if (code == NB_CODE_SLOW) {
+                                ll = nb_fwd_general<SRC>(code, xp, xs, __uint_as_float(rpi[jj]), gc, s_tg + gl * (NB_TAB * 8), p.X, xrow + g,
+                                                         p.genec + GC_LGT * G + g).ll;
+                            } else {
+                                const float2 tcn = *reinterpret_cast<const float2*>(s_tg + gl * (NB_TAB * 8) + code);
+                                if (tcn.x != 0.0f && fminf(xp, xs) < NB_X_RARE) ll = nb_forward_v5<true>(tcn.x, tcn.y, xp, xs, pi, gc.x, gc.y, gc.z).ll;
+                                else ll = nb_forward_v5<false>(tcn.x, tcn.y, xp, xs, pi, gc.x, gc.y, gc.z).ll;
+                            }
+                        }
+                        const float rp = fast_ex2(xp), rs = fast_ex2(xs);
+                        // sigma(pi) and sigma(-pi) each in its accurate form (neither is 1 minus the other): mean keeps its digits
+                        // at mixture logits of either sign
+                        const float sg = 1.0f / (1.0f + __expf(-pi)), sn = 1.0f / (1.0f + __expf(pi));
+                        float* s = slab + lane * EO_PITCH + (j4 - j8 + jj);
+                        s[EO_LL * 32 * EO_PITCH] = ll;
+                        s[EO_RATE_P * 32 * EO_PITCH] = rp;
+                        s[EO_RATE_S * 32 * EO_PITCH] = rs;
+                        s[EO_PI * 32 * EO_PITCH] = pi;
+                        s[EO_MEAN * 32 * EO_PITCH] = fmaf(sg, rp, sn * rs);
+                    }
+                }
+                __syncwarp();
+                const int col = lane % EO_CH, g = n0 + half * WCOLS + j8 + col;
+#pragma unroll
+                for (int o = 0; o < EO_N; ++o) {
+                    float* dst = p.eo[o];
+                    if (dst == nullptr) continue;
+#pragma unroll
+                    for (int r = lane / EO_CH; r < 32; r += 32 / EO_CH) {
+                        const int m = m0 + q * 32 + r;
+                        if (m < p.B && g < p.G) dst[(long)m * p.ld_out + g] = slab[(o * 32 + r) * EO_PITCH + col];
+                    }
+                }
+                __syncwarp();
+            }
+        } else {
         float sll = 0.0f, sep = 0.0f, ses = 0.0f;
         const bool full_tile = n0 + BN <= p.G && m0 + BM <= p.B;  // CTA-uniform
         const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16), lane_z = tmem_z + ((uint32_t)(q * 32) << 16);
-        const uint32_t* cnt_row_p = s_cnt + rloc * CNT_PITCH_W + half * (WCOLS / 2);
 #pragma unroll 1
         for (int j4 = 0; j4 < WCOLS; j4 += 4) {
             const int c0 = half * WCOLS + j4;
@@ -342,6 +425,7 @@ __global__ void __launch_bounds__(THREADS, 3) nb_tc_fwd_kernel(const __grid_cons
         if (mok) {
             float* o = p.part_nb + ((long)(blockIdx.x * 2 + half) * p.B + m) * 3;
             o[0] = sll; o[1] = sep; o[2] = ses;
+        }
         }
         stamp(5);  // epilogue done
     }
@@ -569,6 +653,54 @@ extern "C" int spv_dec_nb_fwd_tc(int src, const void* const* ptrs, long long ldx
     if (src == SPV_SRC_U16_LOG1P) nb_tc_fwd_kernel<SPV_SRC_U16_LOG1P><<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, mz, mzc, p);
     else if (src == SPV_SRC_F32_LOG1P) nb_tc_fwd_kernel<SPV_SRC_F32_LOG1P><<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, mz, mzc, p);
     else return SPV_ERR_ARG;
+    SPV_CHECK_LAUNCH();
+    return SPV_OK;
+}
+
+// Element sweep: the operands and ptrs of spv_dec_nb_fwd_tc (ptrs[11], the row partials, unused), outputs in `outs` (a HOST array
+// of EO_N device pointers, see the header).  The counts (ptrs[0], ptrs[1]) and the count table (ptrs[17]) are read only when the
+// log-likelihood is requested; src SPV_SRC_F32 reads ptrs[0] as target values t (no log1p).
+extern "C" int spv_dec_nb_elems_tc(int src, const void* const* ptrs, long long ldx, const void* amix_bf16, long long ld_amixb,
+                                   const void* wstack_bf16, long long ld_w, int Gp, const void* zc_f16, const void* wz_f16, int B,
+                                   int G, int HD, int P, int S, int kmix, void* const* outs, long long ld_out, void* stream) {
+    if (!ptrs || !outs || !amix_bf16 || !wstack_bf16 || !zc_f16 || !wz_f16 || Gp < G || B <= 0 || G <= 0 || HD < 0 || P <= 0 ||
+        S <= 0 || ld_out < G)
+        return SPV_ERR_ARG;
+    if (P + S > ZK_MAX_LATENT) return SPV_ERR_ARG;
+    if (src != SPV_SRC_F32 && src != SPV_SRC_U16_LOG1P && src != SPV_SRC_F32_LOG1P) return SPV_ERR_ARG;
+    if (!ptrs[5] || !ptrs[6]) return SPV_ERR_ARG;
+    bool any = false;
+    for (int o = 0; o < EO_N; ++o) any = any || outs[o] != nullptr;
+    if (!any) return SPV_ERR_ARG;
+    if (outs[EO_LL] && (!ptrs[0] || !ptrs[17] || (reinterpret_cast<uintptr_t>(ptrs[17]) & 15))) return SPV_ERR_ARG;
+    const int K = kmix > 0 ? kmix : HD + P + S;
+    CUtensorMap ma, mb, mz, mzc;
+    int rc = spv_make_tensor_map_bf16(&ma, amix_bf16, (unsigned long long)K, (unsigned long long)B, (unsigned long long)ld_amixb, 64, BM);
+    if (rc != SPV_OK) return rc;
+    rc = spv_make_tensor_map_bf16(&mb, wstack_bf16, (unsigned long long)K, (unsigned long long)G, (unsigned long long)ld_w, 64, BN);
+    if (rc != SPV_OK) return rc;
+    rc = spv_make_tensor_map_bf16(&mz, wz_f16, 64ull, (unsigned long long)(2 * Gp), 64ull, 64, BN);
+    if (rc != SPV_OK) return rc;
+    rc = spv_make_tensor_map_bf16(&mzc, zc_f16, 64ull, (unsigned long long)B, 64ull, 64, BM);
+    if (rc != SPV_OK) return rc;
+    NbTcParams p{};
+    p.Gp = Gp;
+    p.X = ptrs[0]; p.ldx = ldx; p.rows = (const int*)ptrs[1]; p.bm = (const float*)ptrs[5]; p.genec = (const float*)ptrs[6];
+    p.tgf = (const float2*)ptrs[17]; p.part_nb = nullptr;
+    p.B = B; p.G = G; p.K = K;
+    p.trace = nullptr;
+    for (int o = 0; o < EO_N; ++o) p.eo[o] = reinterpret_cast<float*>(outs[o]);
+    p.ld_out = ld_out;
+    static bool done[3][64] = {};
+    if (set_smem_once(nb_tc_fwd_kernel<SPV_SRC_F32, true>, SMEM_BYTES, done[0]) != SPV_OK ||
+        set_smem_once(nb_tc_fwd_kernel<SPV_SRC_U16_LOG1P, true>, SMEM_BYTES, done[1]) != SPV_OK ||
+        set_smem_once(nb_tc_fwd_kernel<SPV_SRC_F32_LOG1P, true>, SMEM_BYTES, done[2]) != SPV_OK)
+        return SPV_ERR_LAUNCH;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    dim3 grid((G + BN - 1) / BN, (B + BM - 1) / BM);
+    if (src == SPV_SRC_F32) nb_tc_fwd_kernel<SPV_SRC_F32, true><<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, mz, mzc, p);
+    else if (src == SPV_SRC_U16_LOG1P) nb_tc_fwd_kernel<SPV_SRC_U16_LOG1P, true><<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, mz, mzc, p);
+    else nb_tc_fwd_kernel<SPV_SRC_F32_LOG1P, true><<<grid, THREADS, SMEM_BYTES, st>>>(ma, mb, mz, mzc, p);
     SPV_CHECK_LAUNCH();
     return SPV_OK;
 }

@@ -69,6 +69,8 @@ class Dims:
 
 
 PHASE_ENC, PHASE_DEC = 0, 1
+# per-element decoder outputs of decode_elements, in the order of the kernels' output array (include/spvipes_b200.h)
+ELEM_OUTPUTS = ("ll", "rate_p", "rate_s", "pi", "mean")
 _ENCODER_BLOCKS = ("W1", "b1", "W2", "b2", "Whp", "Whs", "bhd", "ghd", "bthd")
 
 
@@ -444,6 +446,9 @@ class StepEngine:
         # the tensor core's operand reads share the shared-memory pipe.
         self.fused_fc1 = os.environ.get("SPV_FUSED_FC1", "0") == "1"
         self.nb_events = None  # bench hook: iterator of (start, end) CUDA events bracketing the NB-loglik sweep
+        # advanced by every forward and every backward pass, eager or replayed from a CUDA graph (note_replay): a pass's decoder
+        # state in the workspaces (what decode_elements reads) is current while the generation is the one it was made in
+        self.generation = 0
 
     # -------------------------------------------------------------------------------- helpers
     def P(self, g, name):
@@ -582,6 +587,7 @@ class StepEngine:
                 with_grad: Optional[bool] = None, decode: bool = True):
         """inference -> generative -> loss.  Returns the workspaces (device tensors) holding every output."""
         with_grad = training if with_grad is None else with_grad
+        self.generation += 1
         ctx = self._encode(batches, training, noise, with_grad, stage_wm=decode)
         if not decode:
             for g in (0, 1):
@@ -714,96 +720,189 @@ class StepEngine:
         aux = self._pairing(batches, ws, Bs)
         self._poe_fwd(ws, Bs, noise, aux)
         ctx = {"batches": batches, "ws": ws, "Bs": Bs, "noise": noise, "srcs": srcs, "aux": aux, "training": training,
-               "with_grad": with_grad, "wm_staged": (not convert) or decode or self.stage_in_adam}
+               "with_grad": with_grad, "wm_staged": (not convert) or decode or self.stage_in_adam, "gen": self.generation}
         self._ctx = ctx
         return ctx
 
+    def note_replay(self, forward: bool):
+        """a CUDA graph replayed a forward (forward=True; with its decoder, whose state is then current) or a backward pass of this
+        engine: advance the generation as forward() / backward() do"""
+        self.generation += 1
+        if forward and self._ctx is not None:
+            self._ctx["dec_gen"] = self.generation
+
     def _decode(self, ctx):
-        d, st, lib = self.d, self._stream(), self.lib
+        # ---------------- decoders + NB likelihood (reference nn/networks.py:314-325, module :751-759, :817-824)
+        Bs, ws = ctx["Bs"], ctx["ws"]
+        for g in self._fork_groups():
+            self._dec_prologue(ctx, g)
+            self._dec_sweep(ctx, g)
+        ctx["dec_gen"] = self.generation
+        if Bs[0] != Bs[1]:
+            raise ValueError("the loss needs equally sized minibatches in both groups (reference :886-893)")
+        L.check(self.lib.spv_loss(L.ptr(ws[0].rec), L.ptr(ws[1].rec), L.ptr(ws[0].klp), L.ptr(ws[0].klq), L.ptr(ws[1].klp),
+                                  L.ptr(ws[1].klq), Bs[0], L.ptr(self.kl_weight), L.ptr(self.loss_out), self._stream()), "spv_loss")
+        return ws
+
+    def _dec_prologue(self, ctx, g):
+        """group g's decoder up to the likelihood sweep: mixture-weight staging, covariate expansion, count tables, hidden layer,
+        BatchNorm fold and softmax normalisers (on the current stream of _fork_groups)"""
+        d, lib = self.d, self.lib
         H, S, P, KZ, KMIX, NST = d.n_hidden, d.n_shared, d.n_private, d.KZ, d.KMIX, d.NST
         batches, ws, Bs, srcs, training, with_grad = ctx["batches"], ctx["ws"], ctx["Bs"], ctx["srcs"], ctx["training"], ctx["with_grad"]
         tr = 1 if training else 0
-        # ---------------- decoders + NB likelihood (reference nn/networks.py:314-325, module :751-759, :817-824)
-        for g in self._fork_groups():
-            bt, w, st = batches[g], ws[g], self._stream()
-            G, B = d.genes[g], Bs[g]
-            src, xptr, ldx, count_rows = srcs[g]
-            if self.bf16 and not ctx["wm_staged"]:  # decode() after an encoder-only pass: the mixture weight's bf16 copy
-                self._to_dec(L.ptr(self.P(g, "Wm")), KMIX, L.ptr(w.Wmb), w.KMp, G, KMIX)
-            zzp = w.amix.data_ptr() + 4 * HD
-            nb, Pb, Sb, KZb = d.nb, d.Pb, d.Sb, d.KZb
-            # zb / ld_zb: the two factor regressors' inputs side by side.  Without covariates these are the latent columns of
-            # amix; with them each regressor's input carries its own copy of the one-hot columns (spv_cov_expand, which also
-            # fills the covariate columns behind [hm | zz] in amix)
-            zb, ld_zb = zzp, KMIX
-            if nb:
-                L.check(lib.spv_cov_expand(zzp, KMIX, L.ptr(bt.batch), L.ptr(w.zzb), KZb, zzp + 4 * KZ, KMIX, B, P, S, nb, st),
-                        "spv_cov_expand")
-                zb, ld_zb = L.ptr(w.zzb), KZb
-            fold = L.ptr_array([self.P(g, "Wp"), self.P(g, "Ws"), self.P(g, "gp"), self.P(g, "bp"), self.P(g, "gs"),
-                                self.P(g, "bs"), self.P(g, "px_r"), self.Bf(g, "rm_p"), self.Bf(g, "rv_p"),
-                                self.Bf(g, "rm_s"), self.Bf(g, "rv_s"), zb, w.zsum, w.cov_part, w.wfold, w.genec, w.zmean,
-                                w.zcov])
-            wz = w.Wstack.data_ptr() + 2 * w.Gp * w.KMp if self.fused_nb else None
-            if self.fused_nb:
-                # count tables of the likelihood sweeps: a function of px_r only, on the second auxiliary stream
-                with self._branch(g, "tg", lane=1):
-                    L.check(lib.spv_dec_theta_tables(L.ptr(self.P(g, "px_r")), G, L.ptr(w.tgf), L.ptr(w.tb1), self._stream()),
-                            "spv_dec_theta_tables")
-                # hidden layer of the mixing net (needs only zz) on the auxiliary stream, beside latent stats / fold / normalisers;
-                # the bf16 operand [hm | zz] of the mixture GEMM in one conversion pass after it
-                with self._branch(g, "hm"):
-                    self._hidden_mix(g, w, B, tr, zzp)
-                    self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
-            L.check(lib.spv_dec_fold(fold, ld_zb, B, G, Pb, Sb, tr, DEC_BN_EPS, DEC_BN_MOM, wz, w.KMp if self.fused_nb else 0,
-                                     w.Gp, HD, L.ptr(w.wzf) if self.fused_nb else None, L.ptr(w.zcb) if self.fused_nb else None, st),
-                    "spv_dec_fold")
-            if self.fused_nb:  # softmax normalisers on the tensor cores (main stream: latent stats -> fold -> normalisers)
-                self._join(g, "lib")
-                L.check(lib.spv_dec_stats_tc(L.ptr(w.zcb), L.ptr(w.wzf), w.Gp, L.ptr(w.genec), L.ptr(w.lib),
-                                             L.ptr(w.part_stats), L.ptr(w.rowc), B, G, Pb, Sb, st), "spv_dec_stats_tc")
-                self._join(g, "hm")
-            else:
+        bt, w, st = batches[g], ws[g], self._stream()
+        G, B = d.genes[g], Bs[g]
+        src, xptr, ldx, count_rows = srcs[g]
+        if self.bf16 and not ctx["wm_staged"]:  # decode() after an encoder-only pass: the mixture weight's bf16 copy
+            self._to_dec(L.ptr(self.P(g, "Wm")), KMIX, L.ptr(w.Wmb), w.KMp, G, KMIX)
+        zzp = w.amix.data_ptr() + 4 * HD
+        nb, Pb, Sb, KZb = d.nb, d.Pb, d.Sb, d.KZb
+        # zb / ld_zb: the two factor regressors' inputs side by side.  Without covariates these are the latent columns of
+        # amix; with them each regressor's input carries its own copy of the one-hot columns (spv_cov_expand, which also
+        # fills the covariate columns behind [hm | zz] in amix)
+        zb, ld_zb = zzp, KMIX
+        if nb:
+            L.check(lib.spv_cov_expand(zzp, KMIX, L.ptr(bt.batch), L.ptr(w.zzb), KZb, zzp + 4 * KZ, KMIX, B, P, S, nb, st),
+                    "spv_cov_expand")
+            zb, ld_zb = L.ptr(w.zzb), KZb
+        fold = L.ptr_array([self.P(g, "Wp"), self.P(g, "Ws"), self.P(g, "gp"), self.P(g, "bp"), self.P(g, "gs"),
+                            self.P(g, "bs"), self.P(g, "px_r"), self.Bf(g, "rm_p"), self.Bf(g, "rv_p"),
+                            self.Bf(g, "rm_s"), self.Bf(g, "rv_s"), zb, w.zsum, w.cov_part, w.wfold, w.genec, w.zmean,
+                            w.zcov])
+        wz = w.Wstack.data_ptr() + 2 * w.Gp * w.KMp if self.fused_nb else None
+        if self.fused_nb:
+            # count tables of the likelihood sweeps: a function of px_r only, on the second auxiliary stream
+            with self._branch(g, "tg", lane=1):
+                L.check(lib.spv_dec_theta_tables(L.ptr(self.P(g, "px_r")), G, L.ptr(w.tgf), L.ptr(w.tb1), self._stream()),
+                        "spv_dec_theta_tables")
+            # hidden layer of the mixing net (needs only zz) on the auxiliary stream, beside latent stats / fold / normalisers;
+            # the bf16 operand [hm | zz] of the mixture GEMM in one conversion pass after it
+            with self._branch(g, "hm"):
                 self._hidden_mix(g, w, B, tr, zzp)
-            dptrs = self._dec_ptrs(g, w, xptr, count_rows, with_grad)
-            self._join(g, "lib")
-            if not self.fused_nb:
-                L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
-            evs = next(self.nb_events) if self.nb_events is not None else None
-            if self.fused_nb:
-                self._join(g, "wm")
-                self._join(g, "tg")
-            elif self.bf16:  # mixture logits on the tensor cores, consumed by the NB sweep
                 self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
-                self._join(g, "wm")
-            if evs is not None:
-                evs[0].record()
-            if self.bf16:
-                if self.fused_nb:
-                    if training and with_grad:  # one sweep: likelihood + everything the backward needs
-                        L.check(lib.spv_dec_nb_train_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp,
-                                                        L.ptr(w.zcb), L.ptr(w.wzf), L.ptr(w.E4T), 4 * w.Bp, L.ptr(w.DPIT), w.Bp, B, G, HD,
-                                                        Pb, Sb, KMIX, st), "spv_dec_nb_train_tc")
-                    else:
-                        L.check(lib.spv_dec_nb_fwd_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb),
-                                                      L.ptr(w.wzf), B, G, HD, Pb, Sb, 0, KMIX, st), "spv_dec_nb_fwd_tc")  # backward recomputes pi
-                    if evs is not None:
-                        evs[1].record()
-                        evs = None
-                    L.check(lib.spv_dec_nb_rowreduce(L.ptr(w.part_nb), G, B, HD, L.ptr(w.rowc), L.ptr(w.rec), st), "spv_dec_nb_rowreduce")
-                else:  # unfused: tensor-core GEMM writes pi, the SIMT sweep consumes it
-                    self._tc_gemm(L.ptr(w.amixb), L.ptr(w.Wmb), L.ptr(w.pi), B, G, KMIX, lda=w.KMp, ldb=w.KMp, ldc=G,
-                                  bias=L.ptr(self.P(g, "bm")))
-                    L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 2 | 4, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
-            else:
-                L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 2, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
-            if evs is not None:
-                evs[1].record()
-        if Bs[0] != Bs[1]:
-            raise ValueError("the loss needs equally sized minibatches in both groups (reference :886-893)")
-        L.check(lib.spv_loss(L.ptr(ws[0].rec), L.ptr(ws[1].rec), L.ptr(ws[0].klp), L.ptr(ws[0].klq), L.ptr(ws[1].klp),
-                             L.ptr(ws[1].klq), Bs[0], L.ptr(self.kl_weight), L.ptr(self.loss_out), self._stream()), "spv_loss")
-        return ws
+        L.check(lib.spv_dec_fold(fold, ld_zb, B, G, Pb, Sb, tr, DEC_BN_EPS, DEC_BN_MOM, wz, w.KMp if self.fused_nb else 0,
+                                 w.Gp, HD, L.ptr(w.wzf) if self.fused_nb else None, L.ptr(w.zcb) if self.fused_nb else None, st),
+                "spv_dec_fold")
+        if self.fused_nb:  # softmax normalisers on the tensor cores (main stream: latent stats -> fold -> normalisers)
+            self._join(g, "lib")
+            L.check(lib.spv_dec_stats_tc(L.ptr(w.zcb), L.ptr(w.wzf), w.Gp, L.ptr(w.genec), L.ptr(w.lib),
+                                         L.ptr(w.part_stats), L.ptr(w.rowc), B, G, Pb, Sb, st), "spv_dec_stats_tc")
+            self._join(g, "hm")
+        else:
+            self._hidden_mix(g, w, B, tr, zzp)
+        dptrs = self._dec_ptrs(g, w, xptr, count_rows, with_grad)
+        self._join(g, "lib")
+        if not self.fused_nb:
+            L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
+
+    def _dec_sweep(self, ctx, g):
+        """group g's reducing likelihood sweep (per-cell reconstruction term; training: also what the backward needs)"""
+        d, lib = self.d, self.lib
+        KMIX = d.KMIX
+        ws, Bs, srcs, training, with_grad = ctx["ws"], ctx["Bs"], ctx["srcs"], ctx["training"], ctx["with_grad"]
+        w, st = ws[g], self._stream()
+        G, B = d.genes[g], Bs[g]
+        src, xptr, ldx, count_rows = srcs[g]
+        nb, Pb, Sb, KZb = d.nb, d.Pb, d.Sb, d.KZb
+        dptrs = self._dec_ptrs(g, w, xptr, count_rows, with_grad)
+        evs = next(self.nb_events) if self.nb_events is not None else None
+        if self.fused_nb:
+            self._join(g, "wm")
+            self._join(g, "tg")
+        elif self.bf16:  # mixture logits on the tensor cores, consumed by the NB sweep
+            self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
+            self._join(g, "wm")
+        if evs is not None:
+            evs[0].record()
+        if self.bf16:
+            if self.fused_nb:
+                if training and with_grad:  # one sweep: likelihood + everything the backward needs
+                    L.check(lib.spv_dec_nb_train_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp,
+                                                    L.ptr(w.zcb), L.ptr(w.wzf), L.ptr(w.E4T), 4 * w.Bp, L.ptr(w.DPIT), w.Bp, B, G, HD,
+                                                    Pb, Sb, KMIX, st), "spv_dec_nb_train_tc")
+                else:
+                    L.check(lib.spv_dec_nb_fwd_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb),
+                                                  L.ptr(w.wzf), B, G, HD, Pb, Sb, 0, KMIX, st), "spv_dec_nb_fwd_tc")  # backward recomputes pi
+                if evs is not None:
+                    evs[1].record()
+                    evs = None
+                L.check(lib.spv_dec_nb_rowreduce(L.ptr(w.part_nb), G, B, HD, L.ptr(w.rowc), L.ptr(w.rec), st), "spv_dec_nb_rowreduce")
+            else:  # unfused: tensor-core GEMM writes pi, the SIMT sweep consumes it
+                self._tc_gemm(L.ptr(w.amixb), L.ptr(w.Wmb), L.ptr(w.pi), B, G, KMIX, lda=w.KMp, ldb=w.KMp, ldc=G,
+                              bias=L.ptr(self.P(g, "bm")))
+                L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 2 | 4, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
+        else:
+            L.check(lib.spv_dec_nb_fwd(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 2, L.ptr(w.zzb) if nb else None, KZb, KMIX, st), "spv_dec_nb_fwd")
+        if evs is not None:
+            evs[1].record()
+
+    def _on_device(self, t):
+        dev = self.device
+        return t.device.type == dev.type and (dev.index is None or t.device.index == dev.index)
+
+    def decode_elements(self, outs, value=None):
+        """per-element decoder outputs of the current pass: outs[g] maps names of ELEM_OUTPUTS to float32 device tensors [B_g, ld]
+        (unit stride along the genes, one row pitch per group, ld >= the group's genes; a group may be omitted or map to {}):
+          ll      log_mixture_nb per element (eps 1e-8) of t = log1p(counts of the minibatch), or of value[g] (float32 [B_g, >= G_g],
+                  unit stride) as given when `value` is a sequence of two such tensors (None entries: that group's counts)
+          rate_p  px_rate_private = exp(lib) softmax(BN_p(z_private_arg Wp^T)),  rate_s  px_rate_shared
+          pi      px_mixing (the mixing logit, bias included),  mean  sigmoid(pi) rate_p + (1 - sigmoid(pi)) rate_s
+        The state is the one the pass left in the workspaces: after forward(..., decode=False) in eval mode the decoder's prologue
+        runs here (not the likelihood sweep: no loss, so the groups may differ in size).  No spv_loss, no gradient state."""
+        ctx = self._ctx
+        if ctx is None:
+            raise RuntimeError("decode_elements() follows a forward pass")
+        if ctx.get("dec_gen") != self.generation:
+            if "dec_gen" in ctx or self.generation != ctx["gen"]:
+                raise RuntimeError("the decoder state of the last forward is gone: a backward or another forward ran since")
+            if ctx["training"]:
+                raise RuntimeError("decode_elements() after a training-mode forward(..., decode=False): running the decoder here would "
+                                   "update its BatchNorm running statistics a second time; decode the training pass instead")
+        d, lib = self.d, self.lib
+        idx = {k: i for i, k in enumerate(ELEM_OUTPUTS)}
+        for g in (0, 1):
+            for k in (outs[g] or {}):
+                if k not in idx:
+                    raise ValueError(f"unknown decoder output {k!r}; choose from {ELEM_OUTPUTS}")
+        run_prologue = ctx.get("dec_gen") != self.generation
+        for g in self._fork_groups():
+            if run_prologue:
+                self._dec_prologue(ctx, g)
+            self._join(g)
+            og = outs[g] or {}
+            if not og:
+                continue
+            w, B, G, st = ctx["ws"][g], ctx["Bs"][g], d.genes[g], self._stream()
+            ld = None
+            for k, t in og.items():
+                if t.dtype != torch.float32 or not self._on_device(t) or t.dim() != 2 or t.shape[0] != B or t.shape[1] < G or \
+                        t.stride(1) != 1 or (ld is not None and t.stride(0) != ld):
+                    raise ValueError(f"decoder output {k!r} of group {g}: a float32 {self.device} tensor [{B}, >= {G}] with unit stride "
+                                     f"along the genes and the row pitch of the group's other outputs is needed, got "
+                                     f"{tuple(t.shape)} {t.dtype} strides {t.stride()}")
+                ld = t.stride(0)
+            arr = L.ptr_array([og.get(k) for k in ELEM_OUTPUTS])
+            src, xptr, ldx, rows = ctx["srcs"][g]
+            v = value[g] if value is not None else None
+            if v is not None:
+                if v.dtype != torch.float32 or not self._on_device(v) or v.dim() != 2 or v.shape[0] != B or v.shape[1] < G or v.stride(1) != 1:
+                    raise ValueError(f"value of group {g}: a float32 {self.device} tensor [{B}, >= {G}] with unit stride along the genes is "
+                                     f"needed, got {tuple(v.shape)} {v.dtype}")
+                src, xptr, ldx, rows = L.SRC_F32, v.data_ptr(), v.stride(0), None
+            dptrs = self._dec_ptrs(g, w, xptr, rows, False)
+            nb, Pb, Sb, KZb, KMIX = d.nb, d.Pb, d.Sb, d.KZb, d.KMIX
+            if self.fused_nb:
+                L.check(lib.spv_dec_nb_elems_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb),
+                                                L.ptr(w.wzf), B, G, HD, Pb, Sb, KMIX, arr, ld, st), "spv_dec_nb_elems_tc")
+                continue
+            if self.bf16:  # the unfused bf16 decoder's mixture logits: the tensor-core GEMM of its sweep
+                self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
+                self._tc_gemm(L.ptr(w.amixb), L.ptr(w.Wmb), L.ptr(w.pi), B, G, KMIX, lda=w.KMp, ldb=w.KMp, ldc=G, bias=L.ptr(self.P(g, "bm")))
+            L.check(lib.spv_dec_nb_elems(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1 if self.bf16 else 0, L.ptr(w.zzb) if nb else None,
+                                         KZb, KMIX, arr, ld, st), "spv_dec_nb_elems")
+        if run_prologue:
+            ctx["dec_gen"] = self.generation
 
     def _dec_ptrs(self, g, w, xptr, rows, with_grad):
         wg = with_grad
@@ -895,6 +994,7 @@ class StepEngine:
         ctx = self._ctx
         if ctx is None or not ctx["training"]:
             raise RuntimeError("backward needs a preceding training-mode forward")
+        self.generation += 1
         if stage not in ("all", "decoder", "encoder") or (adam is not None and stage == "decoder") or \
                 (adam is not None and stage == "encoder" and not adam.get("enc_only")):
             raise ValueError("stage must be 'all', 'decoder' or 'encoder' (the interleaved optimiser step needs 'all', or 'encoder' "

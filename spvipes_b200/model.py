@@ -275,6 +275,8 @@ class spVIPES:
                     if graph is None:
                         graph = loop.capture(batches)
                     graph.replay()
+                    eng.note_replay(forward=True)   # one training step: a forward and a backward pass
+                    eng.note_replay(forward=False)
                 else:
                     loop.step(batches)
                 tot += eng.loss_out[0]
@@ -311,16 +313,34 @@ class spVIPES:
         if normalized:
             raise RuntimeError("normalized=True: the reference collects no shared latents in this branch and fails in "
                                "torch.cat on an empty list (model/spvipes.py:542-544, 634); use normalized=False")
+        n = [len(g) for g in group_indices_list]
+        res = {"shared": [[], []], "private": [[], []], "idx": [[], []]}
+        for batches, ws in self._eval_passes(group_indices_list, batch_size, drop_last, _noise_fn):
+            for g in (0, 1):
+                res["shared"][g].append(ws[g].zpoe.cpu().clone())
+                res["private"][g].append(ws[g].zpriv.cpu().clone())
+                res["idx"][g].append(batches[g].idx.cpu().clone())
+        # reference _format_results (:628-650): truncate to the group sizes; group 2 re-ordered by its within-group index
+        shared = {g: torch.cat(res["shared"][g]).numpy()[:n[g]] for g in (0, 1)}
+        private = {g: torch.cat(res["private"][g]).numpy()[:n[g]] for g in (0, 1)}
+        idx2 = torch.cat(res["idx"][1]).numpy().flatten()[:n[1]]
+        order = np.argsort(idx2)
+        return {"shared": shared, "private": private,
+                "shared_reordered": {0: shared[0], 1: shared[1][order]},
+                "private_reordered": {0: private[0], 1: private[1][order]}}
+
+    def _eval_passes(self, group_indices_list, batch_size, drop_last, _noise_fn):
+        """the minibatches of the reference's latent extraction, each through an eval-mode encoder pass
+        (engine.forward(..., decode=False)): yields (batches, workspaces) per minibatch.  Sequential chunks of batch_size cells per
+        group; reference :478-515: drop_last defaults to False in every mode; the paired OT mode (no labels) then goes through the
+        cycling path, every other mode through one ConcatDataLoader over the two index lists"""
         self._to_device()
         eng = self.module.engine
         batch_size = batch_size or 128  # scvi.settings.batch_size
         n = [len(g) for g in group_indices_list]
         self.module.eval()
-        # reference :478-515: drop_last defaults to False in every mode; the paired OT mode (no labels) then goes through the
-        # cycling path, every other mode through one ConcatDataLoader over the two index lists
         drop_last = False if drop_last is None else bool(drop_last)
         use_cycling = eng.mode == "paired" and not drop_last
-        res = {"shared": [[], []], "private": [[], []], "idx": [[], []]}
         counter = [0]
 
         def process(index_lists):
@@ -342,11 +362,7 @@ class spVIPES:
                     batches.append(GroupBatch(X=d["X"], rows=rows[g], labels=lab, idx=d["idx"][r].contiguous(), B=len(st[g]), batch=bc))
                 noise = _noise_fn(counter[0], len(st[0]), len(st[1])) if _noise_fn is not None else None
                 counter[0] += 1
-                ws = eng.forward(batches, training=False, noise=noise, with_grad=False, decode=False)
-                for g in (0, 1):
-                    res["shared"][g].append(ws[g].zpoe.cpu().clone())
-                    res["private"][g].append(ws[g].zpriv.cpu().clone())
-                    res["idx"][g].append(batches[g].idx.cpu().clone())
+                yield batches, eng.forward(batches, training=False, noise=noise, with_grad=False, decode=False)
 
         if use_cycling:
             # reference _process_all_cells_with_cycling (:578-626): chunks of min(n) cells, the indices of BOTH groups taken
@@ -355,17 +371,59 @@ class spVIPES:
             if lo == 0:
                 raise ValueError("One of the groups is empty")
             for start in range(0, hi, lo):
-                process([[group_indices_list[g][(start + i) % n[g]] for i in range(lo)] for g in (0, 1)])
+                yield from process([[group_indices_list[g][(start + i) % n[g]] for i in range(lo)] for g in (0, 1)])
         else:
-            process(group_indices_list)
-        # reference _format_results (:628-650): truncate to the group sizes; group 2 re-ordered by its within-group index
-        shared = {g: torch.cat(res["shared"][g]).numpy()[:n[g]] for g in (0, 1)}
-        private = {g: torch.cat(res["private"][g]).numpy()[:n[g]] for g in (0, 1)}
-        idx2 = torch.cat(res["idx"][1]).numpy().flatten()[:n[1]]
-        order = np.argsort(idx2)
-        return {"shared": shared, "private": private,
-                "shared_reordered": {0: shared[0], 1: shared[1][order]},
-                "private_reordered": {0: private[0], 1: private[1][order]}}
+            yield from process(group_indices_list)
+
+    # decoded outputs of get_decoded_expression -> StepEngine.decode_elements names
+    DECODED_OUTPUTS = {"mean": "mean", "px_rate_private": "rate_p", "px_rate_shared": "rate_s", "px_mixing": "pi", "log_prob": "ll"}
+
+    @torch.no_grad()
+    def get_decoded_expression(self, group_indices_list: Sequence[Sequence[int]], outputs: Sequence[str] = ("mean",),
+                               gene_indices=None, batch_size: Optional[int] = None, drop_last: Optional[bool] = None,
+                               _noise_fn=None) -> dict:
+        """per-cell, per-gene decoder outputs of the eval-mode model (module/spVIPESmodule.py:751-759) on the latents that
+        get_latent_representation samples with the same arguments (same minibatches, cycling, truncation and noise):
+          mean             sigmoid(px_mixing) px_rate_private + (1 - sigmoid(px_mixing)) px_rate_shared (NegativeBinomialMixture.mean)
+          px_rate_private  exp(library) softmax over the genes of the private factor regressor's output
+          px_rate_shared   the same from the shared latents
+          px_mixing        the mixing logit: how much of a gene's expression the private branch explains (sigmoid of it)
+          log_prob         per-gene log-likelihood of the cell's own counts at log1p(x) (quirk Q3); minus its row sum is the
+                           reconstruction loss
+        gene_indices: None (all of each group's own genes) or one sequence per group of positions within that group's genes
+        (None entries: all); the gene selection is made on the GPU before the copy to the host.
+        Returns {output: {0: ndarray [n0, k0], 1: ndarray [n1, k1]}} float32, rows in the order of group_indices_list[g]; each
+        output takes n * k * 4 bytes of host memory per group (n cells, k genes), and the whole [batch, genes] block of a
+        minibatch passes through GPU memory before the gene selection.
+        _noise_fn (tests): as in get_latent_representation."""
+        outputs = (outputs,) if isinstance(outputs, str) else tuple(outputs)
+        bad = [o for o in outputs if o not in self.DECODED_OUTPUTS]
+        if bad or not outputs:
+            raise ValueError(f"unknown decoded output(s) {bad or outputs}; choose from {sorted(self.DECODED_OUTPUTS)}")
+        eng = self.module.engine
+        genes = eng.d.genes
+        sel = [None, None]
+        if gene_indices is not None:
+            if len(gene_indices) != 2:
+                raise ValueError("gene_indices: one sequence (or None) per group")
+            for g in (0, 1):
+                if gene_indices[g] is None:
+                    continue
+                gi = np.asarray(gene_indices[g], dtype=np.int64).reshape(-1)
+                if gi.size and (gi.min() < 0 or gi.max() >= genes[g]):
+                    raise ValueError(f"gene_indices[{g}]: positions must lie in [0, {genes[g]})")
+                sel[g] = torch.from_numpy(gi).to(eng.device)
+        n = [len(g) for g in group_indices_list]
+        res = {o: [[], []] for o in outputs}
+        for _, ws in self._eval_passes(group_indices_list, batch_size, drop_last, _noise_fn):
+            outs = [{self.DECODED_OUTPUTS[o]: torch.empty(ws[g].B, genes[g], dtype=torch.float32, device=eng.device) for o in outputs}
+                    for g in (0, 1)]
+            eng.decode_elements(outs)
+            for g in (0, 1):
+                for o in outputs:
+                    t = outs[g][self.DECODED_OUTPUTS[o]]
+                    res[o][g].append((t if sel[g] is None else t.index_select(1, sel[g])).cpu())
+        return {o: {g: torch.cat(res[o][g]).numpy()[:n[g]] for g in (0, 1)} for o in outputs}
 
     def get_loadings(self) -> dict:
         """reference model/spvipes.py:652-677"""

@@ -59,15 +59,87 @@ class LossOutput:
         return sum(v.sum() for v in self.kl_local.values())
 
 
+GC_THETA = 8  # row of theta = exp(px_r) in the decoder's per-gene constant table (csrc/decoder_common.cuh)
+
+
 class _NBMixtureHandle:
-    """stands where the reference puts scvi's NegativeBinomialMixture (`px`): the fused kernel has already evaluated
-    -log_prob(log1p(x)).sum(-1) for the minibatch it was built from."""
+    """stands where the reference puts scvi's NegativeBinomialMixture (`px`) of one group (module/spVIPESmodule.py:759).
+    neg_log_prob_sum = -log_prob(log1p(x)).sum(-1), evaluated by the likelihood sweep of the pass.  The per-gene members are
+    device tensors [B, G] without autograd, each computed on first access by one element launch (StepEngine.decode_elements) from
+    the decoder state of the pass that built this handle, and cached: mu1 = px_rate_private, mu2 = px_rate_shared,
+    mixture_logits = px_mixing, theta1 = exp(px_r) (an expanded view), mean = sigmoid(pi) mu1 + (1 - sigmoid(pi)) mu2 and
+    log_prob(value) (eps 1e-8).  Once the engine has run another forward or backward that state is gone: a member not read by
+    then raises RuntimeError; members already read are independent tensors and keep their values."""
 
-    def __init__(self, rec: torch.Tensor):
+    def __init__(self, rec: torch.Tensor, engine=None, group: int = 0, ws=None):
         self.neg_log_prob_sum = rec
+        self._eng, self._g, self._ws = engine, group, ws
+        self._gen = engine.generation if engine is not None else None
+        self._cache = {}
 
-    def log_prob(self, x):  # pragma: no cover - the reference's loss() call site; kept for API shape
-        raise NotImplementedError("the per-gene log-probabilities are never materialised; use neg_log_prob_sum")
+    def _check(self, what):
+        if self._eng is None:
+            raise RuntimeError(f"px.{what}: this handle carries the reconstruction term only")
+        if self._eng.generation != self._gen:
+            raise RuntimeError(f"px.{what} was not read before the engine's next forward or backward pass, which replaced the decoder "
+                               f"state it is computed from; read the px fields of a pass before running the next one")
+
+    def _elements(self, what, key, value=None):
+        self._check(what)
+        w, eng = self._ws, self._eng
+        out = torch.empty(w.B, w.G, dtype=torch.float32, device=eng.device)
+        outs, vals = [{}, {}], None
+        outs[self._g] = {key: out}
+        if value is not None:
+            vals = [None, None]
+            vals[self._g] = value
+        eng.decode_elements(outs, vals)
+        return out
+
+    def _field(self, name, key):
+        if name not in self._cache:
+            self._cache[name] = self._elements(name, key)
+        return self._cache[name]
+
+    @property
+    def mu1(self):
+        return self._field("mu1", "rate_p")
+
+    @property
+    def mu2(self):
+        return self._field("mu2", "rate_s")
+
+    @property
+    def mixture_logits(self):
+        return self._field("mixture_logits", "pi")
+
+    @property
+    def mean(self):
+        return self._field("mean", "mean")
+
+    @property
+    def theta1(self):
+        if "theta1" not in self._cache:
+            self._check("theta1")
+            w = self._ws
+            self._cache["theta1"] = w.genec[GC_THETA, :w.G].clone().unsqueeze(0).expand(w.B, w.G)
+        return self._cache["theta1"]
+
+    @property
+    def theta2(self):  # scvi: theta2 = None means theta1 for both components (the reference's shared dispersion)
+        return None
+
+    def log_prob(self, value):
+        """log_mixture_nb(value; mu1, mu2, theta1, mixture_logits), eps 1e-8, per element [B, G]; value: a [B, G] float tensor,
+        evaluated as given (the reference passes log1p(x): quirk Q3)"""
+        w = self._ws
+        if self._eng is None:
+            self._check("log_prob")
+        v = torch.as_tensor(value, device=self._eng.device)
+        if v.dim() != 2 or tuple(v.shape) != (w.B, w.G):
+            raise ValueError(f"px.log_prob: value must be [{w.B}, {w.G}], got {tuple(v.shape)}")
+        v = v.to(torch.float32).contiguous()
+        return self._elements("log_prob", "ll", v)
 
 
 class _LazyDict(OrderedDict):
@@ -167,11 +239,15 @@ class _CapturedStep:
             with torch.cuda.graph(g):
                 eng.forward(b["batches"], training=True, noise=None)
             b["fwd"] = g
+            b["ctx"] = eng._ctx  # the pass state (count pointers of this buffer set) that decode_elements reads after a replay
             g.replay()
+            eng.note_replay(forward=True)
         else:
             if eng.bf16 and eng.stage_in_adam and eng._staged_version != eng.params.flat._version:
                 eng.stage_weights()  # the parameters were written through torch since the 16-bit operand copies were made
+            eng._ctx = b["ctx"]
             b["fwd"].replay()
+            eng.note_replay(forward=True)
         return eng._ctx["ws"] if eng._ctx is not None else eng.workspace(self.B, self.B, True)
 
     def backward(self, b):
@@ -186,8 +262,10 @@ class _CapturedStep:
                 eng.backward(grad_scale=1.0)
             b["bwd"] = g
             g.replay()
+            eng.note_replay(forward=False)
         else:
             b["bwd"].replay()
+            eng.note_replay(forward=False)
         b["free"].record(torch.cuda.current_stream(eng.device))
 
 
@@ -422,7 +500,7 @@ class spVIPESmodule(nn.Module):
         return self._generative_dict(ws)
 
     def _generative_dict(self, ws):
-        return {"private_shared": {}, "private_poe": {str(g): {"px": _NBMixtureHandle(w.rec)} for g, w in enumerate(ws)}}
+        return {"private_shared": {}, "private_poe": {str(g): {"px": _NBMixtureHandle(w.rec, self.engine, g, w)} for g, w in enumerate(ws)}}
 
     def _loss_output(self, loss, ws):
         out = self.engine.loss_out

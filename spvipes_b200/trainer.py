@@ -222,6 +222,8 @@ class _SyncedGraphs:
         self.grad_sync.finish()
         main.wait_stream(self.side)
         self.g_opt_enc.replay()
+        self.engine.note_replay(forward=True)
+        self.engine.note_replay(forward=False)
         self.side.wait_stream(main)  # the next replay's decoder-range Adam must not start before this step is done
 
 
