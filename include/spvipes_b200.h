@@ -84,25 +84,12 @@ int spv_tc_gemm_ex(int fmt, float alpha, int a_mn, int b_mn, const void* A, long
 int spv_tc_gemm_split(int a_mn, int b_mn, const void* A, const void* A_lo, long long lda, const void* B, const void* B_lo,
                       long long ldb, float* C, long long ldc, int M, int N, int K, const float* bias, int relu, int accumulate,
                       int splits, float* ws, void* stream);
-/* Encoder first layer with the count transform fused into the GEMM's operand path (north_star "Encoder first layer";
- * module/spVIPESmodule.py:428-433 + nn/networks.py:119): producer warps gather uint16 counts by row index, look log1p up as a
- * split-bf16 pair and write the swizzled tcgen05 operand tiles; the weights (resp. dh1) arrive by TMA as bf16 pairs; three MMAs
- * per k-step into one TMEM accumulator.  No [B, G] staging buffer.
- *   spv_enc_fc1_fwd: h1[B, N] = act(log1p(X[rows, :G]) W^T (+ h1, pre_acc != 0: a pre-activation addend) + bias)
- *   spv_enc_fc1_dw : dW[M, :G] = dh1^T log1p(X[rows, :G])   (dh1 [B, ld_d] as a bf16 pair, dW row pitch ld_dw) */
-int spv_enc_fc1_fwd(const void* X, long long ldx, const int* rows, const void* W_hi, const void* W_lo, long long ldw, float* h1,
-                    long long ld_h1, int B, int N, int G, const float* bias, int relu, int pre_acc, int splits, float* ws,
-                    void* stream);
-int spv_enc_fc1_dw(const void* X, long long ldx, const int* rows, const void* d_hi, const void* d_lo, long long ld_d, float* dW,
-                   long long ld_dw, int B, int M, int G, void* stream);
 /* bf16 staging of GEMM operands: dst[r, :C] = bf16(src[r, :C]), zero padded up to ld_dst */
 int spv_to_bf16(const float* src, long long ld_src, void* dst, long long ld_dst, int R, int C, void* stream);
 /* fp16 staging (decoder operands of the fused tensor-core path) */
 int spv_to_f16(const float* src, long long ld_src, void* dst, long long ld_dst, int R, int C, void* stream);
 /* ... as a (hi, lo) pair for spv_tc_gemm_split */
 int spv_to_bf16_split(const float* src, long long ld_src, void* dst_hi, void* dst_lo, long long ld_dst, int R, int C, void* stream);
-/* column block: dst[r, :C] = bf16(src[r, :C]), zeros up to `width`; the other columns of dst (row pitch ld_dst) are untouched */
-int spv_to_bf16_block(const float* src, long long ld_src, void* dst, long long ld_dst, int R, int C, int width, void* stream);
 /* T[b, :G] = bf16(log1p(X[rows[b], :G])), zero padded to ld_dst (a multiple of 8)   module/spVIPESmodule.py:428-433;
  * dst_lo (optional): the bf16 residual plane for spv_tc_gemm_split;
  * lib (optional, [B]): library size log(sum_g log1p(x[b,g])) from the same pass   module/spVIPESmodule.py:433-435 */

@@ -33,8 +33,6 @@ _SIGS = {
     "spv_tc_gemm": [i, i, p, ll, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
     "spv_tc_gemm_ex": [i, f, i, i, p, ll, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
     "spv_tc_gemm_split": [i, i, p, p, ll, p, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
-    "spv_enc_fc1_fwd": [p, ll, p, p, p, ll, p, ll, i, i, i, p, i, i, i, p, p],
-    "spv_enc_fc1_dw": [p, ll, p, p, p, ll, p, ll, i, i, i, p],
     "spv_to_bf16": [p, ll, p, ll, i, i, p],
     "spv_to_f16": [p, ll, p, ll, i, i, p],
     "spv_to_bf16_split": [p, ll, p, p, ll, i, i, p],
@@ -74,7 +72,6 @@ _SIGS = {
     "spv_dec_nb_train_colsum": [p, i, i, f, p, p],
     "spv_dec_zq4": [p, ll, p, p, ll, i, i, i, p],
     "spv_dec_dz4_combine": [p, ll, p, p, ll, i, i, i, p],
-    "spv_to_bf16_block": [p, ll, p, ll, i, i, i, p],
     "spv_dec_dzz_combine": [p, ll, p, p, p, i, p, ll, p, p, i, i, i, p, p],
     "spv_adam_tick": [p, p],
     "spv_adam": [p, p, p, p, ll, f, f, f, f, f, f, p, p, i, p, p, p, p, p, p, p, i, p],

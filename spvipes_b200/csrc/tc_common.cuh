@@ -25,7 +25,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -88,24 +87,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
         "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// A operand in tensor memory (lane = row, 32-bit column = two consecutive k), B in shared memory
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// registers -> tensor memory: thread i of the warp writes 16 consecutive 32-bit columns of lane (base + i)
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-        "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]),
-        "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // arrive on an mbarrier when all previously issued MMAs of this thread have completed
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -143,13 +124,7 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes
     d |= (uint64_t)2 << 61;  // SWIZZLE_128B
     return d;
 }
-// instruction descriptor for kind::f16, BF16 x BF16 -> F32
-__host__ __device__ constexpr uint32_t idesc_bf16(int M, int N, bool a_mn_major, bool b_mn_major) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-// general form: per-operand format (0 = F16, 1 = BF16) and major-ness
+// instruction descriptor for kind::f16 with F32 accumulate: per-operand format (0 = F16, 1 = BF16) and major-ness
 __host__ __device__ constexpr uint32_t idesc_16(int M, int N, bool a_mn_major, bool b_mn_major, bool a_bf16, bool b_bf16) {
     return (1u << 4) | ((a_bf16 ? 1u : 0u) << 7) | ((b_bf16 ? 1u : 0u) << 10) | ((a_mn_major ? 1u : 0u) << 15) |
            ((b_mn_major ? 1u : 0u) << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);

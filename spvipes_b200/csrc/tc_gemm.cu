@@ -6,7 +6,6 @@
 // (dW = dY^T X, dX = dY W) run without materialising transposes.
 // This is the "bf16 tensor-core path" of BASELINE.json's north_star (parity gate 1e-2); the fp32 SIMT path of
 // gemm_simt.cu is the 1e-4 mode.  Replaces the cuBLAS GEMMs behind nn.Linear in reference nn/networks.py:119, 323-325.
-#include <cstdlib>
 #include <cuda_fp16.h>
 #include "tc_common.cuh"
 #include "../../include/spvipes_b200.h"
@@ -438,28 +437,6 @@ extern "C" int spv_to_bf16_split(const float* src, long long ld_src, void* dst_h
     return SPV_OK;
 }
 
-// column block: dst[r, c] = bf16(src[r, c]) for c < C, 0 for C <= c < width; columns beyond `width` of dst are left untouched
-__global__ void to_bf16_block_kernel(const float* __restrict__ src, long ld_src, __nv_bfloat16* __restrict__ dst, long ld_dst, int R,
-                                     int C, int width) {
-    long total = (long)R * width;
-    for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
-        int c = (int)(i % width);
-        long r = i / width;
-        dst[r * ld_dst + c] = __float2bfloat16(c < C ? src[r * ld_src + c] : 0.0f);
-    }
-}
-
-extern "C" int spv_to_bf16_block(const float* src, long long ld_src, void* dst, long long ld_dst, int R, int C, int width,
-                                 void* stream) {
-    if (!src || !dst || R <= 0 || C <= 0 || width < C || ld_dst < width) return SPV_ERR_ARG;
-    long total = (long)R * width;
-    int blocks = (int)min((long)148 * 16, (total + 255) / 256);
-    to_bf16_block_kernel<<<blocks, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(src, ld_src, reinterpret_cast<__nv_bfloat16*>(dst),
-                                                                                     ld_dst, R, C, width);
-    SPV_CHECK_LAUNCH();
-    return SPV_OK;
-}
-
 // T[b, g] = bf16(log1p(X[rows[b], g]))   (the encoder's input, reference module/spVIPESmodule.py:428-433), zero padded to ld_dst,
 // optionally its bf16 residual T_lo (split-operand GEMM), and optionally library[b] = log(sum_g log1p(x[b, g]))
 // (reference :433-435) from the same pass over the row.
@@ -737,595 +714,3 @@ extern "C" int spv_csr_gather(int src, const long long* indptr, const unsigned s
     SPV_CHECK_LAUNCH();
     return SPV_OK;
 }
-
-// =======================================================================================================================
-// Encoder first layer with the count transform fused into the GEMM's operand path (BASELINE.json north_star: "a tcgen05/TMEM GEMM
-// fed by TMA that consumes raw counts and fuses log1p into its prologue"; reference module/spVIPESmodule.py:428-433 +
-// nn/networks.py:119 and the weight gradient of that layer).
-//
-//   forward (DW = false):  C[b, n] = act( sum_g log1p(X[rows[b], g]) W1[n, g] + C_pre + bias )     A produced, B by TMA
-//   gradient (DW = true):  C[m, g] = sum_b dh1[b, m] log1p(X[rows[b], g])                          A by TMA, B produced
-//
-// The produced operand tile is the same in both: rows = cells, 128 bytes = 64 genes per row and swizzle atom.  Eight producer
-// warps gather the uint16 counts of the tile straight from the device-resident matrix (row indices = the minibatch), look
-// log1p up in a shared-memory table that holds the split-bf16 pair (hi | lo << 16) of every count < 256, and write the hi and
-// lo planes in the 128-byte-swizzled layout the UMMA descriptors expect; fence.proxy.async + an mbarrier hand the stage to the
-// MMA warp, which issues hi.hi + hi.lo + lo.hi into one TMEM accumulator.  The other operand (W1 resp. dh1, as bf16 pairs)
-// arrives by TMA.  Nothing [B, G]-sized is written: the bf16 copy of log1p(counts) that the separate staging pass produced
-// (2 x 2 bytes per element written, read again by both GEMMs) is gone.  After the k-loop the producer warps turn into the
-// epilogue (TMEM -> registers -> global).
-// =======================================================================================================================
-namespace fc1 {
-
-constexpr int BM = 128, BN = 128, BK = 64, STAGES = 3;
-constexpr int PROD_WARPS = 8, THREADS = 64 + 32 * PROD_WARPS;
-constexpr int TILE = 128 * 64 * 2;                 // one 16 KB plane of either operand
-constexpr int STAGE_BYTES = 4 * TILE;              // [A hi | A lo | B hi | B lo]
-constexpr int ROWS_CACHE = 4096;                   // minibatch row indices staged in shared memory (gradient kernel)
-constexpr int SMEM = STAGES * STAGE_BYTES + 1024 + 256 * 4 + 256 + ROWS_CACHE * 4;
-
-__device__ __forceinline__ int s_rows_or_global(const int* __restrict__ rows, const int* s_rows, int cell, int n_cached) {
-    return cell < n_cached ? s_rows[cell] : __ldg(rows + cell);
-}
-
-struct Params {
-    const unsigned short* X; long ldx; const int* rows;   // counts, row gather
-    float* C; long ldc;
-    const float* bias; float* ws;
-    int M, N, K;            // GEMM extents: forward M = cells, N = 2H, K = genes; gradient M = 2H, N = genes, K = cells
-    int relu, pre_acc, splits, kb_per_split;
-};
-
-__device__ __forceinline__ unsigned int pack_split_dev(float f) {
-    __nv_bfloat16 hi = __float2bfloat16(f);
-    __nv_bfloat16 lo = __float2bfloat16(f - __bfloat162float(hi));
-    return (unsigned int)__bfloat16_as_ushort(hi) | ((unsigned int)__bfloat16_as_ushort(lo) << 16);
-}
-
-// table miss (count >= 256): rare, kept out of line so that the producer loop stays small (inlined 32 x per k-block the libm
-// log1pf bloated the kernel to 700 KB of code and the loop ran out of the instruction cache: 3.5 us per k-block instead of 0.5)
-__device__ __noinline__ unsigned int lut_miss(unsigned int c) { return pack_split_dev(log1pf((float)c)); }
-__device__ __noinline__ unsigned int lut_any(const unsigned int* lutp, unsigned int c) { return c < 256u ? lutp[c] : lut_miss(c); }
-
-template <bool DW>
-__global__ void __launch_bounds__(THREADS, 1) fc1_kernel(const __grid_constant__ CUtensorMap mapT, const __grid_constant__ CUtensorMap mapTlo,
-                                                         Params p) {
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t raw = tc::smem_u32(smem_raw);
-    uint8_t* tiles = smem_raw + ((1024u - (raw & 1023u)) & 1023u);
-    unsigned int* lutp = reinterpret_cast<unsigned int*>(tiles + STAGES * STAGE_BYTES);
-    uint64_t* full_t = reinterpret_cast<uint64_t*>(lutp + 256);  // TMA operand landed
-    uint64_t* full_p = full_t + STAGES;                           // produced operand written (one arrival per producer warp)
-    uint64_t* empty = full_p + STAGES;
-    uint64_t* tmem_full = empty + STAGES;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-    int* s_rows = reinterpret_cast<int*>(tiles + STAGES * STAGE_BYTES + 256 * 4 + 256);
-    const int s_rows_n = (DW && p.rows) ? min(p.K, ROWS_CACHE) : 0;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n0 = blockIdx.x * BN, m0 = blockIdx.y * BM, split = blockIdx.z;
-    const int num_kb_total = (p.K + BK - 1) / BK;
-    const int kb_begin = split * p.kb_per_split;
-    const int num_kb = max(min(num_kb_total, kb_begin + p.kb_per_split) - kb_begin, 0);
-    for (int i = threadIdx.x; i < s_rows_n; i += THREADS) s_rows[i] = __ldg(p.rows + i);
-
-    if (warp == 0 && lane == 0) {
-        tc::tma_prefetch_desc(&mapT);
-        tc::tma_prefetch_desc(&mapTlo);
-        for (int s = 0; s < STAGES; ++s) {
-            tc::mbar_init(&full_t[s], 1);
-            tc::mbar_init(&full_p[s], PROD_WARPS);
-            tc::mbar_init(&empty[s], 1);
-        }
-        tc::mbar_init(tmem_full, 1);
-        tc::fence_barrier_init();
-    }
-    if (warp == 1) tc::tmem_alloc(tmem_slot, BN);
-    if (warp >= 2) {  // the count table: split-bf16 pair of log1p(c), c < 256
-        const int t = threadIdx.x - 64;
-        lutp[t] = pack_split_dev(t == 0 ? 0.0f : log1pf((float)t));
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tmem_base = *tmem_slot;
-    // stage layout: the TMA operand's two planes first when it is A (gradient), last when it is B (forward)
-    constexpr int OFF_PROD = DW ? 2 * TILE : 0, OFF_TMA = DW ? 0 : 2 * TILE;
-
-    if (warp == 0) {
-        if (tc::elect_one()) {
-            for (int i = 0; i < num_kb; ++i) {
-                const int s = i % STAGES;
-                tc::mbar_wait(&empty[s], ((i / STAGES) & 1) ^ 1);
-                uint8_t* dst = tiles + s * STAGE_BYTES + OFF_TMA;
-                tc::mbar_expect_tx(&full_t[s], 2 * TILE);
-                const int k0 = (kb_begin + i) * BK;
-                if (!DW) {  // W1 [n rows][k]: box {64 k, 128 rows}
-                    tc::tma_load_2d(&mapT, &full_t[s], dst, k0, n0);
-                    tc::tma_load_2d(&mapTlo, &full_t[s], dst + TILE, k0, n0);
-                } else {    // dh1 [k rows][m]: two boxes {64 m, 64 k} per plane
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        tc::tma_load_2d(&mapT, &full_t[s], dst + h * 8192, m0 + 64 * h, k0);
-                        tc::tma_load_2d(&mapTlo, &full_t[s], dst + TILE + h * 8192, m0 + 64 * h, k0);
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (tc::elect_one()) {
-            constexpr uint32_t idesc = tc::idesc_bf16(BM, BN, DW, DW);
-            for (int i = 0; i < num_kb; ++i) {
-                const int s = i % STAGES;
-                const uint32_t ph = (i / STAGES) & 1;
-                tc::mbar_wait(&full_t[s], ph);
-                tc::mbar_wait(&full_p[s], ph);
-                tc::fence_after_sync();
-                const uint32_t st = tc::smem_u32(tiles + s * STAGE_BYTES);
-                const uint32_t a_hi = st, a_lo = st + TILE, b_hi = st + 2 * TILE, b_lo = st + 3 * TILE;
-#pragma unroll
-                for (int kk = 0; kk < BK / 16; ++kk) {
-                    // K-major (forward): 16 k = 32 bytes along the swizzled row; MN-major (gradient): 16 k = 16 rows = 2048 bytes
-                    const uint32_t off = DW ? kk * 2048 : kk * 32;
-                    const uint32_t lbo = DW ? 8192 : 16;
-                    const uint64_t dah = tc::smem_desc(a_hi + off, lbo, 1024), dal = tc::smem_desc(a_lo + off, lbo, 1024);
-                    const uint64_t dbh = tc::smem_desc(b_hi + off, lbo, 1024), dbl = tc::smem_desc(b_lo + off, lbo, 1024);
-                    tc::umma_bf16(tmem_base, dah, dbh, idesc, (i > 0 || kk > 0) ? 1u : 0u);
-                    tc::umma_bf16(tmem_base, dah, dbl, idesc, 1u);
-                    tc::umma_bf16(tmem_base, dal, dbh, idesc, 1u);
-                }
-                tc::umma_commit(&empty[s]);
-            }
-            tc::umma_commit(tmem_full);
-        }
-    } else {
-        // ================= producers (then epilogue): 8 warps =================
-        const int t = threadIdx.x - 64;
-        // forward: 128 cell rows x 64 genes, thread = (row, 32-gene half); gradient: 64 cell rows x 128 genes, thread = (row, quarter)
-        const int r = DW ? (t >> 2) : (t >> 1);
-        const int part = DW ? (t & 3) : (t & 1);           // 32 genes = 4 chunks of 8
-        const int half = DW ? (part >> 1) : 0;             // 64-gene swizzle atom inside the 128-gene tile (gradient)
-        const int chunk0 = DW ? (part & 1) * 4 : part * 4;  // first 16-byte chunk inside the atom's 128-byte row
-        uint8_t* const prod_row = tiles + OFF_PROD + half * 8192 + r * 128;
-        const int ncell = DW ? p.K : p.M, ngene = DW ? p.N : p.K;
-        // forward: this thread's cell is fixed, its row pointer is resolved once
-        const unsigned short* fwd_row = nullptr;
-        if (!DW && m0 + r < ncell) fwd_row = p.X + (p.rows ? (long)__ldg(p.rows + m0 + r) : (long)(m0 + r)) * p.ldx;
-        // The gather is latency bound (one scattered 64-byte read per thread and k-block, ~1.5 us from HBM, after the row-index
-        // lookup in the gradient kernel): the raw counts of the next PF k-blocks are kept in flight in registers.
-        constexpr int PF = 4;
-        uint4 buf[PF][4];
-        auto issue = [&](int i, uint4 (&dst)[4]) {
-            const int kb = kb_begin + i;
-            const int cell = DW ? kb * BK + r : m0 + r;
-            const int gene0 = DW ? n0 + part * 32 : kb * BK + part * 32;
-            const unsigned short* src = nullptr;
-            if (DW) {
-                if (cell < ncell) src = p.X + (p.rows ? (long)s_rows_or_global(p.rows, s_rows, cell, s_rows_n) : (long)cell) * p.ldx + gene0;
-            } else if (fwd_row) {
-                src = fwd_row + gene0;
-            }
-            if (!src || gene0 >= ngene) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) dst[j] = make_uint4(0u, 0u, 0u, 0u);
-                return;
-            }
-            if (((reinterpret_cast<uintptr_t>(src) & 15) == 0) && gene0 + 32 <= ngene) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) dst[j] = __ldg(reinterpret_cast<const uint4*>(src) + j);
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    unsigned int w[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int g = gene0 + j * 8 + q * 2;
-                        const unsigned int c0 = g < ngene ? __ldg(src + j * 8 + q * 2) : 0u;
-                        const unsigned int c1 = g + 1 < ngene ? __ldg(src + j * 8 + q * 2 + 1) : 0u;
-                        w[q] = c0 | (c1 << 16);
-                    }
-                    dst[j] = make_uint4(w[0], w[1], w[2], w[3]);
-                }
-            }
-        };
-#pragma unroll
-        for (int u = 0; u < PF; ++u)
-            if (u < num_kb) issue(u, buf[u]);
-        for (int i0 = 0; i0 < num_kb; i0 += PF) {
-#pragma unroll
-            for (int u = 0; u < PF; ++u) {
-                const int i = i0 + u;
-                if (i < num_kb) {
-                    const int s = i % STAGES;
-                    tc::mbar_wait(&empty[s], ((i / STAGES) & 1) ^ 1);
-                    uint8_t* row_hi = prod_row + s * STAGE_BYTES;
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const unsigned int w[4] = {buf[u][j].x, buf[u][j].y, buf[u][j].z, buf[u][j].w};
-                        unsigned int e[8];
-                        // one table-miss test per 16-byte chunk (any count >= 256 in its 8 genes): the common path is eight
-                        // independent shared-memory lookups with no branch between them
-                        if ((((w[0] | w[1]) | (w[2] | w[3])) & 0xff00ff00u) == 0u) {
-#pragma unroll
-                            for (int q = 0; q < 4; ++q) {
-                                e[2 * q] = lutp[w[q] & 0xffu];
-                                e[2 * q + 1] = lutp[w[q] >> 16];
-                            }
-                        } else {
-#pragma unroll  // (unrolled: a dynamically indexed e[] would live in local memory, on the common path too)
-                            for (int q = 0; q < 4; ++q) {
-                                const unsigned int c0 = w[q] & 0xffffu, c1 = w[q] >> 16;
-                                e[2 * q] = lut_any(lutp, c0);
-                                e[2 * q + 1] = lut_any(lutp, c1);
-                            }
-                        }
-                        unsigned int hi[4], lo[4];
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            hi[q] = __byte_perm(e[2 * q], e[2 * q + 1], 0x5410);
-                            lo[q] = __byte_perm(e[2 * q], e[2 * q + 1], 0x7632);
-                        }
-                        const int sw = ((chunk0 + j) ^ (r & 7)) << 4;  // 128-byte swizzle: 16-byte chunk index XOR (row mod 8)
-                        *reinterpret_cast<uint4*>(row_hi + sw) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                        *reinterpret_cast<uint4*>(row_hi + TILE + sw) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                    }
-                    tc::fence_proxy_async();  // generic-proxy stores -> visible to the tensor core's async proxy
-                    __syncwarp();
-                    if (lane == 0) tc::mbar_arrive(&full_p[s]);
-                    if (i + PF < num_kb) issue(i + PF, buf[u]);
-                }
-            }
-        }
-        // ---- epilogue: warp (w & 3) owns TMEM lanes 32 (w & 3) .., the two warps of a quarter split the 128 columns
-        if (num_kb > 0) {
-            tc::mbar_wait(tmem_full, 0);
-            tc::fence_after_sync();
-        }
-        const int q = warp & 3, chalf = (warp - 2) >> 2;
-        const int m = m0 + q * 32 + lane;
-        float* out = p.splits > 1 ? p.ws + (size_t)split * p.M * p.N : p.C;
-        const long ld = p.splits > 1 ? p.N : p.ldc;
-        const bool fin = p.splits == 1;
-#pragma unroll 1
-        for (int c0 = chalf * 64; c0 < chalf * 64 + 64; c0 += 32) {
-            if (n0 + c0 >= p.N) break;
-            uint32_t v[32];
-            if (num_kb > 0) {
-                tc::tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);
-                tc::tmem_ld_wait();
-            } else {
-#pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = 0u;
-            }
-            if (m < p.M) {
-                float* dst = out + (size_t)m * ld + n0 + c0;
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int n = n0 + c0 + j;
-                    if (n < p.N) {
-                        float x = __uint_as_float(v[j]);
-                        if (fin) {
-                            if (p.pre_acc) x += dst[j];
-                            if (p.bias) x += __ldg(p.bias + n);
-                            if (p.relu) x = fmaxf(x, 0.0f);
-                        }
-                        dst[j] = x;
-                    }
-                }
-            }
-        }
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 1) {
-        tc::fence_after_sync();
-        tc::tmem_dealloc(tmem_base, BN);
-    }
-}
-
-template <bool DW>
-int launch_fc1(const CUtensorMap& mt, const CUtensorMap& mtl, const Params& p, cudaStream_t st) {
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!configured[dev & 63]) {
-        if (cudaFuncSetAttribute(fc1_kernel<DW>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess) return SPV_ERR_LAUNCH;
-        configured[dev & 63] = true;
-    }
-    dim3 grid((p.N + BN - 1) / BN, (p.M + BM - 1) / BM, p.splits);
-    fc1_kernel<DW><<<grid, THREADS, SMEM, st>>>(mt, mtl, p);
-    SPV_CHECK_LAUNCH();
-    return SPV_OK;
-}
-
-}  // namespace fc1
-
-int fc1t_launch(const CUtensorMap& mw, const CUtensorMap& mwl, const fc1::Params& p, cudaStream_t st);  // TMEM-A version, below
-
-// h1[B, N] = act(log1p(X[rows, :G]) W^T (+ h1 as a pre-activation addend) + bias): uint16 counts, W given as a bf16 pair
-// (W_hi, W_lo [N, ldw], spv_to_bf16_split / spv_adam staging).  splits > 1: split over the genes, partials in ws [splits, B, N],
-// reduced by a second launch (bias / ReLU / addend applied there).
-extern "C" int spv_enc_fc1_fwd(const void* X, long long ldx, const int* rows, const void* W_hi, const void* W_lo, long long ldw,
-                               float* h1, long long ld_h1, int B, int N, int G, const float* bias, int relu, int pre_acc, int splits,
-                               float* ws, void* stream) {
-    if (!X || !W_hi || !W_lo || !h1 || B <= 0 || N <= 0 || G <= 0) return SPV_ERR_ARG;
-    if (splits < 1) splits = 1;
-    const int num_kb = (G + 63) / 64;
-    if (splits > num_kb) splits = num_kb;
-    const int kb_per = (num_kb + splits - 1) / splits;
-    splits = (num_kb + kb_per - 1) / kb_per;
-    if (splits > 1 && !ws) return SPV_ERR_ARG;
-    CUtensorMap mt, mtl;
-    int rc = spv_make_tensor_map_bf16(&mt, W_hi, (unsigned long long)G, (unsigned long long)N, (unsigned long long)ldw, 64, fc1::BN);
-    if (rc != SPV_OK) return rc;
-    rc = spv_make_tensor_map_bf16(&mtl, W_lo, (unsigned long long)G, (unsigned long long)N, (unsigned long long)ldw, 64, fc1::BN);
-    if (rc != SPV_OK) return rc;
-    fc1::Params p;
-    p.X = reinterpret_cast<const unsigned short*>(X); p.ldx = ldx; p.rows = rows; p.C = h1; p.ldc = ld_h1; p.bias = bias; p.ws = ws;
-    p.M = B; p.N = N; p.K = G; p.relu = relu; p.pre_acc = pre_acc; p.splits = splits; p.kb_per_split = kb_per;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    static const bool smem_version = getenv("SPV_FC1_SMEM") != nullptr;  // A/B switch: producers write shared-memory tiles
-    rc = smem_version ? fc1::launch_fc1<false>(mt, mtl, p, st) : fc1t_launch(mt, mtl, p, st);
-    if (rc != SPV_OK) return rc;
-    if (splits > 1) {
-        TcParams r;
-        r.C = h1; r.bias = bias; r.ws = ws; r.ldc = ld_h1; r.M = B; r.N = N; r.K = G; r.relu = relu; r.accumulate = pre_acc ? 2 : 0;
-        r.splits = splits; r.kb_per_split = kb_per; r.idesc = 0; r.alpha = 1.0f;
-        const long total = (long)B * N;
-        tc_splitk_reduce_kernel<<<(int)min((long)148 * 8, (total + 255) / 256), 256, 0, st>>>(r);
-        SPV_CHECK_LAUNCH();
-    }
-    return SPV_OK;
-}
-
-// dW[M, :G] = dh1^T log1p(X[rows, :G]): dh1 given as a bf16 pair [B, ld_d] (the fused epilogue of the fc2 input-gradient GEMM
-// writes it), dW row pitch ld_dw
-extern "C" int spv_enc_fc1_dw(const void* X, long long ldx, const int* rows, const void* d_hi, const void* d_lo, long long ld_d,
-                              float* dW, long long ld_dw, int B, int M, int G, void* stream) {
-    if (!X || !d_hi || !d_lo || !dW || B <= 0 || M <= 0 || G <= 0) return SPV_ERR_ARG;
-    CUtensorMap mt, mtl;
-    int rc = spv_make_tensor_map_bf16(&mt, d_hi, (unsigned long long)M, (unsigned long long)B, (unsigned long long)ld_d, 64, 64);
-    if (rc != SPV_OK) return rc;
-    rc = spv_make_tensor_map_bf16(&mtl, d_lo, (unsigned long long)M, (unsigned long long)B, (unsigned long long)ld_d, 64, 64);
-    if (rc != SPV_OK) return rc;
-    fc1::Params p;
-    p.X = reinterpret_cast<const unsigned short*>(X); p.ldx = ldx; p.rows = rows; p.C = dW; p.ldc = ld_dw; p.bias = nullptr; p.ws = nullptr;
-    p.M = M; p.N = G; p.K = B; p.relu = 0; p.pre_acc = 0; p.splits = 1; p.kb_per_split = (B + 63) / 64;
-    return fc1::launch_fc1<true>(mt, mtl, p, reinterpret_cast<cudaStream_t>(stream));
-}
-
-// =======================================================================================================================
-// Forward of the encoder's first layer with the transformed counts written straight into TENSOR MEMORY as the MMA's A operand.
-// The shared-memory version above is bound by shared-memory bandwidth: per 64-gene k-block the tensor core reads 3 x (A + B) =
-// 96 KB of operands while producers and TMA write 64 KB more (measured: 2200 cycles per k-block in the producers' store phase,
-// tools/bench_fc1.py).  Here thread = cell row = TMEM lane: the producer warps gather the row's counts, look the split-bf16 pair
-// up and tcgen05.st the hi and lo halves of the A tile (2 x 32 columns per stage); only the weights go through shared memory
-// (TMA, six stages), and the MMAs are issued in the TS form (A from TMEM).  Same arithmetic as fc1_kernel<false>.
-// =======================================================================================================================
-namespace fc1t {
-
-constexpr int BM = 128, BN = 128, BK = 64;
-constexpr int B_STAGES = 6, A_STAGES = 4;
-constexpr int PROD_WARPS = 8, THREADS = 64 + 32 * PROD_WARPS;
-constexpr int TILE = 128 * 64 * 2;                    // one 16 KB plane of the weight tile
-constexpr int B_STAGE_BYTES = 2 * TILE;               // [W hi | W lo]
-constexpr int A_COLS = 64;                            // TMEM columns per A stage: hi (32) | lo (32)
-constexpr int TMEM_COLS = 512;                        // accumulator 128 + 4 x 64 = 384 -> power of two
-constexpr int SMEM = B_STAGES * B_STAGE_BYTES + 1024 + 256 * 4 + 512;
-
-__global__ void __launch_bounds__(THREADS, 1) fc1_tmem_kernel(const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapWlo,
-                                                              fc1::Params p) {
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t raw = tc::smem_u32(smem_raw);
-    uint8_t* tiles = smem_raw + ((1024u - (raw & 1023u)) & 1023u);
-    unsigned int* lutp = reinterpret_cast<unsigned int*>(tiles + B_STAGES * B_STAGE_BYTES);
-    uint64_t* full_b = reinterpret_cast<uint64_t*>(lutp + 256);
-    uint64_t* empty_b = full_b + B_STAGES;
-    uint64_t* full_a = empty_b + B_STAGES;
-    uint64_t* empty_a = full_a + A_STAGES;
-    uint64_t* tmem_full = empty_a + A_STAGES;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n0 = blockIdx.x * BN, m0 = blockIdx.y * BM, split = blockIdx.z;
-    const int num_kb_total = (p.K + BK - 1) / BK;
-    const int kb_begin = split * p.kb_per_split;
-    const int num_kb = max(min(num_kb_total, kb_begin + p.kb_per_split) - kb_begin, 0);
-
-    if (warp == 0 && lane == 0) {
-        tc::tma_prefetch_desc(&mapW);
-        tc::tma_prefetch_desc(&mapWlo);
-        for (int s = 0; s < B_STAGES; ++s) { tc::mbar_init(&full_b[s], 1); tc::mbar_init(&empty_b[s], 1); }
-        for (int s = 0; s < A_STAGES; ++s) { tc::mbar_init(&full_a[s], PROD_WARPS); tc::mbar_init(&empty_a[s], 1); }
-        tc::mbar_init(tmem_full, 1);
-        tc::fence_barrier_init();
-    }
-    if (warp == 1) tc::tmem_alloc(tmem_slot, TMEM_COLS);
-    if (warp >= 2) {
-        const int t = threadIdx.x - 64;
-        lutp[t] = fc1::pack_split_dev(t == 0 ? 0.0f : log1pf((float)t));
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tmem_base = *tmem_slot;          // accumulator: columns [0, 128)
-    const uint32_t tmem_a0 = tmem_base + BN;        // A stages: columns [128, 128 + 4 x 64)
-
-    if (warp == 0) {
-        if (tc::elect_one()) {
-            for (int i = 0; i < num_kb; ++i) {
-                const int s = i % B_STAGES;
-                tc::mbar_wait(&empty_b[s], ((i / B_STAGES) & 1) ^ 1);
-                uint8_t* dst = tiles + s * B_STAGE_BYTES;
-                tc::mbar_expect_tx(&full_b[s], B_STAGE_BYTES);
-                const int k0 = (kb_begin + i) * BK;
-                tc::tma_load_2d(&mapW, &full_b[s], dst, k0, n0);
-                tc::tma_load_2d(&mapWlo, &full_b[s], dst + TILE, k0, n0);
-            }
-        }
-    } else if (warp == 1) {
-        if (tc::elect_one()) {
-            constexpr uint32_t idesc = tc::idesc_bf16(BM, BN, false, false);
-            for (int i = 0; i < num_kb; ++i) {
-                const int sb = i % B_STAGES, sa = i % A_STAGES;
-                tc::mbar_wait(&full_b[sb], (i / B_STAGES) & 1);
-                tc::mbar_wait(&full_a[sa], (i / A_STAGES) & 1);
-                tc::fence_after_sync();
-                const uint32_t b_hi = tc::smem_u32(tiles + sb * B_STAGE_BYTES), b_lo = b_hi + TILE;
-                const uint32_t a_hi = tmem_a0 + sa * A_COLS, a_lo = a_hi + 32;
-#pragma unroll
-                for (int kk = 0; kk < BK / 16; ++kk) {
-                    const uint64_t dbh = tc::smem_desc(b_hi + kk * 32, 16, 1024), dbl = tc::smem_desc(b_lo + kk * 32, 16, 1024);
-                    tc::umma_bf16_ts(tmem_base, a_hi + kk * 8, dbh, idesc, (i > 0 || kk > 0) ? 1u : 0u);
-                    tc::umma_bf16_ts(tmem_base, a_hi + kk * 8, dbl, idesc, 1u);
-                    tc::umma_bf16_ts(tmem_base, a_lo + kk * 8, dbh, idesc, 1u);
-                }
-                tc::umma_commit(&empty_b[sb]);
-                tc::umma_commit(&empty_a[sa]);
-            }
-            tc::umma_commit(tmem_full);
-        }
-    } else {
-        // ================= producers: warp w owns TMEM lanes 32 (w & 3) .., the two warps of a quarter split the 64 genes
-        const int q = warp & 3, khalf = (warp - 2) >> 2;
-        const int r = q * 32 + lane;                 // row of the tile = TMEM lane
-        const unsigned short* row = nullptr;
-        if (m0 + r < p.M) row = p.X + (p.rows ? (long)__ldg(p.rows + m0 + r) : (long)(m0 + r)) * p.ldx;
-        constexpr int PF = 4;
-        uint4 buf[PF][4];
-        auto issue = [&](int i, uint4 (&dst)[4]) {
-            const int gene0 = (kb_begin + i) * BK + khalf * 32;
-            if (!row || gene0 >= p.K) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) dst[j] = make_uint4(0u, 0u, 0u, 0u);
-                return;
-            }
-            const unsigned short* src = row + gene0;
-            if (((reinterpret_cast<uintptr_t>(src) & 15) == 0) && gene0 + 32 <= p.K) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) dst[j] = __ldg(reinterpret_cast<const uint4*>(src) + j);
-            } else {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    unsigned int w[4];
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const int g = gene0 + j * 8 + e * 2;
-                        const unsigned int c0 = g < p.K ? __ldg(src + j * 8 + e * 2) : 0u;
-                        const unsigned int c1 = g + 1 < p.K ? __ldg(src + j * 8 + e * 2 + 1) : 0u;
-                        w[e] = c0 | (c1 << 16);
-                    }
-                    dst[j] = make_uint4(w[0], w[1], w[2], w[3]);
-                }
-            }
-        };
-#pragma unroll
-        for (int u = 0; u < PF; ++u)
-            if (u < num_kb) issue(u, buf[u]);
-        const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-        for (int i0 = 0; i0 < num_kb; i0 += PF) {
-#pragma unroll
-            for (int u = 0; u < PF; ++u) {
-                const int i = i0 + u;
-                if (i < num_kb) {
-                    const int sa = i % A_STAGES;
-                    uint32_t hi[16], lo[16];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const unsigned int w[4] = {buf[u][j].x, buf[u][j].y, buf[u][j].z, buf[u][j].w};
-                        unsigned int e[8];
-                        if ((((w[0] | w[1]) | (w[2] | w[3])) & 0xff00ff00u) == 0u) {
-#pragma unroll
-                            for (int c = 0; c < 4; ++c) {
-                                e[2 * c] = lutp[w[c] & 0xffu];
-                                e[2 * c + 1] = lutp[w[c] >> 16];
-                            }
-                        } else {
-#pragma unroll
-                            for (int c = 0; c < 4; ++c) {
-                                e[2 * c] = fc1::lut_any(lutp, w[c] & 0xffffu);
-                                e[2 * c + 1] = fc1::lut_any(lutp, w[c] >> 16);
-                            }
-                        }
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) {  // column = two consecutive genes: low half = even gene
-                            hi[4 * j + c] = __byte_perm(e[2 * c], e[2 * c + 1], 0x5410);
-                            lo[4 * j + c] = __byte_perm(e[2 * c], e[2 * c + 1], 0x7632);
-                        }
-                    }
-                    tc::mbar_wait(&empty_a[sa], ((i / A_STAGES) & 1) ^ 1);  // the conversion above overlaps the wait for the stage
-                    tc::fence_after_sync();
-                    const uint32_t a_hi = tmem_a0 + sa * A_COLS + lane_base + khalf * 16;
-                    tc::tmem_st16(a_hi, hi);
-                    tc::tmem_st16(a_hi + 32, lo);
-                    tc::tmem_st_wait();
-                    tc::fence_before_sync();
-                    __syncwarp();
-                    if (lane == 0) tc::mbar_arrive(&full_a[sa]);
-                    if (i + PF < num_kb) issue(i + PF, buf[u]);
-                }
-            }
-        }
-        // ---- epilogue
-        if (num_kb > 0) {
-            tc::mbar_wait(tmem_full, 0);
-            tc::fence_after_sync();
-        }
-        const int m = m0 + r;
-        float* out = p.splits > 1 ? p.ws + (size_t)split * p.M * p.N : p.C;
-        const long ld = p.splits > 1 ? p.N : p.ldc;
-        const bool fin = p.splits == 1;
-#pragma unroll 1
-        for (int c0 = khalf * 64; c0 < khalf * 64 + 64; c0 += 32) {
-            if (n0 + c0 >= p.N) break;
-            uint32_t v[32];
-            if (num_kb > 0) {
-                tc::tmem_ld32(tmem_base + lane_base + (uint32_t)c0, v);
-                tc::tmem_ld_wait();
-            } else {
-#pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = 0u;
-            }
-            if (m < p.M) {
-                float* dst = out + (size_t)m * ld + n0 + c0;
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int n = n0 + c0 + j;
-                    if (n < p.N) {
-                        float x = __uint_as_float(v[j]);
-                        if (fin) {
-                            if (p.pre_acc) x += dst[j];
-                            if (p.bias) x += __ldg(p.bias + n);
-                            if (p.relu) x = fmaxf(x, 0.0f);
-                        }
-                        dst[j] = x;
-                    }
-                }
-            }
-        }
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 1) {
-        tc::fence_after_sync();
-        tc::tmem_dealloc(tmem_base, TMEM_COLS);
-    }
-}
-
-int launch(const CUtensorMap& mw, const CUtensorMap& mwl, const fc1::Params& p, cudaStream_t st) {
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!configured[dev & 63]) {
-        if (cudaFuncSetAttribute(fc1_tmem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess) return SPV_ERR_LAUNCH;
-        configured[dev & 63] = true;
-    }
-    dim3 grid((p.N + BN - 1) / BN, (p.M + BM - 1) / BM, p.splits);
-    fc1_tmem_kernel<<<grid, THREADS, SMEM, st>>>(mw, mwl, p);
-    SPV_CHECK_LAUNCH();
-    return SPV_OK;
-}
-
-}  // namespace fc1t
-
-int fc1t_launch(const CUtensorMap& mw, const CUtensorMap& mwl, const fc1::Params& p, cudaStream_t st) { return fc1t::launch(mw, mwl, p, st); }

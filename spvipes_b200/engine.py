@@ -10,7 +10,6 @@ torch is used for device memory and streams only; every arithmetic step is a lau
 from __future__ import annotations
 
 import contextlib
-import os
 import math
 from collections import OrderedDict
 from dataclasses import dataclass, field
@@ -273,7 +272,7 @@ class _GroupWS:
         nb, KZb = d.nb, d.KZb
         self.amix = torch.zeros(B, KMIX, dtype=torch.float32, device=dev)
         self.zzb = f(B, KZb) if nb else None      # [z_private_arg | oh | z_shared_arg | oh] (batch covariates)
-        self.oh = f(B, nb) if nb else None        # one-hot batch codes (fp32 path of the encoders' first layer)
+        self.oh = f(B, nb) if nb and not bf16 else None  # one-hot batch codes (fp32 path of the encoders' first layer)
         self.zsum, self.zmean, self.zcov = f(KZb), f(KZb), f(KZb, KZb)
         # scratch of the latent statistics (spv_dec_fold, minibatches > 512 rows): per 64-row tile, column sums + centred second moments
         self.cov_part = torch.zeros(self.nTB, KZb + KZb * KZb, dtype=torch.float32, device=dev)
@@ -302,7 +301,7 @@ class _GroupWS:
             h = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)
             hd = lambda *s: torch.zeros(*s, dtype=torch.float16 if fused else torch.bfloat16, device=dev)  # decoder operands
             self.amixb = hd(B, self.KMp)
-            self.Tb = self.Tb_lo = None  # log1p(counts) as a bf16 pair: only the unfused first layer needs it (need_tb)
+            self.Tb, self.Tb_lo = h(B, self.Gpe), h(B, self.Gpe)  # log1p(counts) as a bf16 pair: the first layer's input
             # fp16 operands of the branch-logit MMAs (spv_dec_fold writes them): centred latents and folded weights
             self.zcb = torch.zeros(B, 64, dtype=torch.float16, device=dev)
             self.wzf = torch.zeros(2 * self.Gp, 64, dtype=torch.float16, device=dev)
@@ -347,11 +346,6 @@ class _GroupWS:
             self.dstats, self.dr = f(B, NST), f(B, NST)
             self.g_own, self.g_contrib, self.dexpert = f(B, 2 * S), f(B, 2 * S), f(B, 2 * S)
             self.dh2, self.dh1 = f(B, 2 * H), f(B, 2 * H)
-
-    def need_tb(self, dev):
-        if self.Tb is None:
-            self.Tb = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
-            self.Tb_lo = torch.zeros(self.B, self.Gpe, dtype=torch.bfloat16, device=dev)
 
     def need_xs(self, dtype, dev):
         """dense staging tile [B, Gp] of a CSR minibatch (spv_csr_gather): what every count consumer reads with rows = NULL"""
@@ -437,14 +431,6 @@ class StepEngine:
         self.stage_in_adam = False
         self._staged_version = -1
         self.adam_ticket = torch.zeros(1, dtype=torch.int32, device=self.device)
-        # Encoder first layer with the count transform fused into the GEMM's operand path (spv_enc_fc1_fwd / _dw: producer warps
-        # gather the uint16 counts, look log1p up as a split-bf16 pair and write the A operand into tensor memory resp. the B
-        # operand into swizzled shared memory).  Correct and tested (tests/test_gpu_kernels.py), but OPT-IN (SPV_FUSED_FC1=1):
-        # measured at the C5 shape (tools/bench_fc1.py, profiles/r2_fc1_fusion.md) the fused forward takes 125 us and the fused
-        # weight gradient 183 us per group against 60 (staging pass, HBM bound) + 71 resp. 88 us for the TMA-fed split GEMMs:
-        # one scattered 16-byte access per lane makes every warp load 32 L1 wavefronts, and table look-ups, operand stores and
-        # the tensor core's operand reads share the shared-memory pipe.
-        self.fused_fc1 = os.environ.get("SPV_FUSED_FC1", "0") == "1"
         self.nb_events = None  # bench hook: iterator of (start, end) CUDA events bracketing the NB-loglik sweep
         # advanced by every forward and every backward pass, eager or replayed from a CUDA graph (note_replay): a pass's decoder
         # state in the workspaces (what decode_elements reads) is current while the generation is the one it was made in
@@ -629,7 +615,6 @@ class StepEngine:
             nb, Gc = d.nb, G + d.nb
             if nb and bt.batch is None:
                 raise ValueError("batch codes are required when the model was built with n_batch > 1")
-            fused1 = self.bf16 and self.fused_fc1 and src == L.SRC_U16_LOG1P
             # (src, xptr, ldx, count_rows): where every consumer of the counts reads this minibatch
             if isinstance(bt.X, CsrCounts):
                 if bt.col0 != 0 or bt.X.shape[1] != G:
@@ -638,9 +623,7 @@ class StepEngine:
                 # gather the minibatch into the dense staging tile; in the default bf16 mode the same launch writes the encoder's
                 # split-bf16 input and the library size (what spv_counts_to_bf16 does on dense rows)
                 xs = w.need_xs(bt.X.dtype, self.device)
-                conv = self.bf16 and not fused1
-                if conv:
-                    w.need_tb(self.device)
+                conv = self.bf16
                 L.check(lib.spv_csr_gather(src, L.ptr(bt.X.indptr), L.ptr(bt.X.indices), L.ptr(bt.X.values), L.ptr(bt.rows), B, G,
                                            L.ptr(xs), w.Gp, L.ptr(w.Tb) if conv else None, L.ptr(w.Tb_lo) if conv else None, w.Gpe,
                                            L.ptr(w.lib) if conv else None, L.ptr(bt.batch) if (conv and nb) else None,
@@ -659,24 +642,9 @@ class StepEngine:
                 if decode or self.stage_in_adam:
                     with self._branch(g, "wm"):
                         self._to_dec(L.ptr(self.P(g, "Wm")), KMIX, L.ptr(w.Wmb), w.KMp, G, KMIX)
-            if fused1:
-                # first layer straight from the raw counts: the producer warps of the GEMM gather the rows, look log1p up as a
-                # split-bf16 pair and write the tensor-core operand tiles (spv_enc_fc1_fwd); the library size on the side
-                with self._branch(g, "lib"):
-                    L.check(lib.spv_library_size(src, xptr, ldx, L.ptr(count_rows), B, G, L.ptr(w.lib), self._stream()),
-                            "spv_library_size")
-                if nb:  # covariate term + bias as a pre-activation addend
-                    L.check(lib.spv_one_hot(L.ptr(bt.batch), L.ptr(w.oh), nb, B, nb, st), "spv_one_hot")
-                    self._gemm(L.ptr(w.oh), self.P(g, "W1").data_ptr() + 4 * G, L.ptr(w.h1), B, 2 * H, nb, lda=nb, ldb=Gc, ldc=2 * H,
-                               tb=1, bias=L.ptr(self.P(g, "b1")))
-                self._join(g, "w1")
-                L.check(lib.spv_enc_fc1_fwd(xptr, ldx, L.ptr(count_rows), L.ptr(w.W1b), L.ptr(w.W1b_lo), w.Gpe, L.ptr(w.h1), 2 * H, B,
-                                            2 * H, G, None if nb else L.ptr(self.P(g, "b1")), 1, 1 if nb else 0, w.tc_splits_fc1,
-                                            L.ptr(w.ws), st), "spv_enc_fc1_fwd")
-            elif self.bf16:  # encoder input and library size from one pass over the gathered rows
+            if self.bf16:  # encoder input and library size from one pass over the gathered rows
                 # (with batch covariates: their one-hot columns behind the genes, so that fc1 stays one GEMM over K = G + nb)
                 if not conv:  # (a CSR minibatch was converted by its gather)
-                    w.need_tb(self.device)
                     L.check(lib.spv_counts_to_bf16(src, xptr, ldx, L.ptr(count_rows), L.ptr(w.Tb), L.ptr(w.Tb_lo), w.Gpe, B, G,
                                                    L.ptr(w.lib), L.ptr(bt.batch) if nb else None, nb, st), "spv_counts_to_bf16")
                 self._join(g, "w1")
@@ -1194,15 +1162,8 @@ class StepEngine:
                 if not fuse1:
                     L.check(lib.spv_to_bf16_split(L.ptr(w.dh1), 2 * H, L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H, B, 2 * H, st),
                             "spv_to_bf16_split")
-                if self.fused_fc1 and src == L.SRC_U16_LOG1P:  # counts transformed in the GEMM's producer warps (as the forward)
-                    L.check(lib.spv_enc_fc1_dw(xptr, ldx, L.ptr(count_rows), L.ptr(w.dh1b), L.ptr(w.dh1b_lo), 2 * H,
-                                               L.ptr(self.Gd(g, "W1")), G + d.nb, B, 2 * H, G, st), "spv_enc_fc1_dw")
-                    if d.nb:  # covariate columns of the first layer's weight: dh1^T one_hot
-                        self._gemm(L.ptr(w.dh1), L.ptr(w.oh), self.Gd(g, "W1").data_ptr() + 4 * G, 2 * H, d.nb, B, lda=2 * H,
-                                   ldb=d.nb, ldc=G + d.nb, ta=1)
-                else:
-                    self._tc_gemm_split(L.ptr(w.dh1b), L.ptr(w.dh1b_lo), L.ptr(w.Tb), L.ptr(w.Tb_lo), L.ptr(self.Gd(g, "W1")), 2 * H,
-                                        G + d.nb, B, lda=2 * H, ldb=w.Gpe, ldc=G + d.nb, a_mn=1, b_mn=1)
+                self._tc_gemm_split(L.ptr(w.dh1b), L.ptr(w.dh1b_lo), L.ptr(w.Tb), L.ptr(w.Tb_lo), L.ptr(self.Gd(g, "W1")), 2 * H,
+                                    G + d.nb, B, lda=2 * H, ldb=w.Gpe, ldc=G + d.nb, a_mn=1, b_mn=1)
             else:
                 self._gemm(L.ptr(w.dh1), xptr, L.ptr(self.Gd(g, "W1")), 2 * H, G, B, lda=2 * H, ldb=ldx, ldc=G + d.nb, ta=1, srcB=src,
                            rowsB=count_rows)

@@ -87,7 +87,6 @@ class TrainLoop:
         self.epoch = 0
         self.grad_sync = None  # optional callable(engine) run between backward and the optimiser step (data parallel)
         self._dp_stream = None
-        self.early_adam = os.environ.get("SPV_EARLY_ADAM", "1") == "1"  # A/B switch for the per-range optimiser step
         # this loop owns the optimiser step: Adam also refreshes the bf16 tensor-core copies of the large weights
         # (largest staged block must stay below 2^24 elements, the range of the kernel's index arithmetic)
         if engine.bf16 and max(engine.d.genes) * max(engine.d.KMIX, 2 * engine.d.n_hidden) < (1 << 24):
@@ -101,11 +100,8 @@ class TrainLoop:
     def step(self, batches: Sequence[GroupBatch], noise: Optional[Noise] = None):
         e = self.engine
         e.forward(batches, training=True, noise=noise)
-        if self.grad_sync is None and self.early_adam:  # single GPU: the optimiser step is interleaved with the backward
+        if self.grad_sync is None:  # single GPU: the optimiser step is interleaved with the backward
             e.backward(adam={"lr": self.lr, "eps": self.eps, "weight_decay": self.weight_decay})
-        elif self.grad_sync is None:
-            e.backward()
-            e.adam_step(lr=self.lr, eps=self.eps, weight_decay=self.weight_decay, grad_scale=1.0)
         elif getattr(self.grad_sync, "in_graph", False):
             self._step_nvlink(e)
         else:  # data parallel: the decoder range is all-reduced while the encoder backward runs

@@ -135,29 +135,26 @@ def _noise(seed=8):
                  [((torch.rand(BE, 2 * H, generator=gen) < 0.9).float() / 0.9).cuda() for _ in (0, 1)])
 
 
-ENGINE_CASES = [  # (id, mode, precision, env, n_batch, counts, training)
-    ("label-bf16", "label", "bf16", {}, 0, "u16", True),
-    ("label-fp32", "label", "fp32", {}, 0, "u16", True),
-    ("paired-bf16", "paired", "bf16", {}, 0, "u16", True),
-    ("cluster-bf16", "cluster", "bf16", {}, 0, "u16", True),
-    ("paired-fp32", "paired", "fp32", {}, 0, "u16", True),
-    ("label-bf16-covariates", "label", "bf16", {}, 3, "u16", True),
-    ("label-fp32-covariates", "label", "fp32", {}, 3, "u16", True),
-    ("label-bf16-fused-fc1", "label", "bf16", {"SPV_FUSED_FC1": "1"}, 0, "u16", True),
-    ("label-bf16-float-counts", "label", "bf16", {}, 0, "f32", True),
-    ("label-fp32-float-counts", "label", "fp32", {}, 0, "f32", True),
-    ("label-bf16-eval", "label", "bf16", {}, 0, "u16", False),
-    ("label-fp32-eval", "label", "fp32", {}, 0, "u16", False),
+ENGINE_CASES = [  # (id, mode, precision, n_batch, counts, training)
+    ("label-bf16", "label", "bf16", 0, "u16", True),
+    ("label-fp32", "label", "fp32", 0, "u16", True),
+    ("paired-bf16", "paired", "bf16", 0, "u16", True),
+    ("cluster-bf16", "cluster", "bf16", 0, "u16", True),
+    ("paired-fp32", "paired", "fp32", 0, "u16", True),
+    ("label-bf16-covariates", "label", "bf16", 3, "u16", True),
+    ("label-fp32-covariates", "label", "fp32", 3, "u16", True),
+    ("label-bf16-float-counts", "label", "bf16", 0, "f32", True),
+    ("label-fp32-float-counts", "label", "fp32", 0, "f32", True),
+    ("label-bf16-eval", "label", "bf16", 0, "u16", False),
+    ("label-fp32-eval", "label", "fp32", 0, "u16", False),
 ]
 
 
 @pytest.mark.parametrize("case", ENGINE_CASES, ids=[c[0] for c in ENGINE_CASES])
-def test_engine_step_csr_equals_dense(case, monkeypatch):
+def test_engine_step_csr_equals_dense(case):
     from spvipes_b200 import synth
     from spvipes_b200.trainer import TrainLoop
-    _, mode, precision, env, n_batch, counts, training = case
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+    _, mode, precision, n_batch, counts, training = case
     data, dense, csr = _engine_data(counts)
     gen = torch.Generator(device="cuda").manual_seed(77)
     rows = [torch.randint(0, n, (BE,), generator=gen, device="cuda", dtype=torch.int32) for n in (N0, N1)]

@@ -153,19 +153,6 @@ def test_smallk_gemm(tb, M, N, K, batch):
         assert torch.equal(C[:, batch * N:], C0[:, batch * N:])  # padding column untouched
 
 
-def test_to_bf16_block():
-    from spvipes_b200 import _lib as L
-    lib = L.load()
-    g = torch.Generator(device="cuda").manual_seed(4)
-    src = torch.randn(100, 291, generator=g, device="cuda")
-    dst = torch.full((100, 296), 7.0, device="cuda", dtype=torch.bfloat16)
-    L.check(lib.spv_to_bf16_block(src.data_ptr() + 4 * 256, 291, dst.data_ptr() + 2 * 256, 296, 100, 35, 40, _stream()), "to_bf16_block")
-    torch.cuda.synchronize()
-    assert torch.equal(dst[:, 256:291], src[:, 256:291].bfloat16())
-    assert float(dst[:, 291:296].abs().max()) == 0.0
-    assert float((dst[:, :256] - 7.0).abs().max()) == 0.0
-
-
 def test_adam_ranges_and_staging():
     """spv_adam on sub-ranges with bf16 staging == one launch over the whole vector == torch.optim.Adam semantics"""
     from spvipes_b200 import _lib as L
@@ -214,55 +201,3 @@ def test_adam_ranges_and_staging():
                          ticket.data_ptr(), 0, None, None, None, None, None, None, None, 0, _stream()), "spv_adam")
     torch.cuda.synchronize()
     assert int(step2) == t and int(ticket) == 0 and torch.equal(p, pa)
-
-
-@pytest.mark.parametrize("B,G,N", [(300, 1003, 256), (512, 5000, 256), (64, 130, 64)])
-def test_enc_fc1_fused_count_transform(B, G, N):
-    """spv_enc_fc1_fwd / spv_enc_fc1_dw: the encoder's first layer and its weight gradient straight from uint16 counts (row gather,
-    log1p looked up as a split-bf16 pair by the GEMM's producer warps, three MMAs per k-step) against float64; fp32-grade."""
-    from spvipes_b200 import _lib as L
-    lib = L.load()
-    g = torch.Generator(device="cuda").manual_seed(8)
-    Nrows = 3 * B
-    ldx = G + 5 if G % 8 else G  # a pitch that breaks the 16-byte alignment of the rows exercises the scalar gather
-    Xf = torch.zeros(Nrows, ldx, device="cuda")
-    Xf[:, :G] = torch.poisson(torch.rand(Nrows, G, generator=g, device="cuda") * 3.0, generator=g)
-    Xf[::7, 3] = 40000.0  # beyond the 256-entry table
-    Xf[1::5, G - 1] = 300.0
-    X = Xf.to(torch.int32).to(torch.uint16)
-    rows = torch.randperm(Nrows, generator=g, device="cuda")[:B].to(torch.int32)
-    r8 = lambda x: (x + 7) // 8 * 8
-    W = (torch.rand(N, G, generator=g, device="cuda") * 2 - 1) * 0.05
-    bias = torch.randn(N, generator=g, device="cuda") * 0.1
-    Wh = torch.zeros(N, r8(G), device="cuda", dtype=torch.bfloat16); Wl = torch.zeros_like(Wh)
-    L.check(lib.spv_to_bf16_split(W.data_ptr(), G, Wh.data_ptr(), Wl.data_ptr(), Wh.stride(0), N, G, _stream()), "split")
-    T = torch.log1p(Xf[rows.long(), :G].double())
-    want = torch.relu(T @ W.double().t() + bias.double())
-    ws = torch.empty(8 * B * N, device="cuda")
-    for splits in (1, 4):
-        h1 = torch.full((B, N), float("nan"), device="cuda")
-        L.check(lib.spv_enc_fc1_fwd(X.data_ptr(), ldx, rows.data_ptr(), Wh.data_ptr(), Wl.data_ptr(), Wh.stride(0), h1.data_ptr(), N, B, N, G,
-                                    bias.data_ptr(), 1, 0, splits, ws.data_ptr(), _stream()), "spv_enc_fc1_fwd")
-        torch.cuda.synchronize()
-        err = float((h1.double() - want).abs().max() / want.abs().max())
-        assert err < 5e-5, ("fwd", splits, err)
-    # pre-activation addend (batch covariates): h1 <- relu(counts term + h1)
-    pre = torch.randn(B, N, generator=g, device="cuda")
-    h1 = pre.clone()
-    L.check(lib.spv_enc_fc1_fwd(X.data_ptr(), ldx, rows.data_ptr(), Wh.data_ptr(), Wl.data_ptr(), Wh.stride(0), h1.data_ptr(), N, B, N, G,
-                                None, 1, 1, 2, ws.data_ptr(), _stream()), "spv_enc_fc1_fwd")
-    torch.cuda.synchronize()
-    want2 = torch.relu(T @ W.double().t() + pre.double())
-    assert float((h1.double() - want2).abs().max() / want2.abs().max()) < 5e-5
-    # weight gradient
-    d = torch.randn(B, N, generator=g, device="cuda") * (torch.rand(B, N, generator=g, device="cuda") < 0.5)
-    dh = torch.zeros(B, N, device="cuda", dtype=torch.bfloat16); dl = torch.zeros_like(dh)
-    L.check(lib.spv_to_bf16_split(d.data_ptr(), N, dh.data_ptr(), dl.data_ptr(), N, B, N, _stream()), "split")
-    dW = torch.full((N, G + 3), float("nan"), device="cuda")
-    L.check(lib.spv_enc_fc1_dw(X.data_ptr(), ldx, rows.data_ptr(), dh.data_ptr(), dl.data_ptr(), N, dW.data_ptr(), G + 3, B, N, G, _stream()),
-            "spv_enc_fc1_dw")
-    torch.cuda.synchronize()
-    wantW = d.double().t() @ T
-    err = float((dW[:, :G].double() - wantW).abs().max() / wantW.abs().max())
-    assert err < 5e-5, ("dw", err)
-    assert bool(torch.isnan(dW[:, G:]).all())  # columns beyond the genes are left alone

@@ -139,11 +139,15 @@ def test_early_adam_is_the_same_update():
     out = []
     for early in (True, False):
         eng, batches, noise = engine_from_golden(gd, precision="bf16")
-        loop = TrainLoop(eng)
-        loop.early_adam = early
+        loop = TrainLoop(eng)  # (also for the reference: it sets the engine's stage_in_adam)
         loop.set_epoch(1)
         for _ in range(3):
-            loop.step(batches, noise)
+            if early:
+                loop.step(batches, noise)
+            else:
+                eng.forward(batches, training=True, noise=noise)
+                eng.backward()
+                eng.adam_step(lr=loop.lr, eps=loop.eps, weight_decay=loop.weight_decay)
         torch.cuda.synchronize()
         out.append((eng.params.flat.clone(), eng.adam_m.clone(), eng.adam_v.clone(), int(eng.step_dev), eng.wb[0][0].clone(),
                     eng.wb[0][1][:eng.d.genes[0]].clone()))
