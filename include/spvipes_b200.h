@@ -206,7 +206,7 @@ int spv_dec_nb_bwd(int src, const void* const* ptrs, long long ldx, long long ld
  * amix_bf16 [B, ld_amixb] = [hm | zz] and wstack_bf16 [>= G, ld_w] (the mixture weight) hold FP16 values (spv_to_f16 /
  * spv_adam staging; the parameter names predate the switch); zc_f16 [B, 64], wz_f16 [2 Gp, 64]: the fp16 branch operands
  * written by spv_dec_fold.  part_nb (ptrs[11]) needs spv_dec_nb_part_floats(B, G) floats.
- * store_pi: also write the mixture logits to ptrs[10] (fp32). */
+ * store_pi must be 0 (any other value: SPV_ERR_ARG): the mixture logits stay in tensor memory. */
 int spv_dec_nb_fwd_tc(int src, const void* const* ptrs, long long ldx, const void* amix_bf16, long long ld_amixb,
                       const void* wstack_bf16, long long ld_w, int Gp, const void* zc_f16, const void* wz_f16, int B, int G,
                       int HD, int P, int S, int store_pi, int kmix, void* stream);
