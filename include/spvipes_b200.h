@@ -227,6 +227,23 @@ int spv_dec_nb_elems_tc(int src, const void* const* ptrs, long long ldx, const v
                         int HD, int P, int S, int kmix, void* const* outs, long long ld_out, void* stream);
 int spv_dec_nb_elems(int src, const void* const* ptrs, long long ldx, long long ld_amix, int B, int G, int HD, int P, int S,
                      int pi_ready, const float* zzb, long long ld_zzb, int kmix, void* const* outs, long long ld_out, void* stream);
+/* count draws from the NB mixture (scvi NegativeBinomialMixture.sample, theta2 = None), per element and draw:
+ *   mu = rate_p if Bernoulli(sigmoid(pi)) else rate_s;  lam = min(Gamma(theta, rate theta / mu), 1e8);  count = Poisson(lam)
+ * (0 where mu = 0).  Draws d = draw0 .. draw0 + n_draws - 1 go to out + (d - draw0) * draw_pitch, each [B, ld_out] fp32 row-major
+ * (draw_pitch >= (B - 1) * ld_out + G unless n_draws = 1).  A draw is a function of (seed, group, d, row b of the minibatch,
+ * gene g) only; group in [0, 127], draw0 + n_draws <= 2^32.  The counters are disjoint from those of the reparameterisation noise
+ * and the dropout masks under the same seed.
+ * spv_dec_nb_sample_tc: the tensor-core sampling sweep on the operands of spv_dec_nb_elems_tc (state of the same pass; counts,
+ * count table and part_nb unused); rate_p, rate_s and pi are those spv_dec_nb_elems_tc writes and are not stored.
+ * spv_nb_mixture_sample: the same draws from given parameters mu1 = rate_p, mu2 = rate_s, pi ([B, ld_in] fp32 each) and
+ * theta [G] (exp(px_r)); bitwise equal to the sweep's on the sweep's own rates. */
+int spv_dec_nb_sample_tc(const void* const* ptrs, const void* amix_bf16, long long ld_amixb, const void* wstack_bf16, long long ld_w,
+                         int Gp, const void* zc_f16, const void* wz_f16, int B, int G, int HD, int P, int S, int kmix,
+                         unsigned long long seed, int group, unsigned int draw0, int n_draws, float* out, long long ld_out,
+                         long long draw_pitch, void* stream);
+int spv_nb_mixture_sample(const float* mu1, const float* mu2, const float* pi, long long ld_in, const float* theta, int B, int G,
+                          int n_draws, float* out, long long ld_out, long long draw_pitch, unsigned long long seed, int group,
+                          unsigned int draw0, void* stream);
 /* tensor-core version of phase 1 of spv_dec_nb_fwd: softmax normalisers rowc[b, 0:2] = lib[b] - logsumexp_g(y_p), (y_s)
  * from the fp16 branch operands (spv_dec_fold); part_stats: scratch of 2 * ceil(G/64) * B * 4 floats.
  * nn/networks.py:318-320, module/spVIPESmodule.py:751-757 */

@@ -15,6 +15,7 @@ POE_LABEL, POE_PAIRED, POE_CLUSTER = 0, 1, 2
 PARTNER_PAD, PARTNER_ABSENT = -1, -2
 POE_MODES = {"label": POE_LABEL, "paired": POE_PAIRED, "cluster": POE_CLUSTER}
 GENEC_ROWS = 21  # decoder_common.cuh GC_N
+GC_THETA = 8  # row of theta = exp(px_r) in the per-gene constant table (decoder_common.cuh)
 # widest latent input (P + S, plus one copy of the batch covariates per branch) of the decoder kernels: the fused tensor-core
 # decoder (decoder_common.cuh ZK_MAX_LATENT) and every decoder path (DEC_MAX_LATENT: spv_dec_fold, spv_dec_gene_bwd)
 ZK_MAX_LATENT = 58
@@ -62,6 +63,8 @@ _SIGS = {
     "spv_dec_nb_fwd_tc": [i, p, ll, p, ll, p, ll, i, p, p, i, i, i, i, i, i, i, p],
     "spv_dec_nb_elems_tc": [i, p, ll, p, ll, p, ll, i, p, p, i, i, i, i, i, i, p, ll, p],
     "spv_dec_nb_elems": [i, p, ll, ll, i, i, i, i, i, i, p, ll, i, p, ll, p],
+    "spv_dec_nb_sample_tc": [p, p, ll, p, ll, i, p, p, i, i, i, i, i, i, u64, i, u32, i, p, ll, ll, p],
+    "spv_nb_mixture_sample": [p, p, p, ll, p, i, i, i, p, ll, ll, u64, i, u32, p],
     "spv_dec_nb_rowreduce": [p, i, i, i, p, p, p],
     "spv_dec_gene_bwd": [p, ll, i, i, i, i, i, p],
     "spv_dec_gene_bwd_parts": [i],

@@ -435,6 +435,8 @@ class StepEngine:
         # advanced by every forward and every backward pass, eager or replayed from a CUDA graph (note_replay): a pass's decoder
         # state in the workspaces (what decode_elements reads) is current while the generation is the one it was made in
         self.generation = 0
+        # calls of px.sample() without a seed: each draws under seed + this counter (module.py _NBMixtureHandle.sample)
+        self.sample_calls = 0
 
     # -------------------------------------------------------------------------------- helpers
     def P(self, g, name):
@@ -818,16 +820,8 @@ class StepEngine:
           pi      px_mixing (the mixing logit, bias included),  mean  sigmoid(pi) rate_p + (1 - sigmoid(pi)) rate_s
         The state is the one the pass left in the workspaces: after forward(..., decode=False) in eval mode the decoder's prologue
         runs here (not the likelihood sweep: no loss, so the groups may differ in size).  No spv_loss, no gradient state."""
-        ctx = self._ctx
-        if ctx is None:
-            raise RuntimeError("decode_elements() follows a forward pass")
-        if ctx.get("dec_gen") != self.generation:
-            if "dec_gen" in ctx or self.generation != ctx["gen"]:
-                raise RuntimeError("the decoder state of the last forward is gone: a backward or another forward ran since")
-            if ctx["training"]:
-                raise RuntimeError("decode_elements() after a training-mode forward(..., decode=False): running the decoder here would "
-                                   "update its BatchNorm running statistics a second time; decode the training pass instead")
-        d, lib = self.d, self.lib
+        ctx = self._decoder_ctx("decode_elements()")
+        d = self.d
         idx = {k: i for i, k in enumerate(ELEM_OUTPUTS)}
         for g in (0, 1):
             for k in (outs[g] or {}):
@@ -850,25 +844,96 @@ class StepEngine:
                                      f"along the genes and the row pitch of the group's other outputs is needed, got "
                                      f"{tuple(t.shape)} {t.dtype} strides {t.stride()}")
                 ld = t.stride(0)
-            arr = L.ptr_array([og.get(k) for k in ELEM_OUTPUTS])
-            src, xptr, ldx, rows = ctx["srcs"][g]
             v = value[g] if value is not None else None
             if v is not None:
                 if v.dtype != torch.float32 or not self._on_device(v) or v.dim() != 2 or v.shape[0] != B or v.shape[1] < G or v.stride(1) != 1:
                     raise ValueError(f"value of group {g}: a float32 {self.device} tensor [{B}, >= {G}] with unit stride along the genes is "
                                      f"needed, got {tuple(v.shape)} {v.dtype}")
-                src, xptr, ldx, rows = L.SRC_F32, v.data_ptr(), v.stride(0), None
-            dptrs = self._dec_ptrs(g, w, xptr, rows, False)
-            nb, Pb, Sb, KZb, KMIX = d.nb, d.Pb, d.Sb, d.KZb, d.KMIX
-            if self.fused_nb:
-                L.check(lib.spv_dec_nb_elems_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb),
-                                                L.ptr(w.wzf), B, G, HD, Pb, Sb, KMIX, arr, ld, st), "spv_dec_nb_elems_tc")
+            self._elements_launch(ctx, g, og, ld, v)
+        if run_prologue:
+            ctx["dec_gen"] = self.generation
+
+    def _decoder_ctx(self, what):
+        """the context of the pass whose decoder state the element launches read (decode_elements, decode_sample)"""
+        ctx = self._ctx
+        if ctx is None:
+            raise RuntimeError(f"{what} follows a forward pass")
+        if ctx.get("dec_gen") != self.generation:
+            if "dec_gen" in ctx or self.generation != ctx["gen"]:
+                raise RuntimeError("the decoder state of the last forward is gone: a backward or another forward ran since")
+            if ctx["training"]:
+                raise RuntimeError(f"{what} after a training-mode forward(..., decode=False): running the decoder here would "
+                                   "update its BatchNorm running statistics a second time; decode the training pass instead")
+        return ctx
+
+    def _elements_launch(self, ctx, g, og, ld, v=None):
+        """the element launch of group g (after its prologue): the outputs og (checked) with row pitch ld; v: target values or None"""
+        d, lib = self.d, self.lib
+        w, B, G, st = ctx["ws"][g], ctx["Bs"][g], d.genes[g], self._stream()
+        arr = L.ptr_array([og.get(k) for k in ELEM_OUTPUTS])
+        src, xptr, ldx, rows = ctx["srcs"][g]
+        if v is not None:
+            src, xptr, ldx, rows = L.SRC_F32, v.data_ptr(), v.stride(0), None
+        dptrs = self._dec_ptrs(g, w, xptr, rows, False)
+        nb, Pb, Sb, KZb, KMIX = d.nb, d.Pb, d.Sb, d.KZb, d.KMIX
+        if self.fused_nb:
+            L.check(lib.spv_dec_nb_elems_tc(src, dptrs, ldx, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb),
+                                            L.ptr(w.wzf), B, G, HD, Pb, Sb, KMIX, arr, ld, st), "spv_dec_nb_elems_tc")
+            return
+        if self.bf16:  # the unfused bf16 decoder's mixture logits: the tensor-core GEMM of its sweep
+            self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
+            self._tc_gemm(L.ptr(w.amixb), L.ptr(w.Wmb), L.ptr(w.pi), B, G, KMIX, lda=w.KMp, ldb=w.KMp, ldc=G, bias=L.ptr(self.P(g, "bm")))
+        L.check(lib.spv_dec_nb_elems(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1 if self.bf16 else 0, L.ptr(w.zzb) if nb else None,
+                                     KZb, KMIX, arr, ld, st), "spv_dec_nb_elems")
+
+    def decode_sample(self, outs, seed, draw0=0):
+        """count draws from the NB mixture of the current pass (scvi NegativeBinomialMixture.sample, theta2 = None): outs[g] is a
+        float32 device tensor [n_draws, B_g, >= G_g] (unit stride along the genes) that receives draws draw0 .. draw0 + n_draws - 1
+        of group g, or None (group not sampled).  A draw is a function of (seed, group, draw index, row of the minibatch, gene)
+        only: sampling one group, a range of draw indices or both groups at once gives the same values for the same key.  Same
+        decoder state and rules as decode_elements.  The fused bf16 decoder samples in one tensor-core sweep that writes nothing
+        else; the other paths write rate_p, rate_s and pi with the element launch and sample them (spv_nb_mixture_sample)."""
+        ctx = self._decoder_ctx("decode_sample()")
+        d, lib = self.d, self.lib
+        if len(outs) != 2:
+            raise ValueError("outs: one tensor (or None) per group")
+        seed, draw0 = int(seed), int(draw0)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError(f"seed must lie in [0, 2**64), got {seed}")
+        for g in (0, 1):
+            t = outs[g]
+            if t is None:
                 continue
-            if self.bf16:  # the unfused bf16 decoder's mixture logits: the tensor-core GEMM of its sweep
-                self._to_dec(L.ptr(w.amix), KMIX, L.ptr(w.amixb), w.KMp, B, KMIX)
-                self._tc_gemm(L.ptr(w.amixb), L.ptr(w.Wmb), L.ptr(w.pi), B, G, KMIX, lda=w.KMp, ldb=w.KMp, ldc=G, bias=L.ptr(self.P(g, "bm")))
-            L.check(lib.spv_dec_nb_elems(src, dptrs, ldx, KMIX, B, G, HD, Pb, Sb, 1 if self.bf16 else 0, L.ptr(w.zzb) if nb else None,
-                                         KZb, KMIX, arr, ld, st), "spv_dec_nb_elems")
+            B, G = ctx["Bs"][g], d.genes[g]
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or not self._on_device(t) or t.dim() != 3 or \
+                    t.shape[0] < 1 or t.shape[1] != B or t.shape[2] < G or t.stride(2) != 1 or \
+                    (t.shape[0] > 1 and t.stride(0) < (B - 1) * t.stride(1) + G):
+                raise ValueError(f"sample output of group {g}: a float32 {self.device} tensor [n_draws, {B}, >= {G}] with unit stride "
+                                 f"along the genes and non-overlapping draws is needed, got "
+                                 f"{tuple(t.shape) if isinstance(t, torch.Tensor) else type(t).__name__}")
+            if not 0 <= draw0 <= 2 ** 32 - t.shape[0]:
+                raise ValueError(f"draw indices [{draw0}, {draw0 + t.shape[0]}) must lie in [0, 2**32)")
+        run_prologue = ctx.get("dec_gen") != self.generation
+        for g in self._fork_groups():
+            if run_prologue:
+                self._dec_prologue(ctx, g)
+            self._join(g)
+            t = outs[g]
+            if t is None:
+                continue
+            w, B, G, st = ctx["ws"][g], ctx["Bs"][g], d.genes[g], self._stream()
+            n = t.shape[0]
+            if self.fused_nb:
+                dptrs = self._dec_ptrs(g, w, None, None, False)
+                L.check(lib.spv_dec_nb_sample_tc(dptrs, L.ptr(w.amixb), w.KMp, L.ptr(w.Wstack), w.KMp, w.Gp, L.ptr(w.zcb), L.ptr(w.wzf),
+                                                 B, G, HD, d.Pb, d.Sb, d.KMIX, seed, g, draw0, n, t.data_ptr(), t.stride(1), t.stride(0),
+                                                 st), "spv_dec_nb_sample_tc")
+                continue
+            par = torch.empty(3, B, G, dtype=torch.float32, device=self.device)
+            self._elements_launch(ctx, g, {"rate_p": par[0], "rate_s": par[1], "pi": par[2]}, G)
+            L.check(lib.spv_nb_mixture_sample(par[0].data_ptr(), par[1].data_ptr(), par[2].data_ptr(), G,
+                                              w.genec.data_ptr() + 4 * L.GC_THETA * G, B, G, n, t.data_ptr(), t.stride(1), t.stride(0),
+                                              seed, g, draw0, st), "spv_nb_mixture_sample")
         if run_prologue:
             ctx["dec_gen"] = self.generation
 

@@ -402,17 +402,7 @@ class spVIPES:
             raise ValueError(f"unknown decoded output(s) {bad or outputs}; choose from {sorted(self.DECODED_OUTPUTS)}")
         eng = self.module.engine
         genes = eng.d.genes
-        sel = [None, None]
-        if gene_indices is not None:
-            if len(gene_indices) != 2:
-                raise ValueError("gene_indices: one sequence (or None) per group")
-            for g in (0, 1):
-                if gene_indices[g] is None:
-                    continue
-                gi = np.asarray(gene_indices[g], dtype=np.int64).reshape(-1)
-                if gi.size and (gi.min() < 0 or gi.max() >= genes[g]):
-                    raise ValueError(f"gene_indices[{g}]: positions must lie in [0, {genes[g]})")
-                sel[g] = torch.from_numpy(gi).to(eng.device)
+        sel = self._gene_selection(gene_indices)
         n = [len(g) for g in group_indices_list]
         res = {o: [[], []] for o in outputs}
         for _, ws in self._eval_passes(group_indices_list, batch_size, drop_last, _noise_fn):
@@ -424,6 +414,67 @@ class spVIPES:
                     t = outs[g][self.DECODED_OUTPUTS[o]]
                     res[o][g].append((t if sel[g] is None else t.index_select(1, sel[g])).cpu())
         return {o: {g: torch.cat(res[o][g]).numpy()[:n[g]] for g in (0, 1)} for o in outputs}
+
+    def _gene_selection(self, gene_indices):
+        """gene_indices (None, or one sequence or None per group) -> per group None or a device index tensor, checked"""
+        eng = self.module.engine
+        genes = eng.d.genes
+        sel = [None, None]
+        if gene_indices is not None:
+            if len(gene_indices) != 2:
+                raise ValueError("gene_indices: one sequence (or None) per group")
+            for g in (0, 1):
+                if gene_indices[g] is None:
+                    continue
+                gi = np.asarray(gene_indices[g], dtype=np.int64).reshape(-1)
+                if gi.size and (gi.min() < 0 or gi.max() >= genes[g]):
+                    raise ValueError(f"gene_indices[{g}]: positions must lie in [0, {genes[g]})")
+                sel[g] = torch.from_numpy(gi).to(eng.device)
+        return sel
+
+    @torch.no_grad()
+    def posterior_predictive_sample(self, group_indices_list: Sequence[Sequence[int]], n_samples: int = 1, gene_indices=None,
+                                    batch_size: Optional[int] = None, drop_last: Optional[bool] = None, seed: Optional[int] = None,
+                                    _noise_fn=None) -> dict:
+        """counts drawn from the eval-mode model's NB mixture (scvi 0.20 posterior_predictive_sample / VAE.sample): each of the
+        n_samples draws takes its own latent sample (its own eval pass over the minibatches of get_decoded_expression, with the
+        same cycling, truncation and row order) and one count draw per cell and gene from it (px.sample).
+        gene_indices: as in get_decoded_expression (selected on the GPU before the copy to the host).
+        seed: an int gives reproducible count draws for given latents; None takes the engine's seed plus its sample-call counter.
+        Every eval pass draws under its own draw index (its position among all passes), so no two minibatches share counters.  The latent noise comes from the engine's Philox streams (or _noise_fn).
+        Returns {0: ndarray, 1: ndarray} float32: [n_g, k_g] when n_samples == 1, else [n_g, k_g, n_samples]."""
+        n_samples = int(n_samples)
+        if n_samples < 1:
+            raise ValueError(f"n_samples must be >= 1, got {n_samples}")
+        eng = self.module.engine
+        if seed is None:
+            seed = (eng.seed + eng.sample_calls) % 2 ** 64
+            eng.sample_calls += 1
+        elif not 0 <= int(seed) < 2 ** 64:
+            raise ValueError(f"seed must lie in [0, 2**64), got {seed}")
+        seed = int(seed)
+        genes = eng.d.genes
+        sel = self._gene_selection(gene_indices)
+        n = [len(g) for g in group_indices_list]
+        res = [[[] for _ in range(n_samples)] for _ in (0, 1)]
+        passes = 0
+
+        def noise_fn(_, b0, b1):  # the test hook numbers the passes across all samples
+            return _noise_fn(passes, b0, b1)
+
+        for s in range(n_samples):
+            for _, ws in self._eval_passes(group_indices_list, batch_size, drop_last, noise_fn if _noise_fn is not None else None):
+                outs = [torch.empty(1, ws[g].B, genes[g], dtype=torch.float32, device=eng.device) for g in (0, 1)]
+                eng.decode_sample(outs, seed, draw0=passes)
+                passes += 1
+                for g in (0, 1):
+                    t = outs[g][0]
+                    res[g][s].append((t if sel[g] is None else t.index_select(1, sel[g])).cpu())
+        out = {}
+        for g in (0, 1):
+            draws = [torch.cat(res[g][s]).numpy()[:n[g]] for s in range(n_samples)]
+            out[g] = draws[0] if n_samples == 1 else np.stack(draws, axis=-1)
+        return out
 
     def get_loadings(self) -> dict:
         """reference model/spvipes.py:652-677"""

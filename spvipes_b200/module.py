@@ -31,6 +31,7 @@ import torch
 from torch import nn
 from torch.distributions import Normal
 
+from ._lib import GC_THETA
 from .engine import GroupBatch, Noise, StepEngine
 
 X_KEY, BATCH_KEY, LABELS_KEY = "X", "batch", "labels"  # scvi.REGISTRY_KEYS
@@ -59,16 +60,13 @@ class LossOutput:
         return sum(v.sum() for v in self.kl_local.values())
 
 
-GC_THETA = 8  # row of theta = exp(px_r) in the decoder's per-gene constant table (csrc/decoder_common.cuh)
-
-
 class _NBMixtureHandle:
     """stands where the reference puts scvi's NegativeBinomialMixture (`px`) of one group (module/spVIPESmodule.py:759).
     neg_log_prob_sum = -log_prob(log1p(x)).sum(-1), evaluated by the likelihood sweep of the pass.  The per-gene members are
     device tensors [B, G] without autograd, each computed on first access by one element launch (StepEngine.decode_elements) from
     the decoder state of the pass that built this handle, and cached: mu1 = px_rate_private, mu2 = px_rate_shared,
     mixture_logits = px_mixing, theta1 = exp(px_r) (an expanded view), mean = sigmoid(pi) mu1 + (1 - sigmoid(pi)) mu2 and
-    log_prob(value) (eps 1e-8).  Once the engine has run another forward or backward that state is gone: a member not read by
+    log_prob(value) (eps 1e-8); sample(sample_shape, seed) draws counts (not cached).  Once the engine has run another forward or backward that state is gone: a member not read by
     then raises RuntimeError; members already read are independent tensors and keep their values."""
 
     def __init__(self, rec: torch.Tensor, engine=None, group: int = 0, ws=None):
@@ -128,6 +126,24 @@ class _NBMixtureHandle:
     @property
     def theta2(self):  # scvi: theta2 = None means theta1 for both components (the reference's shared dispersion)
         return None
+
+    def sample(self, sample_shape=torch.Size(), seed=None):
+        """count draws [*sample_shape, B, G] float32 on the device (scvi NegativeBinomialMixture.sample, theta2 = None): per draw
+        and element, mu1 with probability sigmoid(mixture_logits), else mu2; then Poisson(min(Gamma(theta1, theta1 / mu), 1e8)).
+        seed: an int gives reproducible draws (a function of seed, group, draw index, cell and gene); None takes the engine's
+        seed plus a counter the engine advances on every such call, so that repeated calls differ.  Not cached."""
+        self._check("sample")
+        shape = torch.Size(sample_shape)
+        w, eng = self._ws, self._eng
+        if seed is None:
+            seed = (eng.seed + eng.sample_calls) % 2 ** 64
+            eng.sample_calls += 1
+        out = torch.empty(shape.numel(), w.B, w.G, dtype=torch.float32, device=eng.device)
+        if out.numel():
+            outs = [None, None]
+            outs[self._g] = out
+            eng.decode_sample(outs, seed)
+        return out.view(*shape, w.B, w.G)
 
     def log_prob(self, value):
         """log_mixture_nb(value; mu1, mu2, theta1, mixture_logits), eps 1e-8, per element [B, G]; value: a [B, G] float tensor,
