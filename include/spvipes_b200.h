@@ -169,6 +169,11 @@ int spv_poe_bwd(int mode, int S, int P, int B0, int B1, const void* const* ptrs0
 /* out[0] = loss (:886-893), out[1..4] = mean KL private0, poe0, private1, poe1 (:870-875), out[5..6] = mean rec0, rec1 */
 int spv_loss(const float* rec0, const float* rec1, const float* klp0, const float* klq0, const float* klp1, const float* klq1,
              int B, const float* kl_weight, float* out, void* stream);
+/* one evaluation pass added to a float64 accumulator acc[8] (validation epochs, get_elbo); the groups may differ in size:
+ * acc[0..5] += sum rec0, sum rec1, sum klp0, sum klq0, sum klp1, sum klq1 (each group over its own B_g cells, fp32 sums),
+ * acc[6] += B0 (n_obs), acc[7] += sum rec0 + sum rec1 + (*kl_weight) * (sum of the four KL sums).  One CTA, graph-capturable */
+int spv_elbo_accumulate(const float* rec0, const float* rec1, const float* klp0, const float* klq0, const float* klp1,
+                        const float* klq1, int B0, int B1, const float* kl_weight, double* acc, void* stream);
 
 /* decoder: closed-form per-gene BatchNorm fold + NB constants.
  * ptrs (18): Wp, Ws, gamma_p, beta_p, gamma_s, beta_s, px_r, rm_p, rv_p, rm_s, rv_s, zz, zsum, scratch [ceil(B/64), (P+S) + (P+S)^2]

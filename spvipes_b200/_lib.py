@@ -57,6 +57,7 @@ _SIGS = {
     "spv_poe_fwd": [i, i, i, i, i, p, p, p, p, u64, p, p],
     "spv_poe_bwd": [i, i, i, i, i, p, p, p, p, u64, p, p, f, p],
     "spv_loss": [p, p, p, p, p, p, i, p, p, p],
+    "spv_elbo_accumulate": [p, p, p, p, p, p, i, i, p, p, p],
     "spv_dec_fold": [p, ll, i, i, i, i, i, f, f, p, ll, i, i, p, p, p],
     "spv_dec_nb_fwd": [i, p, ll, ll, i, i, i, i, i, i, p, ll, i, p],
     "spv_dec_nb_bwd": [i, p, ll, ll, i, i, i, i, i, f, p, p, ll, p, ll, i, p],

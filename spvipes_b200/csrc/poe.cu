@@ -585,3 +585,46 @@ extern "C" int spv_loss(const float* rec0, const float* rec1, const float* klp0,
     SPV_CHECK_LAUNCH();
     return SPV_OK;
 }
+
+// one evaluation pass's loss terms added to a float64 accumulator (validation epochs, get_elbo):
+// acc[0..5] += sum rec0, sum rec1, sum klp0, sum klq0, sum klp1, sum klq1 (each group over its own B_g cells, fp32 as loss_kernel),
+// acc[6] += B0 (n_obs of the minibatch: group 0's size), acc[7] += sum rec0 + sum rec1 + w (sum of the four KL sums).
+// The groups may differ in size: nothing is paired across them.  float64 so that ~50 minibatch sums of an epoch do not drift.
+__global__ void elbo_accumulate_kernel(const float* __restrict__ rec0, const float* __restrict__ rec1,
+                                       const float* __restrict__ klp0, const float* __restrict__ klq0,
+                                       const float* __restrict__ klp1, const float* __restrict__ klq1, int B0, int B1,
+                                       const float* __restrict__ kl_weight, double* __restrict__ acc) {
+    __shared__ float red[6][32];
+    float a[6] = {0, 0, 0, 0, 0, 0};
+    for (int b = threadIdx.x; b < B0; b += blockDim.x) {
+        a[0] += rec0[b]; a[2] += klp0[b]; a[3] += klq0[b];
+    }
+    for (int b = threadIdx.x; b < B1; b += blockDim.x) {
+        a[1] += rec1[b]; a[4] += klp1[b]; a[5] += klq1[b];
+    }
+    for (int k = 0; k < 6; ++k) {
+        float v = warp_sum(a[k]);
+        if ((threadIdx.x & 31) == 0) red[k][threadIdx.x >> 5] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s[6];
+        for (int k = 0; k < 6; ++k) {
+            float v = 0.0f;
+            for (int w2 = 0; w2 < (int)(blockDim.x >> 5); ++w2) v += red[k][w2];
+            s[k] = (double)v;
+            acc[k] += s[k];
+        }
+        acc[6] += (double)B0;
+        acc[7] += s[0] + s[1] + (double)*kl_weight * (s[2] + s[3] + s[4] + s[5]);
+    }
+}
+
+extern "C" int spv_elbo_accumulate(const float* rec0, const float* rec1, const float* klp0, const float* klq0, const float* klp1,
+                                   const float* klq1, int B0, int B1, const float* kl_weight, double* acc, void* stream) {
+    if (!rec0 || !rec1 || !klp0 || !klq0 || !klp1 || !klq1 || !kl_weight || !acc || B0 <= 0 || B1 <= 0) return SPV_ERR_ARG;
+    elbo_accumulate_kernel<<<1, 1024, 0, reinterpret_cast<cudaStream_t>(stream)>>>(rec0, rec1, klp0, klq0, klp1, klq1, B0, B1,
+                                                                                    kl_weight, acc);
+    SPV_CHECK_LAUNCH();
+    return SPV_OK;
+}

@@ -572,8 +572,10 @@ class StepEngine:
 
     # -------------------------------------------------------------------------------- forward
     def forward(self, batches: Sequence[GroupBatch], training: bool = True, noise: Optional[Noise] = None,
-                with_grad: Optional[bool] = None, decode: bool = True):
-        """inference -> generative -> loss.  Returns the workspaces (device tensors) holding every output."""
+                with_grad: Optional[bool] = None, decode: bool = True, loss: bool = True):
+        """inference -> generative -> loss.  Returns the workspaces (device tensors) holding every output.
+        loss=False: no spv_loss (loss_out is left alone), so the groups' minibatches may differ in size; the per-cell rec / klp / klq
+        of both groups are written all the same (evaluation passes: accumulate_elbo)."""
         with_grad = training if with_grad is None else with_grad
         self.generation += 1
         ctx = self._encode(batches, training, noise, with_grad, stage_wm=decode)
@@ -581,7 +583,7 @@ class StepEngine:
             for g in (0, 1):
                 self._join(g)
             return ctx["ws"]
-        return self._decode(ctx)
+        return self._decode(ctx, loss)
 
     def decode(self):
         """generative + loss on the latents of the preceding forward(decode=False) (same minibatch, same noise, BatchNorm
@@ -701,18 +703,42 @@ class StepEngine:
         if forward and self._ctx is not None:
             self._ctx["dec_gen"] = self.generation
 
-    def _decode(self, ctx):
+    def _decode(self, ctx, loss=True):
         # ---------------- decoders + NB likelihood (reference nn/networks.py:314-325, module :751-759, :817-824)
         Bs, ws = ctx["Bs"], ctx["ws"]
         for g in self._fork_groups():
             self._dec_prologue(ctx, g)
             self._dec_sweep(ctx, g)
         ctx["dec_gen"] = self.generation
+        if not loss:
+            return ws
         if Bs[0] != Bs[1]:
             raise ValueError("the loss needs equally sized minibatches in both groups (reference :886-893)")
         L.check(self.lib.spv_loss(L.ptr(ws[0].rec), L.ptr(ws[1].rec), L.ptr(ws[0].klp), L.ptr(ws[0].klq), L.ptr(ws[1].klp),
                                   L.ptr(ws[1].klq), Bs[0], L.ptr(self.kl_weight), L.ptr(self.loss_out), self._stream()), "spv_loss")
         return ws
+
+    def accumulate_elbo(self, ws, acc: torch.Tensor):
+        """add the loss terms of the pass that wrote the workspaces ws (forward(..., loss=False) or a training forward) to acc, a float64
+        device tensor [8]: [sum rec0, sum rec1, sum klp0, sum klq0, sum klp1, sum klq1, sum n_obs (= B0), sum of rec0 + rec1 +
+        kl_weight * KL] (spv_elbo_accumulate).  No host synchronisation: a validation epoch reads acc once, at its end."""
+        if acc.dtype != torch.float64 or acc.numel() != 8 or not acc.is_contiguous() or not self._on_device(acc):
+            raise ValueError(f"acc: a contiguous float64 {self.device} tensor of 8 elements is needed")
+        L.check(self.lib.spv_elbo_accumulate(L.ptr(ws[0].rec), L.ptr(ws[1].rec), L.ptr(ws[0].klp), L.ptr(ws[0].klq), L.ptr(ws[1].klp),
+                                             L.ptr(ws[1].klq), ws[0].B, ws[1].B, L.ptr(self.kl_weight), L.ptr(acc), self._stream()),
+                "spv_elbo_accumulate")
+
+    @contextlib.contextmanager
+    def noise_counter(self, counter: torch.Tensor):
+        """draw the Philox noise of the enclosed passes on `counter` (an int32 device tensor [1]) instead of noise_dev: evaluation passes
+        between training steps then leave the training noise stream exactly where it was.  The tensor is swapped, not its contents,
+        so a captured training graph (which holds noise_dev's address) is unaffected."""
+        keep = self.noise_dev
+        self.noise_dev = counter
+        try:
+            yield
+        finally:
+            self.noise_dev = keep
 
     def _dec_prologue(self, ctx, g):
         """group g's decoder up to the likelihood sweep: mixture-weight staging, covariate expansion, count tables, hidden layer,

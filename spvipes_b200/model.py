@@ -24,7 +24,13 @@ import torch
 
 from .engine import CsrCounts, GroupBatch
 from .module import spVIPESmodule
-from .trainer import TrainLoop, epoch_batches, split_indices
+from .trainer import (VALIDATION_METRICS, EarlyStopping, TrainLoop, elbo_metrics, epoch_batches, is_validation_epoch,
+                      split_indices, validation_interval)
+
+TRAIN_METRICS = ("elbo_train", "reconstruction_loss_train", "kl_local_train")
+# Philox counter of the evaluation passes of a validation run or get_elbo (reset to this value at the start of each run): the top
+# bit of the counter word, so it stays disjoint from the training passes, which count up from 0
+EVAL_NOISE_BASE = -2 ** 31  # int32 bit pattern 0x80000000
 
 
 @dataclass
@@ -172,6 +178,7 @@ class spVIPES:
                                     dropout_rate=dropout_rate, **model_kwargs)
         self.is_trained_ = False
         self.history: Dict[str, List[float]] = {"train_loss_epoch": []}
+        self.early_stopped_epoch_: Optional[int] = None
         self._device_data = None
 
     # ------------------------------------------------------------------ device-resident data
@@ -233,16 +240,37 @@ class spVIPES:
     def train(self, group_indices_list: Sequence[Sequence[int]], max_epochs: Optional[int] = None, use_gpu=None,
               train_size: float = 0.9, validation_size: Optional[float] = None, batch_size: int = 128,
               early_stopping: bool = False, n_steps_kl_warmup: Optional[int] = None, n_epochs_kl_warmup: Optional[int] = 400,
-              plan_kwargs: Optional[dict] = None, seed: int = 0, use_cuda_graph: bool = True, **kwargs):
-        """reference model/base/training_mixin.py:19-123 + scvi TrainingPlan / TrainRunner semantics"""
+              plan_kwargs: Optional[dict] = None, seed: int = 0, use_cuda_graph: bool = True,
+              check_val_every_n_epoch: Optional[int] = None, early_stopping_monitor: str = "elbo_validation",
+              early_stopping_patience: int = 45, early_stopping_min_delta: float = 0.0, early_stopping_mode: str = "min",
+              _noise_fn=None, **kwargs):
+        """reference model/base/training_mixin.py:19-123 + scvi TrainingPlan / TrainRunner / Trainer semantics.
+
+        Validation (scvi 0.20 Trainer arguments): after epoch e when (e + 1) % check_val_every_n_epoch == 0; None means every epoch
+        with early_stopping and never without.  A validation run takes the minibatches get_latent_representation takes on
+        self.val_idx (batch_size, drop_last=False) through eval-mode passes and appends elbo_validation,
+        reconstruction_loss_validation, kl_local_validation and validation_loss to history (trainer.elbo_metrics).  Its latent
+        noise comes from a Philox counter of its own and eval mode updates no BatchNorm statistics, so validation leaves the
+        training itself unchanged.  early_stopping: Lightning's EarlyStopping rule (trainer.EarlyStopping) on
+        early_stopping_monitor after each validation run; a stop ends training after that epoch (early_stopped_epoch_) with the
+        last epoch's parameters.  Every epoch also appends elbo_train, reconstruction_loss_train and kl_local_train.
+        _noise_fn (tests): as in get_latent_representation, for the validation passes."""
         n_obs = self.adata.X.shape[0]
         if max_epochs is None:
             max_epochs = int(min(round((20000 / n_obs) * 400), 400))  # reference :89-91
         plan_kwargs = dict(plan_kwargs or {})
         lr, eps, wd = plan_kwargs.get("lr", 1e-3), plan_kwargs.get("eps", 0.01), plan_kwargs.get("weight_decay", 1e-6)
-        self._to_device()
+        every = validation_interval(check_val_every_n_epoch, early_stopping)
+        stopper = EarlyStopping(early_stopping_monitor, early_stopping_patience, early_stopping_min_delta, early_stopping_mode)
         train_idx, self.val_idx, self.test_idx = split_indices(group_indices_list, train_size, validation_size, seed)
         self.train_idx = train_idx
+        if every is not None and min(len(v) for v in self.val_idx) == 0:
+            raise ValueError("validation (early_stopping or check_val_every_n_epoch) needs a non-empty validation split in both "
+                             f"groups, got {[len(v) for v in self.val_idx]} cells: lower train_size or set validation_size")
+        self._to_device()
+        for k in TRAIN_METRICS + (VALIDATION_METRICS if every is not None else ()):
+            self.history.setdefault(k, [])
+        self.early_stopped_epoch_ = None
         eng = self.module.engine
         if eng.mode != "label":
             # the OT modes index the plan / cluster labels with per-minibatch arrays: gather them on the host per step
@@ -259,7 +287,7 @@ class spVIPES:
                 raise ValueError("batch_size is larger than the training split of a group")
             local = [[torch.from_numpy(self._local_rows(g, st[g]).astype(np.int32)) for g in (0, 1)] for st in steps]
             dev_rows = [torch.stack([l[g] for l in local]).to(eng.device) for g in (0, 1)]
-            tot = torch.zeros((), device=eng.device)
+            tot = torch.zeros(7, device=eng.device)  # per-step loss_out[:7] summed over the epoch
             for s in range(len(steps)):
                 if n_steps_kl_warmup:  # scvi TrainingPlan: the step-based warm-up takes precedence over the epoch-based one
                     eng.set_kl_weight(min(1.0, global_step / n_steps_kl_warmup))
@@ -279,8 +307,24 @@ class spVIPES:
                     eng.note_replay(forward=False)
                 else:
                     loop.step(batches)
-                tot += eng.loss_out[0]
-            self.history["train_loss_epoch"].append(float(tot.item()) / len(steps))
+                tot += eng.loss_out[:7]
+            t = [float(v) for v in tot.cpu()]
+            self.history["train_loss_epoch"].append(t[0] / len(steps))
+            # every training minibatch holds batch_size cells in both groups: the mean over steps of the per-step means is the sum
+            # over the epoch divided by the epoch's n_obs
+            rec, kl = (t[5] + t[6]) / len(steps), (t[1] + t[2] + t[3] + t[4]) / len(steps)
+            for k, v in zip(TRAIN_METRICS, (rec + kl, rec, kl)):
+                self.history[k].append(v)
+            if is_validation_epoch(epoch, every):
+                if n_steps_kl_warmup:  # the weight after the epoch's last step (the next step sets its own before it runs)
+                    eng.set_kl_weight(min(1.0, global_step / n_steps_kl_warmup))
+                metrics = elbo_metrics(self._elbo_sums(self.val_idx, batch_size, False, _noise_fn))
+                self.module.train()
+                for k, v in metrics.items():
+                    self.history[k].append(v)
+                if early_stopping and stopper.update(metrics[early_stopping_monitor]):
+                    self.early_stopped_epoch_ = epoch
+                    break
         self.module.eval()
         self.is_trained_ = True
         return self
@@ -329,9 +373,10 @@ class spVIPES:
                 "shared_reordered": {0: shared[0], 1: shared[1][order]},
                 "private_reordered": {0: private[0], 1: private[1][order]}}
 
-    def _eval_passes(self, group_indices_list, batch_size, drop_last, _noise_fn):
+    def _eval_passes(self, group_indices_list, batch_size, drop_last, _noise_fn, decode=False):
         """the minibatches of the reference's latent extraction, each through an eval-mode encoder pass
-        (engine.forward(..., decode=False)): yields (batches, workspaces) per minibatch.  Sequential chunks of batch_size cells per
+        (engine.forward(..., decode=False); decode=True: the whole pass without the loss, engine.forward(..., loss=False)): yields
+        (batches, workspaces) per minibatch.  Sequential chunks of batch_size cells per
         group; reference :478-515: drop_last defaults to False in every mode; the paired OT mode (no labels) then goes through the
         cycling path, every other mode through one ConcatDataLoader over the two index lists"""
         self._to_device()
@@ -352,7 +397,9 @@ class spVIPES:
             largest = int(np.argmax([len(c) for c in chunks]))
             its = [iter(c) if g == largest else cycle(c) for g, c in enumerate(chunks)]
             for st in zip(*its):
-                rows = [torch.from_numpy(self._local_rows(g, st[g]).astype(np.int32)).to(eng.device) for g in (0, 1)]
+                # (pinned host memory: the upload does not wait for the previous minibatch's kernels)
+                rows = [torch.from_numpy(self._local_rows(g, st[g]).astype(np.int32)).pin_memory().to(eng.device, non_blocking=True)
+                        for g in (0, 1)]
                 batches = []
                 for g in (0, 1):
                     d = self._device_data[g]
@@ -362,7 +409,7 @@ class spVIPES:
                     batches.append(GroupBatch(X=d["X"], rows=rows[g], labels=lab, idx=d["idx"][r].contiguous(), B=len(st[g]), batch=bc))
                 noise = _noise_fn(counter[0], len(st[0]), len(st[1])) if _noise_fn is not None else None
                 counter[0] += 1
-                yield batches, eng.forward(batches, training=False, noise=noise, with_grad=False, decode=False)
+                yield batches, eng.forward(batches, training=False, noise=noise, with_grad=False, decode=decode, loss=False)
 
         if use_cycling:
             # reference _process_all_cells_with_cycling (:578-626): chunks of min(n) cells, the indices of BOTH groups taken
@@ -374,6 +421,34 @@ class spVIPES:
                 yield from process([[group_indices_list[g][(start + i) % n[g]] for i in range(lo)] for g in (0, 1)])
         else:
             yield from process(group_indices_list)
+
+    def _elbo_sums(self, group_indices_list, batch_size, drop_last, _noise_fn):
+        """float64 [8] host tensor of StepEngine.accumulate_elbo summed over the eval passes of _eval_passes (one host read).  The
+        latent noise is drawn on a counter that starts at EVAL_NOISE_BASE for every run: the training noise stream is not
+        advanced, and the same weights give the same value on every call."""
+        eng = self.module.engine
+        self._to_device()
+        acc = torch.zeros(8, dtype=torch.float64, device=eng.device)
+        counter = torch.full((1,), EVAL_NOISE_BASE, dtype=torch.int32, device=eng.device)
+        with eng.noise_counter(counter):
+            for _, ws in self._eval_passes(group_indices_list, batch_size, drop_last, _noise_fn, decode=True):
+                eng.accumulate_elbo(ws, acc)
+        # the passes overwrote the engine's per-pass decoder state: decode_elements / decode_sample need a forward of their own
+        eng._ctx = None
+        acc = acc.cpu()
+        if acc[6] <= 0:
+            raise ValueError("no minibatch to evaluate: a group's index list is empty (or drop_last removed every minibatch)")
+        return acc
+
+    @torch.no_grad()
+    def get_elbo(self, group_indices_list: Sequence[Sequence[int]], batch_size: Optional[int] = None,
+                 drop_last: Optional[bool] = None, _noise_fn=None) -> float:
+        """the evidence lower bound of the eval-mode model on the given cells (scvi VAEMixin.get_elbo sign convention: the ELBO,
+        i.e. minus the elbo metric (reconstruction loss + local KL per observation) that history["elbo_validation"] records).
+        Same minibatches as get_latent_representation (batch_size, drop_last, cycling); n_obs of a minibatch is the size of
+        group 0's part.  get_elbo(model.val_idx, batch_size) reproduces -history["elbo_validation"][-1] for the current weights.
+        _noise_fn (tests): as in get_latent_representation."""
+        return -elbo_metrics(self._elbo_sums(group_indices_list, batch_size, drop_last, _noise_fn))["elbo_validation"]
 
     # decoded outputs of get_decoded_expression -> StepEngine.decode_elements names
     DECODED_OUTPUTS = {"mean": "mean", "px_rate_private": "rate_p", "px_rate_shared": "rate_s", "px_mixing": "pi", "log_prob": "ll"}

@@ -77,6 +77,70 @@ def epoch_batches(train_idx: Sequence[np.ndarray], batch_size: int, shuffle=True
     return out
 
 
+# validation metrics of one validation run (scvi 0.20 ElboMetric names); early stopping monitors one of them
+VALIDATION_METRICS = ("elbo_validation", "reconstruction_loss_validation", "kl_local_validation", "validation_loss")
+
+
+def elbo_metrics(acc, suffix: str = "validation") -> dict:
+    """metrics from the float64 sums of StepEngine.accumulate_elbo over the minibatches of one run (scvi 0.20 ElboMetric over
+    LossOutput: every sum over all minibatches, divided by the sum of n_obs, the sizes of group 0's minibatches):
+      reconstruction_loss = sum(rec0 + rec1) / n_obs,  kl_local = sum(klp0 + klq0 + klp1 + klq1) / n_obs,
+      elbo = reconstruction_loss + kl_local (no global KL),  loss = sum(rec0 + rec1 + kl_weight * KL) / n_obs (validation only)"""
+    a = [float(v) for v in acc]
+    n = a[6]
+    rec, kl = (a[0] + a[1]) / n, (a[2] + a[3] + a[4] + a[5]) / n
+    out = {f"elbo_{suffix}": rec + kl, f"reconstruction_loss_{suffix}": rec, f"kl_local_{suffix}": kl}
+    if suffix == "validation":
+        out["validation_loss"] = a[7] / n
+    return out
+
+
+def validation_interval(check_val_every_n_epoch: Optional[int], early_stopping: bool) -> Optional[int]:
+    """epochs between validation runs (scvi 0.20 Trainer): None -> 1 with early stopping, else no validation (None)"""
+    if check_val_every_n_epoch is None:
+        return 1 if early_stopping else None
+    n = int(check_val_every_n_epoch)
+    if n != check_val_every_n_epoch or n < 1:
+        raise ValueError(f"check_val_every_n_epoch must be a positive integer or None, got {check_val_every_n_epoch!r}")
+    return n
+
+
+def is_validation_epoch(epoch: int, every: Optional[int]) -> bool:
+    """validation runs after epoch `epoch` (0-based) when (epoch + 1) % every == 0"""
+    return every is not None and (epoch + 1) % every == 0
+
+
+class EarlyStopping:
+    """the stopping rule of Lightning's EarlyStopping (check_finite=True), applied to one value per validation run:
+    the first finite value is an improvement; after it a value improves when value < best - min_delta (mode "min") or
+    value > best + min_delta (mode "max"); an improvement resets the wait count, anything else increments it, and training
+    stops when the count reaches `patience`.  A non-finite value stops at once."""
+
+    def __init__(self, monitor: str = "elbo_validation", patience: int = 45, min_delta: float = 0.0, mode: str = "min"):
+        if monitor not in VALIDATION_METRICS:
+            raise ValueError(f"early_stopping_monitor must be one of {VALIDATION_METRICS}, got {monitor!r}")
+        if mode not in ("min", "max"):
+            raise ValueError(f"early_stopping_mode must be 'min' or 'max', got {mode!r}")
+        self.monitor, self.patience, self.min_delta, self.mode = monitor, int(patience), float(min_delta), mode
+        self.best: Optional[float] = None
+        self.wait = 0
+        self.stopped = False
+
+    def update(self, value: float) -> bool:
+        """record one validation value; True when training should stop now"""
+        value = float(value)
+        if not math.isfinite(value):
+            self.stopped = True
+            return True
+        if self.best is None or (value < self.best - self.min_delta if self.mode == "min" else value > self.best + self.min_delta):
+            self.best, self.wait = value, 0
+        else:
+            self.wait += 1
+            if self.wait >= self.patience:
+                self.stopped = True
+        return self.stopped
+
+
 class TrainLoop:
     """fwd + bwd + Adam per minibatch on one GPU (one process per GPU; see parallel.py for the data-parallel wrapper)."""
 
